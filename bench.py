@@ -4,6 +4,7 @@ reference mel -> mel -> waveform) on B200.
 
     python bench.py --gpus N --steps K --warmup W            # ours (CUDA path)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU PyTorch path
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[1], SURVEY.md §8d config 2): per GPU, 16 utterances x 150 phoneme
 tokens, a 3 s reference mel (240 frames) each, forced integer durations summing to 400 per
@@ -14,6 +15,15 @@ reference's checkpoints are not redistributable (SURVEY.md F2).
 One JSON line on stdout (rank 0).  `value` = audio-seconds synthesised per wall-second with inputs
 resident in HBM; `e2e` = the same through the public API with pinned HOST inputs (H2D of tokens /
 reference mels, D2H of the waveforms inside the timed region).
+
+`--dump-outputs DIR` (CUDA arm) writes what the last timed step of the resident-input arm returned to its
+caller (rank 0): `wav.npy` float32 [B, 300 * frames], `mel.npy` float32 [B, 80, frames] and
+`mel_lengths.npy` float64 [B].  That step ran on input set
+`(warmup_calls(warmup, pipeline) + steps - 1) % N_INPUT_SETS` of `make_inputs(rank, ...)`.  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.  The
+outputs are copied on the device after the timed region and written once the clock sampling has stopped;
+more than 64 MB in all is cut to a seeded sample of utterances, whose indices are then written as
+`utterance_index.npy`.
 """
 from __future__ import annotations
 
@@ -153,6 +163,28 @@ def peaks():
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, wav, mel_lengths, mel) -> None:
+    """Write one step's (wav, mel_lengths, mel), in the order ``Synthesizer.synthesize`` returns them, as
+    ``out_dir/<name>.npy`` (float32 / float64).  Above DUMP_LIMIT_BYTES a seeded sample of utterances (the same
+    rows of every array) is written instead."""
+    import numpy as np
+    arrays = {"wav": wav.detach().float().cpu().numpy(), "mel": mel.detach().float().cpu().numpy(),
+              "mel_lengths": mel_lengths.detach().cpu().numpy().astype(np.float64)}
+    B = arrays["wav"].shape[0]
+    row_bytes = sum(a.nbytes for a in arrays.values()) / B
+    if B * row_bytes > DUMP_LIMIT_BYTES:
+        keep = max(1, int(DUMP_LIMIT_BYTES // row_bytes) - 1)     # one row's worth left for the index array
+        idx = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["utterance_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 # ------------------------------------------------------------------------------------------------
 # reference arm: the reference's own CPU PyTorch path (oracle/restate.py is its pinned restatement;
 # the reference tree itself does not exist on the GPU box)
@@ -224,6 +256,11 @@ def run_reference(args):
 # ------------------------------------------------------------------------------------------------
 def _events():
     return torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+
+
+def warmup_calls(warmup: int, depth: int) -> int:
+    """Untimed calls of each arm before its timed steps: at least 3, and two per batch in flight."""
+    return max(warmup, 3, 2 * depth)
 
 
 def _median(xs):
@@ -564,13 +601,15 @@ def run_ours(args):
     host_sets = [(t.pin_memory(), m.pin_memory(), d) for t, _, m, _, d in sets]
     wav_hs = [torch.empty(B_PER_GPU, FRAMES * 300, dtype=torch.float32).pin_memory() for _ in range(max(depth, 1) + 1)]
     calls = [0, 0]
+    last_resident = [None]
     wav_lens_d = torch.full((B_PER_GPU,), FRAMES * 300, device=dev)
     gat = engine.WaveformGatherer(dev, [(B_PER_GPU, FRAMES * 300)] * world, torch.float32, dst=0) if world > 1 else None
 
     def step_resident():
         t, m, d = dev_sets[calls[0] % N_INPUT_SETS]
         calls[0] += 1
-        return syn.synthesize(t, tok_lens, m, mel_lens, d, predict_durations=True)
+        last_resident[0] = syn.synthesize(t, tok_lens, m, mel_lens, d, predict_durations=True)
+        return last_resident[0]
 
     def step_e2e():
         t, m, d = host_sets[calls[1] % N_INPUT_SETS]
@@ -608,7 +647,7 @@ def run_ours(args):
         return ms
 
     warm = max(args.warmup, 3)
-    for _ in range(max(warm, 2 * depth)):
+    for _ in range(warmup_calls(args.warmup, depth)):
         step_resident()
         step_e2e()
     barrier()
@@ -621,8 +660,16 @@ def run_ours(args):
     l0 = ops.launch_count
     ms = timed(step_resident, args.steps)
     launches = ops.launch_count - l0
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # the graphs' output buffers are reused by the next call with the same shapes: a device copy now, written to
+        # disk after the clock sampling window
+        dumped = [t.clone() for t in last_resident[0]]
     ms_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop() if sampler else None
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, *dumped)
+        del dumped
     assert syn.stats["captures"] == captures_after_warmup, "the timed region must replay graphs, not capture them"
 
     # BASELINE config 5 on every rank (strong scaling over the run's N GPUs)
@@ -834,7 +881,13 @@ def main():
                     help="batches in flight per GPU (2: the acoustic model of step i+1 overlaps the vocoder of step i)")
     ap.add_argument("--cpu-utts", type=int, default=16, help="utterances of the CPU baseline sample (~0.6 s each on 16 cores)")
     ap.add_argument("--skip-configs", action="store_true", help="headline + rooflines only (no config1/3/4/5 extras)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA arm's outputs (--impl ours)")
     # stdout carries exactly ONE line (the JSON): libraries that write to fd 1 (NCCL prints its version banner there
     # when NCCL_DEBUG is set) are sent to stderr for the whole run, the JSON line goes to the saved descriptor
     global _JSON_FD

@@ -1,7 +1,8 @@
 """TEST INFRASTRUCTURE — generate the committed fixtures under tests/golden from the *unmodified*
 reference (run in the build container, where /root/reference is mounted):
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden          # every fixture
+    python -m oracle.make_golden live     # tests/golden/live_reference.pt only
 
 Checkpoints are not stored: both sides rebuild them from a seed with
 ``artspeech_b200.checkpoint`` (the state-dict layout is identical to the reference's, which this
@@ -37,6 +38,34 @@ def make_inputs(seed, Tt, Tr, dur_spec):
         hi = int(dur_spec[-1])
         dur = torch.randint(1, hi + 1, (1, Tt), generator=g)
     return tok, mel, dur
+
+
+def live_inputs():
+    """Inputs of tests/test_oracle_pinning.py's live case (checkpoint seed 3)."""
+    g = torch.Generator().manual_seed(11)
+    tok = torch.randint(1, 178, (1, 23), generator=g)
+    mel = torch.randn(1, 80, 97, generator=g) * 0.5
+    return tok, mel
+
+
+def live_case():
+    """The reference's acoustic model on the live case's inputs (predicted durations), then the reference's vocoder
+    on the mel it produced -> tests/golden/live_reference.pt."""
+    os.makedirs(OUT, exist_ok=True)
+    dist = rl.load_distribution()
+    ours = checkpoint.build_random_artsspeech(3, dist)
+    ref = rl.build_reference_artsspeech(dist)
+    ref.load_state_dict(ours.state_dict(), strict=True)
+    tok, mel = live_inputs()
+    r = ref_runner.reference_test_step(ref, tok, mel)
+    refg = rl.build_reference_generator()
+    refg.remove_weight_norm()
+    refg.load_state_dict(checkpoint.build_random_generator(3).state_dict(), strict=True)
+    with torch.no_grad():
+        wav = refg(r["mel"])
+    torch.save(dict(checkpoint_seed=3, tokens=tok, ref_mel=mel, pred_dur=r["pred_dur"], mel=r["mel"], wav=wav),
+               os.path.join(OUT, "live_reference.pt"))
+    print("live case: mel", tuple(r["mel"].shape), "wav", tuple(wav.shape))
 
 
 def main():
@@ -97,8 +126,13 @@ def main():
             mas[key + "_path1"] = np.packbits(p1.astype(np.uint8), axis=None)
             mas[key + "_path2"] = np.packbits(p2.astype(np.uint8), axis=None)
     np.savez_compressed(os.path.join(OUT, "mas.npz"), **mas)
+    live_case()
     print("done:", os.listdir(OUT))
 
 
 if __name__ == "__main__":
-    main()
+    import sys
+    if sys.argv[1:] == ["live"]:
+        live_case()
+    else:
+        main()

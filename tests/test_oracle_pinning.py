@@ -1,5 +1,5 @@
 """Pin oracle/restate.py (the travelling CPU restatement) to the reference: against the committed
-fixtures everywhere, and against the unmodified reference modules where /root/reference exists."""
+fixtures everywhere, and against the unmodified reference modules where the original source tree is available."""
 import os
 
 import pytest
@@ -26,26 +26,37 @@ def test_restatement_matches_reference_goldens(case):
     assert (out - o["mel"]).abs().max().item() < 5e-5
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_loader.available(), reason="reference checkout not mounted")
+LIVE_GOLDEN = os.path.join(util.GOLDEN, "live_reference.pt")
+
+
+@pytest.mark.skipif(not (os.path.isfile(LIVE_GOLDEN) or ref_loader.available()),
+                    reason="needs the original ArtSpeech source tree, or tests/golden/live_reference.pt generated "
+                           "from it (python -m oracle.make_golden live)")
 def test_restatement_matches_live_reference():
+    """Checkpoint seed 3: the acoustic model, then the vocoder on the mel the reference's acoustic model produced,
+    against the reference's stored outputs, and against the reference itself where its source tree is available."""
     from artspeech_b200 import checkpoint
-    from oracle import ref_runner
-    dist = ref_loader.load_distribution()
-    ours = checkpoint.build_random_artsspeech(3, dist)
-    ref = ref_loader.build_reference_artsspeech(dist)
-    ref.load_state_dict(ours.state_dict(), strict=True)      # identical parameter tree
-    g = torch.Generator().manual_seed(11)
-    tok = torch.randint(1, 178, (1, 23), generator=g)
-    mel = torch.randn(1, 80, 97, generator=g) * 0.5
-    r = ref_runner.reference_test_step(ref, tok, mel)
-    out, aux = restate.artsspeech_test(ours.state_dict(), tok, mel, dist, want_aux=True)
-    assert torch.equal(aux["pred_dur"].view(-1), r["pred_dur"].view(-1))
-    assert (out - r["mel"]).abs().max().item() < 5e-5
+    from oracle import make_golden
+    ours = checkpoint.build_random_artsspeech(3)
     gen = checkpoint.build_random_generator(3)
-    refg = ref_loader.build_reference_generator()
-    refg.remove_weight_norm()
-    refg.load_state_dict(gen.state_dict(), strict=True)
-    with torch.no_grad():
-        w = refg(r["mel"])
-    assert (restate.generator_forward(gen.state_dict(), r["mel"]) - w).abs().max().item() < 1e-5
+    tok, mel = make_golden.live_inputs()
+    want = []                                              # the reference's (pred_dur, mel, wav)
+    if os.path.isfile(LIVE_GOLDEN):
+        g = util.load_golden("live_reference.pt")
+        assert g["checkpoint_seed"] == 3 and torch.equal(g["tokens"], tok) and torch.equal(g["ref_mel"], mel)
+        want.append((g["pred_dur"], g["mel"], g["wav"]))
+    if ref_loader.available():
+        from oracle import ref_runner
+        ref = ref_loader.build_reference_artsspeech(ref_loader.load_distribution())
+        ref.load_state_dict(ours.state_dict(), strict=True)      # identical parameter tree
+        r = ref_runner.reference_test_step(ref, tok, mel)
+        refg = ref_loader.build_reference_generator()
+        refg.remove_weight_norm()
+        refg.load_state_dict(gen.state_dict(), strict=True)
+        with torch.no_grad():
+            want.append((r["pred_dur"], r["mel"], refg(r["mel"])))
+    out, aux = restate.artsspeech_test(ours.state_dict(), tok, mel, checkpoint.default_distribution(), want_aux=True)
+    for pred_dur, ref_mel_out, ref_wav in want:
+        assert torch.equal(aux["pred_dur"].view(-1), pred_dur.view(-1))
+        assert (out - ref_mel_out).abs().max().item() < 5e-5
+        assert (restate.generator_forward(gen.state_dict(), ref_mel_out) - ref_wav).abs().max().item() < 1e-5

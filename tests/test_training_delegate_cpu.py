@@ -1,5 +1,6 @@
-"""SURVEY.md §8b: "training branches delegate to the original PyTorch code".  Needs the reference checkout (it IS
-the original code), so it runs where /root/reference is mounted and is skipped on the GPU box."""
+"""SURVEY.md §8b: "training branches delegate to the original PyTorch code".  Running the original code needs the
+original source tree (ARTSPEECH_REFERENCE); without a delegate, and when attaching one, the module is checked
+everywhere."""
 import random
 
 import numpy as np
@@ -9,8 +10,25 @@ import torch
 from oracle import ref_loader
 
 
+def test_training_steps_need_a_delegate_that_shares_the_parameters():
+    from artspeech_b200 import checkpoint
+    ours = checkpoint.build_random_artsspeech(4)
+    keys_before = list(ours.state_dict().keys())
+    for step in ("first", "second"):
+        with pytest.raises(NotImplementedError):
+            ours([None] * 7, None, None, step=step)
+    # a module with the reference's parameter tree (our own class has the same state_dict layout)
+    stand_in = checkpoint.build_random_artsspeech(5)
+    ours.attach_training_delegate(stand_in)
+    assert list(ours.state_dict().keys()) == keys_before                       # the delegate is not a sub-module
+    own = dict(ours.named_parameters())
+    assert all(p is own[n] for n, p in stand_in.named_parameters())             # every parameter is the same object
+    own_b = dict(ours.named_buffers())
+    assert all(b is own_b[n] for n, b in stand_in.named_buffers() if n in own_b)
+
+
 @pytest.mark.reference
-@pytest.mark.skipif(not ref_loader.available(), reason="reference checkout not mounted")
+@pytest.mark.skipif(not ref_loader.available(), reason="needs the original ArtSpeech source tree")
 def test_training_steps_run_the_reference_code_on_shared_parameters():
     from artspeech_b200 import checkpoint
     dist = ref_loader.load_distribution()
