@@ -115,6 +115,9 @@ SIGNATURES.update({
     "as_repeat_rows": (C.c_int, [_V, _I, _L, _I, _I, _I, _I, _V, _V, _I, _L, _V]),
     "as_length_regulate": (C.c_int, [_V, _I, _L, _I, _I, _I, _V, _V, _I, _I, _V, _I, _L, _V, _V]),
     "as_round_durations": (C.c_int, [_V, _L, _I, _I, _V, _V, _V, _V]),
+    "as_round_durations_scaled": (C.c_int, [_V, _L, _I, _I, _V, _V, _L, _V, _V, _V]),
+    "as_prosody_apply": (C.c_int, [_V, _L, _V, _L, _V, _L, _I, _I, _V, _V, C.c_double, C.c_double, C.c_double,
+                                   _V]),
     "as_conv_small": (C.c_int, [_V, _I, _L, _I, _I, _I, _I, _V, _V, _I, c_i32_p, c_i32_p, _I, _V,
                                 _V, _I, _L, _V, _I, _L, _I, _F, _V]),
     "as_dwconv": (C.c_int, [_V, _I, _L, _I, _I, _I, _I, _I, _V, _V, _I, _I, _I, _I, _I, _I, _I, _I,

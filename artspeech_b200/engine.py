@@ -18,6 +18,7 @@ from typing import List, Optional, Sequence
 import torch
 
 from . import _lib, nn_util, ops
+from . import prosody as prosody_mod
 
 SAMPLE_RATE = 24000
 HOP = 300
@@ -30,11 +31,12 @@ def _ceil_to(v: int, q: int) -> int:
 class _Captured:
     """One captured CUDA graph with its static inputs / outputs (all owned by the graph's memory pool)."""
     __slots__ = ("graph", "tok", "mels", "voice", "meta", "dur", "lens_t", "mel_lens", "pin_meta", "pin_free", "out",
-                 "launches", "state", "uid")
+                 "launches", "state", "uid", "pros", "pin_pros", "ctrl", "dscale")
 
     def __init__(self):
         self.graph = self.tok = self.mels = self.voice = self.meta = self.dur = self.lens_t = self.mel_lens = None
         self.pin_meta = self.pin_free = self.out = self.state = None
+        self.pros = self.pin_pros = self.ctrl = self.dscale = None
         self.launches = 0
         self.uid = 0
 
@@ -85,7 +87,13 @@ class Synthesizer:
     are views of the graph's static output buffers -- they stay valid until the next call that lands in the same
     slot *and* bucket; enqueue the copy that consumes them (on ``last_stream``) before making that call.
     ``pcm16=True`` returns int16 samples (``rint(32767 * wav)``, the on-disk format of ``soundfile.write`` at
-    test.py:119) written directly by the vocoder's last kernel: half the device->host bytes per utterance."""
+    test.py:119) written directly by the vocoder's last kernel: half the device->host bytes per utterance.
+
+    **Prosody.**  ``synthesize(..., prosody=[Prosody, ...])`` (one per utterance, ``artspeech_b200.prosody``) scales
+    the predicted durations and edits the predicted F0 / energy / EMA tracks.  The controls are graph inputs like the
+    durations (a control block and a per-token duration scale staged through one pinned buffer), so one graph serves
+    controls that change on every call.  Controlled calls have graphs of their own (one extra launch); calls
+    without ``prosody`` replay the same graphs as before."""
 
     def __init__(self, model, generator, device="cuda:0", use_cuda_graph: bool = True, pipeline_depth: int = 1,
                  pcm16: bool = False, acoustic_sms: Optional[int] = None, token_quantum: int = 32,
@@ -109,6 +117,7 @@ class Synthesizer:
         self.last = {}
         self.model = model.to(self.device).eval()
         self.model.distribution = {k: v.to(self.device) for k, v in self.model.distribution.items()}
+        self.model.prosody_constants()          # host floats of the pitch / energy statistics: read once, here
         self.generator = generator.to(self.device).eval()
         self.use_cuda_graph = use_cuda_graph
         self._graphs = [OrderedDict() for _ in range(self.pipeline_depth)]     # per slot: key -> _Captured (LRU)
@@ -151,21 +160,21 @@ class Synthesizer:
         if self.acoustic_sms and self.pipeline_depth > 1:
             _lib.load().as_set_sm_limit(n)
 
-    def _phase_a(self, tok, lens_t, mels, mel_lens_dev, host_mel_lens, voice, predict):
+    def _phase_a(self, tok, lens_t, mels, mel_lens_dev, host_mel_lens, voice, predict, dscale=None):
         self._sm_limit(self.acoustic_sms)
         try:
             with self._nvtx("asb.encode (text / arts / style encoders, duration predictor)"):
-                return self.model.encode(tok, lens_t, mels, mel_lens_dev, host_mel_lens, voice, predict)
+                return self.model.encode(tok, lens_t, mels, mel_lens_dev, host_mel_lens, voice, predict, dscale)
         finally:
             self._sm_limit(0)
 
-    def _phase_b(self, st, dur, Lmax):
+    def _phase_b(self, st, dur, Lmax, ctrl=None):
         total = torch.cuda.get_device_properties(self.device).multi_processor_count
         gen = self.generator
         try:
             self._sm_limit(self.acoustic_sms)
             with self._nvtx("asb.decode (length regulator, F0/N/EMA predictors, mel decoder)"):
-                mel_cl, aux = self.model.decode(st, dur, Lmax, mel16_dtype=gen.compute_dtype)
+                mel_cl, aux = self.model.decode(st, dur, Lmax, mel16_dtype=gen.compute_dtype, ctrl=ctrl)
             self._sm_limit(max(2, total - self.acoustic_sms))
             with self._nvtx("asb.vocoder (HiFi-GAN generator)"):
                 wav = gen.forward_channels_last(aux["mel16"], aux["mel_lengths"],
@@ -176,7 +185,7 @@ class Synthesizer:
         return dict(wav=wav.view(wav.shape[0], -1), mel_lengths=aux["mel_lengths"], mel=mel,
                     duration=st["duration"], pred_dur=st["pred_dur"])
 
-    def _eager(self, tokens, tl, mels, ml, durations, voice, predict):
+    def _eager(self, tokens, tl, mels, ml, durations, voice, predict, pros=None):
         """No graph: ragged reference mels, ``use_cuda_graph=False`` or a bucket not captured yet."""
         dev = self.device
         self.stats["eager"] += 1
@@ -184,14 +193,19 @@ class Synthesizer:
         mels = mels.to(dev, non_blocking=True)
         lens_t = torch.tensor(tl, dtype=torch.int32).to(dev, non_blocking=True)
         mel_lens_dev = torch.tensor(ml, dtype=torch.int64).to(dev, non_blocking=True)
-        st = self._phase_a(tokens, lens_t, mels, mel_lens_dev, ml, voice, predict or durations is None)
+        ctrl = dscale = None
+        if pros is not None:
+            ctrl, dscale = (t.to(dev) for t in prosody_mod.pack(pros, tokens.shape[1]))
+            if durations is not None:
+                dscale = None
+        st = self._phase_a(tokens, lens_t, mels, mel_lens_dev, ml, voice, predict or durations is None, dscale)
         if durations is None:
             dur = st["pred_dur"]
             sums = [int(v) for v in st["pred_sum"].tolist()]                       # the one host sync
         else:
             dur = durations.to(torch.int32).to(dev, non_blocking=True).contiguous()
             sums = [int(durations[b, :tl[b]].sum()) for b in range(len(tl))]
-        out = self._phase_b(st, dur, max(sums))
+        out = self._phase_b(st, dur, max(sums), ctrl)
         self.last = dict(out, frames=[2 * v for v in sums], graph=False)
         return out["wav"], out["mel_lengths"], out["mel"]
 
@@ -247,7 +261,7 @@ class Synthesizer:
         self._epoch = nn_util.plan_epoch()          # the warm-up pass may have packed weights for the first time
         return g, out, ops.launch_count - before
 
-    def _static_inputs(self, B, Tt_b, mels, voice):
+    def _static_inputs(self, B, Tt_b, mels, voice, controlled):
         dev = self.device
         ent = _Captured()
         self._uid += 1
@@ -262,11 +276,20 @@ class Synthesizer:
         ent.lens_t = ent.meta[B * Tt_b:]
         ent.pin_meta = torch.zeros(B * Tt_b + B, dtype=torch.int32).pin_memory()
         ent.pin_free = torch.cuda.Event()
+        if controlled:
+            # prosody controls: [B, 24] control block + [B, Tt_b] duration scale, identity for the warm-up pass
+            W = prosody_mod.CTRL_WIDTH
+            ent.pros = torch.ones(B * W + B * Tt_b, dtype=torch.float32, device=dev)
+            ent.ctrl = ent.pros[:B * W].view(B, W)
+            ent.ctrl.copy_(torch.tensor(prosody_mod.Prosody().ctrl_row()).expand(B, W))
+            ent.dscale = ent.pros[B * W:].view(B, Tt_b)
+            ent.pin_pros = torch.zeros(B * W + B * Tt_b, dtype=torch.float32).pin_memory()
         return ent
 
-    def _stage(self, ent, tokens, tl, mels, durations, voice, run_stream):
+    def _stage(self, ent, tokens, tl, mels, durations, voice, run_stream, pros=None):
         """Refresh the graph's inputs (on ``run_stream``): tokens, reference mels / voice, and -- through ONE pinned
-        staging buffer -- the zero-padded durations and the token lengths."""
+        staging buffer -- the zero-padded durations and the token lengths (and through a second one, released by the
+        same event, the prosody controls of a controlled graph)."""
         B, Tt_b = ent.tok.shape
         Tt = tokens.shape[1]
         ent.pin_free.synchronize()                      # the previous replay's copy has read the staging buffer
@@ -280,6 +303,12 @@ class Synthesizer:
             ent.meta.copy_(pm, non_blocking=True)
         else:
             ent.lens_t.copy_(pm[B * Tt_b:], non_blocking=True)
+        if ent.pros is not None:
+            ctrl, dscale = prosody_mod.pack(pros, Tt_b)
+            W = prosody_mod.CTRL_WIDTH
+            ent.pin_pros[:B * W].view(B, W).copy_(ctrl)
+            ent.pin_pros[B * W:].view(B, Tt_b).copy_(dscale)
+            ent.pros.copy_(ent.pin_pros, non_blocking=True)
         ent.pin_free.record(run_stream)
         ent.tok[:, :Tt].copy_(tokens, non_blocking=True)
         if Tt < Tt_b:
@@ -293,7 +322,7 @@ class Synthesizer:
     # ---------------------------------------------------------------------------------------
     @torch.no_grad()
     def synthesize(self, tokens, tok_lens, mels, mel_lens, durations=None, voice=None, predict_durations: bool = False,
-                   exact_frames: bool = False, defer: bool = False):
+                   exact_frames: bool = False, defer: bool = False, prosody=None):
         """``tokens`` int64 [B,Tt] and ``mels`` fp32 [B,80,Tr]: device tensors or (pinned) HOST tensors -- host inputs
         are copied straight into the graph's static buffers; ``tok_lens`` / ``mel_lens`` int64 [B] HOST tensors (or
         lists); ``durations`` int64 [B,Tt] HOST tensor or None (predict them, one device->host sync of B integers);
@@ -305,7 +334,9 @@ class Synthesizer:
         forces the two-graph path with the frame-count read-back).
         ``defer=True`` returns a ticket instead of the result; ``finish(ticket)`` completes the call.  With predicted
         durations the ticket is handed out BEFORE the host waits for the frame counts, so a caller can issue the next
-        call's graph A first (``synthesize_many`` does): the GPU then always has work queued while the host wakes up."""
+        call's graph A first (``synthesize_many`` does): the GPU then always has work queued while the host wakes up.
+        ``prosody``: one ``prosody.Prosody`` per utterance (``ValueError`` for a ``duration_scale`` other than 1 when
+        ``durations`` are given); ``last["pred_dur"]`` then holds the scaled durations."""
         dev = self.device
         cur = torch.cuda.current_stream(dev)
         self.last_stream = cur
@@ -317,6 +348,8 @@ class Synthesizer:
         ml = [int(v) for v in (mel_lens.tolist() if torch.is_tensor(mel_lens) else mel_lens)]
         B, Tt = tokens.shape
         Tr = mels.shape[2]
+        pros = prosody_mod.check(prosody, tl, durations is not None)
+        controlled = pros is not None
         predict = bool(predict_durations) or durations is None
         Tt_b = _ceil_to(Tt, self.token_quantum)
         sums = None
@@ -326,16 +359,16 @@ class Synthesizer:
         bounded = durations is None and self.duration_bound is not None and not exact_frames
         if bounded:
             L_bound = _ceil_to(int(-(-Tt_b * self.duration_bound // 1)), self.frame_quantum)
-            key_a = ("abp", voice is not None, B, Tt_b, Tr, True, L_bound)
+            key_a = ("abp", voice is not None, controlled, B, Tt_b, Tr, True, L_bound)
         else:
-            key_a = ("ab" if durations is not None else "a", voice is not None, B, Tt_b, Tr, predict,
+            key_a = ("ab" if durations is not None else "a", voice is not None, controlled, B, Tt_b, Tr, predict,
                      _ceil_to(max(sums), self.frame_quantum) if sums is not None else 0)
         if graphable:
             n = self._seen.get(key_a, 0) + 1
             self._seen[key_a] = n
             graphable = n >= self.capture_after
         if not graphable:
-            res = self._eager(tokens, tl, mels, ml, durations, voice, predict)
+            res = self._eager(tokens, tl, mels, ml, durations, voice, predict, pros)
             return self._done_ticket(res) if defer else res
         if self._epoch != nn_util.plan_epoch():
             self.drop_graphs()
@@ -350,7 +383,7 @@ class Synthesizer:
 
         ent = self._lookup(slot, key_a)
         if ent is None:
-            ent = self._static_inputs(B, Tt_b, mels, voice)
+            ent = self._static_inputs(B, Tt_b, mels, voice, controlled)
             mel_lens_dev = torch.full((B,), Tr, dtype=torch.int64, device=dev)
             ent.mel_lens = mel_lens_dev                 # a graph input like the others: lives as long as the graph
             if durations is not None:
@@ -358,18 +391,18 @@ class Synthesizer:
 
                 def fn(ent=ent):
                     st = self._phase_a(ent.tok, ent.lens_t, ent.mels, mel_lens_dev, ml, ent.voice, predict)
-                    return self._phase_b(st, ent.dur, L_b)
+                    return self._phase_b(st, ent.dur, L_b, ent.ctrl)
             elif bounded:
                 L_b = key_a[-1]
 
                 def fn(ent=ent):
-                    st = self._phase_a(ent.tok, ent.lens_t, ent.mels, mel_lens_dev, ml, ent.voice, True)
-                    out = self._phase_b(st, st["pred_dur"], L_b)
+                    st = self._phase_a(ent.tok, ent.lens_t, ent.mels, mel_lens_dev, ml, ent.voice, True, ent.dscale)
+                    out = self._phase_b(st, st["pred_dur"], L_b, ent.ctrl)
                     out["pred_sum"] = st["pred_sum"]
                     return out
             else:
                 def fn(ent=ent):
-                    return self._phase_a(ent.tok, ent.lens_t, ent.mels, mel_lens_dev, ml, ent.voice, True)
+                    return self._phase_a(ent.tok, ent.lens_t, ent.mels, mel_lens_dev, ml, ent.voice, True, ent.dscale)
             ent.graph, ent.out, ent.launches = self._capture(slot, fn)
             if durations is None and not bounded:
                 ent.state = ent.out
@@ -388,7 +421,7 @@ class Synthesizer:
                     t.record_stream(run_stream)
         launches = ent.launches
         with torch.cuda.stream(run_stream):
-            self._stage(ent, tokens, tl, mels, durations, voice, run_stream)
+            self._stage(ent, tokens, tl, mels, durations, voice, run_stream, pros)
             ent.graph.replay()
             if durations is None and not bounded:
                 # the only device->host hand-off of the pass: B frame counts (the other slot keeps the GPU busy)
@@ -441,7 +474,9 @@ class Synthesizer:
                 eb = _Captured()
                 eb.state = ent
                 st = ent.state
-                eb.graph, eb.out, eb.launches = self._capture(slot, lambda: self._phase_b(st, st["pred_dur"], L_b))
+                # the control block of the A entry: staged with this call's graph A, in the same slot
+                eb.graph, eb.out, eb.launches = self._capture(
+                    slot, lambda: self._phase_b(st, st["pred_dur"], L_b, ent.ctrl))
                 self._insert(slot, key_b, eb)
             eb.graph.replay()
             out = eb.out
@@ -567,7 +602,7 @@ class HostArena:
 def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels: Sequence[torch.Tensor],
                     durations: Optional[Sequence[torch.Tensor]] = None, max_batch: int = 16,
                     max_padded_frames: Optional[int] = 25600, to_host: bool = False, arena: Optional[HostArena] = None,
-                    frames_per_token: float = 5.34):
+                    frames_per_token: float = 5.34, prosody: Optional[Sequence["prosody_mod.Prosody"]] = None):
     """Mixed-length utterances through ``syn`` in length-bucketed ragged micro-batches (BASELINE config 5).
 
     ``tokens[i]`` int64 [Tt_i], ``ref_mels[i]`` fp32 [80, Tr_i], ``durations[i]`` int64 [Tt_i] (host tensors) or
@@ -576,12 +611,16 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     bounded set of CUDA graphs.  Returns ``(wavs, frames)``: ``wavs[i]`` holds the ``300 * frames[i]`` samples of
     utterance ``i`` (fp32, or int16 when ``syn.pcm16``), independent of what it was batched with (batch-1
     semantics) -- device tensors, or views of the pinned ``arena`` when ``to_host`` (valid after this function
-    returns: it synchronises the copies)."""
+    returns: it synchronises the copies).  ``prosody``: one ``prosody.Prosody`` per utterance (or None); the planning
+    estimate of an utterance then grows with its mean ``duration_scale``."""
     n = len(tokens)
+    pros = prosody_mod.check(prosody, [int(t.shape[0]) for t in tokens], durations is not None)
     if durations is not None:
         plan_frames = [2 * int(d.sum()) for d in durations]
     else:
-        plan_frames = [int(round(frames_per_token * int(t.shape[0]))) for t in tokens]
+        plan_frames = [int(round(frames_per_token * int(t.shape[0]) *
+                                 (pros[i].mean_duration_scale(int(t.shape[0])) if pros else 1.0)))
+                       for i, t in enumerate(tokens)]
     frames: List[int] = list(plan_frames)
     wavs: List[Optional[torch.Tensor]] = [None] * n
     dt = torch.int16 if syn.pcm16 else torch.float32
@@ -631,7 +670,8 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
             mel[j, :, :ref_mels[i].shape[1]] = ref_mels[i]
         tl = [int(tokens[i].shape[0]) for i in idx]
         ml = [int(ref_mels[i].shape[1]) for i in idx]
-        waiting.append((idx, syn.synthesize(tok, tl, mel, ml, dur, defer=True)))
+        waiting.append((idx, syn.synthesize(tok, tl, mel, ml, dur, defer=True,
+                                            prosody=[pros[i] for i in idx] if pros else None)))
         while len(waiting) > lookahead:
             collect(*waiting.pop(0))
         pending.append((tok, mel))            # pinned inputs must outlive their asynchronous copies
@@ -649,7 +689,8 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
                 redo.append(i)
     for i in redo:                                         # rare: exact two-graph pass for the utterances that overflowed
         w, _, _ = syn.synthesize(tokens[i].view(1, -1).pin_memory(), [int(tokens[i].shape[0])],
-                                 ref_mels[i].unsqueeze(0).pin_memory(), [int(ref_mels[i].shape[1])], None, exact_frames=True)
+                                 ref_mels[i].unsqueeze(0).pin_memory(), [int(ref_mels[i].shape[1])], None, exact_frames=True,
+                                 prosody=[pros[i]] if pros else None)
         frames[i] = syn.last["frames"][0]
         with torch.cuda.stream(syn.last_stream):
             wavs[i] = w[0, :HOP * frames[i]].clone() if not to_host else w[0, :HOP * frames[i]].to("cpu")

@@ -23,6 +23,7 @@ import torch.nn as nn
 from torch.nn.utils import spectral_norm, weight_norm
 
 from . import nn_util, ops
+from . import prosody as prosody_mod
 from .blocks import (AdainResBlk1d, LRELU, Placeholder, ResBlk, ResBlk1d, StyleFC, run_adain_block, run_resblk1d,
                      run_resblk2d)
 from .ema import EMA_Predictor
@@ -544,9 +545,10 @@ class ArtsSpeech(nn.Module):
     # -- phase A: everything that does not depend on the durations -------------------------------------------
     @torch.no_grad()
     def encode(self, texts, lens_t, mels, mel_input_length, host_mel_lens=None, voice=None,
-               predict_durations: bool = True):
+               predict_durations: bool = True, dscale: Optional[torch.Tensor] = None):
         """Text / arts / style encoders (models.py:357-359) and, when ``predict_durations``, the duration
         predictor with its device-side ``round().clamp(min=1)`` (:360-361).  ``lens_t`` int32 [B] on the device.
+        ``dscale``: prosody duration scale fp32 [B,Tt] on the device, rounds ``duration * dscale`` instead.
         Returns the state ``decode`` consumes; no host synchronisation when ``host_mel_lens`` is given."""
         dev = texts.device
         dp = self.durationPredictor
@@ -569,16 +571,21 @@ class ArtsSpeech(nn.Module):
         if predict_durations:
             duration = dp(texts, ema_ext, lens_t, mel_input_length, host_mel_lengths=host_mel_lens, d_text=res[2])
             st["duration"] = duration                                                             # (:360)
-            st["pred_dur"], st["pred_sum"] = ops.round_durations(duration, lens_t)                # (:361) on the device
+            if dscale is None:
+                st["pred_dur"], st["pred_sum"] = ops.round_durations(duration, lens_t)            # (:361) on the device
+            else:
+                st["pred_dur"], st["pred_sum"] = ops.round_durations(duration, lens_t, dscale)
         return st
 
     # -- phase B: length regulation -> predictors -> decoder -------------------------------------------------
     @torch.no_grad()
-    def decode(self, st, dur, Lmax: int, mel16_dtype=None):
+    def decode(self, st, dur, Lmax: int, mel16_dtype=None, ctrl: Optional[torch.Tensor] = None):
         """``dur`` int32 [B,Tt] on the device (zeros or anything beyond ``lens_t``: the regulator reads
         ``dur[b, :lens_t[b]]`` only), ``Lmax`` >= max_b sum(dur[b]) (host int; a shape bucket may round it up: the
         extra rows come back as zeros).  Returns (mel_cl fp32 [B,2*Lmax,80], aux); ``mel16_dtype`` adds
-        ``aux["mel16"]``, the 16-bit channels-last copy the vocoder consumes."""
+        ``aux["mel16"]``, the 16-bit channels-last copy the vocoder consumes.  ``ctrl``: prosody control block fp32
+        [B,24] on the device (``prosody.pack``): the F0 / energy / EMA tracks are edited before the decoder reads
+        them."""
         dev, dt = dur.device, self.compute_dtype
         T_en, A_en, lens_t = st["T_en"], st["A_en"], st["lens_t"]
         B = T_en.shape[0]
@@ -593,6 +600,8 @@ class ArtsSpeech(nn.Module):
         if cat16 is not cat_res:
             ops.length_regulate(T_en, dur, lens_t, 2, Tm, out=cat16[..., :D])
         f0, n, ema, _ = self.artsPredictor.forward_cl(a_reg, style16, lens_l, lens_up=lens_m)    # (:369)
+        if ctrl is not None:
+            ops.prosody_apply(f0, n, ema, lens_m, ctrl, *self.prosody_constants())
         mel_cl = self.decoder.forward_cl(cat_res, cat16, style16, f0, n, ema, lens_m, mel16_dtype)   # (:370)
         mel16 = None
         if mel16_dtype is not None:
@@ -602,7 +611,7 @@ class ArtsSpeech(nn.Module):
     @torch.no_grad()
     def forward(self, batch, s2s_attn=None, s2s_attn_mono=None, step="test", mode="train", epoch=0,
                 durations: Optional[torch.Tensor] = None, return_aux: bool = False, host_meta: Optional[dict] = None,
-                voice: Optional[tuple] = None, predict_durations: Optional[bool] = None):
+                voice: Optional[tuple] = None, predict_durations: Optional[bool] = None, prosody=None):
         """``step="test"`` (models.py:356-371).  ``durations`` (extension): integer durations [B,Tt] used INSTEAD of
         the predictor's (north_star: "durations are fed from the reference's integer output"); the predictor then
         runs only if ``predict_durations`` is true (its output is returned in the aux dict, the forced durations
@@ -612,6 +621,9 @@ class ArtsSpeech(nn.Module):
         ``sum(durations[b, :len_b])``; ``Lmax`` requires ``durations``.
         ``voice`` (optional): ``(f0, n, ema, Style)`` as returned by the style encoder for these utterances'
         reference recordings; skips the style encoder (``mels`` is then only used for its shape).
+        ``prosody`` (optional): one ``prosody.Prosody`` per utterance; with ``return_aux`` the aux dict then holds
+        the edited ``F0`` / ``N`` / ``EMA`` tracks and the scaled ``pred_dur`` (``duration`` stays the predictor's
+        raw output).
         Training branches (``step != "test"``) are delegated to ``self.training_delegate`` (an instance of the
         reference's own ``ArtsSpeech`` sharing this module's parameters, see ``attach_training_delegate``)."""
         if step != "test":
@@ -629,7 +641,13 @@ class ArtsSpeech(nn.Module):
         lens_t = _i32(input_lengths, dev)
         hm = host_meta or {}
         predict = durations is None if predict_durations is None else (bool(predict_durations) or durations is None)
-        st = self.encode(texts, lens_t, mels, mel_input_length, hm.get("mel_lens"), voice, predict)
+        ctrl = dscale = None
+        if prosody is not None:
+            tl = [int(v) for v in (input_lengths.tolist() if torch.is_tensor(input_lengths) else input_lengths)]
+            pros = prosody_mod.check(prosody, tl, durations is not None)
+            ctrl, dscale = (t.to(dev) for t in prosody_mod.pack(pros, Tt))
+        st = self.encode(texts, lens_t, mels, mel_input_length, hm.get("mel_lens"), voice, predict,
+                         dscale if durations is None else None)
         if durations is None:
             dur = st["pred_dur"]
             Lmax = int(st["pred_sum"].max().item())                                       # one host sync (ref: 2*Tt+1)
@@ -644,7 +662,7 @@ class ArtsSpeech(nn.Module):
             else:
                 valid = torch.arange(Tt, device=dev)[None, :] < lens_t[:, None]
                 Lmax = int((dur * valid).sum(dim=1).max().item())
-        mel_cl, aux = self.decode(st, dur, Lmax)
+        mel_cl, aux = self.decode(st, dur, Lmax, ctrl=ctrl)
         mel = ops.to_channels_first(mel_cl, torch.float32)                               # [B,80,Tm]
         if return_aux:
             aux.update(pred_dur=pred_dur, duration=st["duration"], predicted_dur=st["pred_dur"], style=st["style"],
@@ -674,6 +692,15 @@ class ArtsSpeech(nn.Module):
                     mod._buffers[k] = own_b[full]
         object.__setattr__(self, "training_delegate", ref_module)     # not a sub-module: keeps state_dict unchanged
         return self
+
+    def prosody_constants(self):
+        """(pitch_mean, pitch_std, energy_std) of ``self.distribution`` as host floats, read once per distribution
+        (``as_prosody_apply`` takes them by value; reading a device tensor per call would synchronise)."""
+        cached = getattr(self, "_prosody_consts", None)
+        if cached is None or cached[0] is not self.distribution:
+            cached = (self.distribution, prosody_mod.constants(self.distribution))
+            self._prosody_consts = cached
+        return cached[1]
 
     def invalidate_plans(self):
         for m in self.modules():

@@ -380,18 +380,47 @@ def length_regulate(x, dur, lens_t, rep, To, out=None, out_dtype=None):
     return out, olens
 
 
-def round_durations(pred, lens_t):
+def round_durations(pred, lens_t, scale=None):
     """``pred`` fp32 [B,Tt] (the duration predictor's output) -> (dur int32 [B,Tt] = ``round(pred).clamp(min=1)``
-    for ``t < lens_t[b]`` and 0 beyond, sums int32 [B]); models.py:361 on the device."""
+    for ``t < lens_t[b]`` and 0 beyond, sums int32 [B]); models.py:361 on the device.  ``scale`` (prosody
+    ``duration_scale``): fp32 [B,Tt'] with Tt' >= Tt, or [B] (one value per utterance); rounds ``pred * scale``."""
     _require_cuda(pred, "round_durations")
     B, Tt = pred.shape
     if pred.stride(1) != 1:
         pred = pred.contiguous()
     dur = torch.empty(B, Tt, dtype=torch.int32, device=pred.device)
     sums = torch.empty(B, dtype=torch.int32, device=pred.device)
-    _run("as_round_durations", pred, pred.data_ptr(), pred.stride(0), B, Tt, _p(_i32(lens_t, "round_durations")),
-         dur.data_ptr(), sums.data_ptr())
+    lens_t = _i32(lens_t, "round_durations")
+    if scale is None:
+        _run("as_round_durations", pred, pred.data_ptr(), pred.stride(0), B, Tt, _p(lens_t), dur.data_ptr(),
+             sums.data_ptr())
+        return dur, sums
+    if scale.dtype != torch.float32 or scale.device != pred.device or scale.shape[0] != B or scale.dim() > 2 or \
+            (scale.dim() == 2 and (scale.shape[1] < Tt or scale.stride(1) != 1)):
+        raise _lib.AsError(f"round_durations: scale must be fp32 [B] or [B, >= Tt] on {pred.device}, got "
+                           f"{scale.dtype} {tuple(scale.shape)} on {scale.device}")
+    if scale.dim() == 1 and scale.stride(0) != 1:
+        scale = scale.contiguous()
+    _run("as_round_durations_scaled", pred, pred.data_ptr(), pred.stride(0), B, Tt, _p(lens_t), scale.data_ptr(),
+         scale.stride(0) if scale.dim() == 2 else 0, dur.data_ptr(), sums.data_ptr())
     return dur, sums
+
+
+def prosody_apply(f0, n, ema, lens, ctrl, pitch_mean: float, pitch_std: float, energy_std: float):
+    """Prosody edits of the arts predictor's tracks, in place (``as_prosody_apply``; semantics in
+    ``artspeech_b200.prosody``): ``f0`` / ``n`` fp32 [B,Tm,1], ``ema`` fp32 [B,Tm,10] channels-last, ``lens`` int32
+    [B] valid frames, ``ctrl`` fp32 [B,24] (``prosody.pack``).  The pitch / energy statistics are host floats."""
+    _require_cuda(f0, "prosody_apply")
+    B, Tm, _ = f0.shape
+    for t, name, ch in ((f0, "f0", 1), (n, "n", 1), (ema, "ema", 10)):
+        if t.dtype != torch.float32 or t.device != f0.device or tuple(t.shape) != (B, Tm, ch):
+            raise _lib.AsError(f"prosody_apply: {name} must be fp32 [{B}, {Tm}, {ch}], got {t.dtype} {tuple(t.shape)}")
+    if ctrl.dtype != torch.float32 or tuple(ctrl.shape) != (B, 24) or ctrl.stride() != (24, 1) or \
+            ctrl.device != f0.device:
+        raise _lib.AsError(f"prosody_apply: ctrl must be a dense fp32 [{B}, 24] device tensor")
+    _run("as_prosody_apply", f0, f0.data_ptr(), _rows_ld(f0, "prosody.f0"), n.data_ptr(), _rows_ld(n, "prosody.n"),
+         ema.data_ptr(), _rows_ld(ema, "prosody.ema"), B, Tm, _p(_i32(lens, "prosody_apply")), ctrl.data_ptr(),
+         float(pitch_mean), float(pitch_std), float(energy_std))
 
 
 @dataclass

@@ -263,6 +263,26 @@ int as_length_regulate(const void* x, int32_t x_dtype, int64_t x_ld, int32_t B, 
 int as_round_durations(const float* pred, int64_t pred_ld, int32_t B, int32_t Tt, const int32_t* lens_t,
                        int32_t* dur, int32_t* sum, void* stream);
 
+/* as_round_durations with a speaking-rate scale (prosody duration_scale): dur[b,t] = max(1, rint(pred[b,t] * s)),
+ * s = scale[b * scale_ld + t] fp32, or scale[b] (one value per utterance) when scale_ld == 0.  A scale of 1 gives
+ * the bits of as_round_durations. */
+int as_round_durations_scaled(const float* pred, int64_t pred_ld, int32_t B, int32_t Tt, const int32_t* lens_t,
+                              const float* scale, int64_t scale_ld, int32_t* dur, int32_t* sum, void* stream);
+
+/* Per-utterance prosody edits of the arts predictor's tracks (models.py:369), in place, frames t < lens[b] only:
+ *   F0  fp32 [B,Tm,1] (z-normalised, hz = f0 * pitch_std + pitch_mean): on voiced frames (hz >= 50 Hz)
+ *       hz' = exp(mu + range * (ln hz - mu) + shift * ln2 / 12), f0' = f0 + (hz' - hz) / pitch_std, mu = mean of
+ *       ln hz over the utterance's voiced frames (no voiced frame: F0 unchanged);
+ *   N   fp32 [B,Tm,1] (log-norm energy): n' = n + dB * ln10 / 10 / energy_std;
+ *   EMA fp32 [B,Tm,10]: e' = m_c + scale_c * (e - m_c) + offset_c, m_c = channel mean over the valid frames.
+ * ctrl fp32 [B, AS_PROSODY_CTRL] = {shift, range, dB, 0, scale[10], offset[10]}; *_ld are row strides (elements
+ * per frame) of dense [B,Tm,*] buffers.  A track whose controls are identity is not written.  One CTA per
+ * utterance with a fixed reduction order: an utterance's result does not depend on B, Tm or its batch-mates. */
+#define AS_PROSODY_CTRL 24
+int as_prosody_apply(float* f0, int64_t f0_ld, float* n, int64_t n_ld, float* ema, int64_t ema_ld, int32_t B,
+                     int32_t Tm, const int32_t* lens, const float* ctrl, double pitch_mean, double pitch_std,
+                     double energy_std, void* stream);
+
 /* Direct convolution for tiny input-channel counts (Cin <= 16) on CUDA cores: first layers of the
  * 2-D stacks (1 -> 64, 3x3), F0/N/EMA 1x1 convs of the decoder (models.py:480-482, 502-504).
  * x [B,T,F,Cin]; w fp32 [ntaps][Cout][Cin]; taps host arrays; stride 1; zero padding; outputs as
