@@ -132,4 +132,6 @@ SIGNATURES.update({
     "as_transpose_cast": (C.c_int, [_V, _I, _V, _I, _I, _I, _I, _L, _I, _V, _V, _V, _V]),
     "as_mas_align": (C.c_int, [_V, _V, _V, _V, _V, _V, _I, _I, _I, _I, _V, C.c_size_t, _V]),
     "as_expand_tokens": (C.c_int, [_V, _V, _V, _I, _I, _I, _I, _V]),
+    "as_resample_smem_bytes": (C.c_size_t, [_I, _I, _I, _I]),
+    "as_resample_encode": (C.c_int, [_V, _L, _I, _I, _V, _V, _I, _I, _I, _I, _I, _I, _I, _V, _L, _I, _V, _V]),
 })

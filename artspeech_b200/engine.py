@@ -18,6 +18,7 @@ from typing import List, Optional, Sequence
 import torch
 
 from . import _lib, nn_util, ops
+from . import audio as audio_mod
 from . import prosody as prosody_mod
 
 SAMPLE_RATE = 24000
@@ -44,10 +45,10 @@ class _Captured:
 class _Ticket:
     """A call issued with ``synthesize(..., defer=True)``: with predicted durations everything up to the frame-count
     read-back is enqueued; ``Synthesizer.finish`` synchronises on it and enqueues the rest."""
-    __slots__ = ("result", "last", "last_stream", "slot", "run_stream", "is_side", "ent", "got", "B", "launches")
+    __slots__ = ("result", "last", "last_stream", "slot", "run_stream", "is_side", "ent", "got", "B", "launches", "fmt")
 
     def __init__(self):
-        self.result = self.last = self.last_stream = self.ent = self.got = self.run_stream = None
+        self.result = self.last = self.last_stream = self.ent = self.got = self.run_stream = self.fmt = None
         self.slot = self.B = self.launches = 0
         self.is_side = False
 
@@ -93,7 +94,14 @@ class Synthesizer:
     the predicted durations and edits the predicted F0 / energy / EMA tracks.  The controls are graph inputs like the
     durations (a control block and a per-token duration scale staged through one pinned buffer), so one graph serves
     controls that change on every call.  Controlled calls have graphs of their own (one extra launch); calls
-    without ``prosody`` replay the same graphs as before."""
+    without ``prosody`` replay the same graphs as before.
+
+    **Output formats.**  ``synthesize(..., audio=AudioFormat(rate, encoding))`` (``artspeech_b200.audio``) returns the
+    waveforms resampled and encoded (e.g. 8 kHz G.711 mu-law for telephony, 16 kHz PCM for recognisers): one
+    ``as_resample_encode`` launch on the call's stream after the graph replay, into a fresh stream-ordered allocation.
+    It is not captured, so the format may change on every call without new graphs.  A format equal to the engine's
+    native output (24 kHz fp32, or 24 kHz PCM with ``pcm16=True``) takes the unformatted path; any other format needs
+    ``pcm16=False`` (the resampler reads fp32)."""
 
     def __init__(self, model, generator, device="cuda:0", use_cuda_graph: bool = True, pipeline_depth: int = 1,
                  pcm16: bool = False, acoustic_sms: Optional[int] = None, token_quantum: int = 32,
@@ -177,13 +185,14 @@ class Synthesizer:
                 mel_cl, aux = self.model.decode(st, dur, Lmax, mel16_dtype=gen.compute_dtype, ctrl=ctrl)
             self._sm_limit(max(2, total - self.acoustic_sms))
             with self._nvtx("asb.vocoder (HiFi-GAN generator)"):
-                wav = gen.forward_channels_last(aux["mel16"], aux["mel_lengths"],
-                                                torch.int16 if self.pcm16 else torch.float32)
+                wav, wav_lengths = gen.forward_channels_last(aux["mel16"], aux["mel_lengths"],
+                                                             torch.int16 if self.pcm16 else torch.float32,
+                                                             return_lengths=True)
         finally:
             self._sm_limit(0)
         mel = ops.to_channels_first(mel_cl, torch.float32)
         return dict(wav=wav.view(wav.shape[0], -1), mel_lengths=aux["mel_lengths"], mel=mel,
-                    duration=st["duration"], pred_dur=st["pred_dur"])
+                    duration=st["duration"], pred_dur=st["pred_dur"], wav_lengths=wav_lengths)
 
     def _eager(self, tokens, tl, mels, ml, durations, voice, predict, pros=None):
         """No graph: ragged reference mels, ``use_cuda_graph=False`` or a bucket not captured yet."""
@@ -322,7 +331,7 @@ class Synthesizer:
     # ---------------------------------------------------------------------------------------
     @torch.no_grad()
     def synthesize(self, tokens, tok_lens, mels, mel_lens, durations=None, voice=None, predict_durations: bool = False,
-                   exact_frames: bool = False, defer: bool = False, prosody=None):
+                   exact_frames: bool = False, defer: bool = False, prosody=None, audio=None):
         """``tokens`` int64 [B,Tt] and ``mels`` fp32 [B,80,Tr]: device tensors or (pinned) HOST tensors -- host inputs
         are copied straight into the graph's static buffers; ``tok_lens`` / ``mel_lens`` int64 [B] HOST tensors (or
         lists); ``durations`` int64 [B,Tt] HOST tensor or None (predict them, one device->host sync of B integers);
@@ -336,7 +345,10 @@ class Synthesizer:
         durations the ticket is handed out BEFORE the host waits for the frame counts, so a caller can issue the next
         call's graph A first (``synthesize_many`` does): the GPU then always has work queued while the host wakes up.
         ``prosody``: one ``prosody.Prosody`` per utterance (``ValueError`` for a ``duration_scale`` other than 1 when
-        ``durations`` are given); ``last["pred_dur"]`` then holds the scaled durations."""
+        ``durations`` are given); ``last["pred_dur"]`` then holds the scaled durations.
+        ``audio``: an ``audio.AudioFormat``; the returned waveforms are then ``[B, audio.out_samples(300*Tm_max)]``
+        of ``audio.dtype`` with silence codes beyond each utterance, and ``last["sample_lengths"]`` holds the
+        utterances' sample counts at the target rate (int32, device)."""
         dev = self.device
         cur = torch.cuda.current_stream(dev)
         self.last_stream = cur
@@ -349,6 +361,7 @@ class Synthesizer:
         B, Tt = tokens.shape
         Tr = mels.shape[2]
         pros = prosody_mod.check(prosody, tl, durations is not None)
+        fmt = self._out_format(audio)
         controlled = pros is not None
         predict = bool(predict_durations) or durations is None
         Tt_b = _ceil_to(Tt, self.token_quantum)
@@ -369,6 +382,8 @@ class Synthesizer:
             graphable = n >= self.capture_after
         if not graphable:
             res = self._eager(tokens, tl, mels, ml, durations, voice, predict, pros)
+            if fmt is not None:
+                res = self._format_stage(res, fmt)
             return self._done_ticket(res) if defer else res
         if self._epoch != nn_util.plan_epoch():
             self.drop_graphs()
@@ -431,6 +446,7 @@ class Synthesizer:
                 t.got = torch.cuda.Event()
                 t.got.record(run_stream)
                 t.slot, t.run_stream, t.is_side, t.ent, t.B, t.launches = slot, run_stream, run_stream is not cur, ent, B, launches
+                t.fmt = fmt
                 if defer:
                     return t
                 return self.finish(t)
@@ -450,7 +466,39 @@ class Synthesizer:
             Tm = 2 * max(sums)
             self.last = dict(out, frames=[2 * v for v in sums], graph=True)
             res = (out["wav"][:, :HOP * Tm], out["mel_lengths"], out["mel"][:, :, :Tm])
+        if fmt is not None:
+            res = self._format_stage(res, fmt, slot if run_stream is not cur else None)
         return self._done_ticket(res) if defer else res
+
+    def _out_format(self, audio):
+        """The format stage's format, or None for the native output (``audio`` None or equal to it)."""
+        if audio is None:
+            return None
+        if not isinstance(audio, audio_mod.AudioFormat):
+            raise ValueError(f"audio: expected an AudioFormat, got {type(audio).__name__}")
+        if audio == audio_mod.AudioFormat(SAMPLE_RATE, "pcm16" if self.pcm16 else "float32"):
+            return None
+        if self.pcm16:
+            raise ValueError(f"audio={audio}: output formats resample the fp32 waveform; use Synthesizer(pcm16=False) "
+                             f"(AudioFormat(24000, 'pcm16') gives the same samples as pcm16=True)")
+        return audio
+
+    def _format_stage(self, res, fmt, side_slot=None):
+        """One ``as_resample_encode`` launch on ``last_stream`` after the pass, into a fresh stream-ordered
+        allocation; not captured, so it adds no graphs.  ``side_slot``: the pipeline slot whose side stream ran the
+        call (``join`` then also waits for the format stage)."""
+        wav, mel_lengths, mel = res
+        with torch.cuda.stream(self.last_stream):
+            n = torch.empty(wav.shape[0], dtype=torch.int32, device=wav.device)
+            y = ops.resample_encode(wav, self.last["wav_lengths"], fmt, fmt.out_samples(wav.shape[1]), out_lens=n)
+            if side_slot is not None:
+                done = torch.cuda.Event()
+                done.record(self.last_stream)
+                self._slot_done[side_slot] = done
+        self.last["sample_lengths"] = n
+        if self.last.get("graph"):
+            self.launches_per_call += 1
+        return y, mel_lengths, mel
 
     def _done_ticket(self, res):
         t = _Ticket()
@@ -492,8 +540,10 @@ class Synthesizer:
         Tm = 2 * max(sums)
         self.last = dict(out, frames=[2 * v for v in sums], graph=True, duration=ent.state["duration"],
                          pred_dur=ent.state["pred_dur"])
-        ticket.result, ticket.last, ticket.last_stream = (out["wav"][:, :HOP * Tm], out["mel_lengths"], out["mel"][:, :, :Tm]), \
-            self.last, self.last_stream
+        res = (out["wav"][:, :HOP * Tm], out["mel_lengths"], out["mel"][:, :, :Tm])
+        if ticket.fmt is not None:
+            res = self._format_stage(res, ticket.fmt, slot if ticket.is_side else None)
+        ticket.result, ticket.last, ticket.last_stream = res, self.last, self.last_stream
         return ticket.result
 
     def join(self):
@@ -602,7 +652,8 @@ class HostArena:
 def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels: Sequence[torch.Tensor],
                     durations: Optional[Sequence[torch.Tensor]] = None, max_batch: int = 16,
                     max_padded_frames: Optional[int] = 25600, to_host: bool = False, arena: Optional[HostArena] = None,
-                    frames_per_token: float = 5.34, prosody: Optional[Sequence["prosody_mod.Prosody"]] = None):
+                    frames_per_token: float = 5.34, prosody: Optional[Sequence["prosody_mod.Prosody"]] = None,
+                    audio: Optional["audio_mod.AudioFormat"] = None):
     """Mixed-length utterances through ``syn`` in length-bucketed ragged micro-batches (BASELINE config 5).
 
     ``tokens[i]`` int64 [Tt_i], ``ref_mels[i]`` fp32 [80, Tr_i], ``durations[i]`` int64 [Tt_i] (host tensors) or
@@ -612,7 +663,9 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     utterance ``i`` (fp32, or int16 when ``syn.pcm16``), independent of what it was batched with (batch-1
     semantics) -- device tensors, or views of the pinned ``arena`` when ``to_host`` (valid after this function
     returns: it synchronises the copies).  ``prosody``: one ``prosody.Prosody`` per utterance (or None); the planning
-    estimate of an utterance then grows with its mean ``duration_scale``."""
+    estimate of an utterance then grows with its mean ``duration_scale``.  ``audio``: an ``audio.AudioFormat`` (see
+    ``Synthesizer.synthesize``); ``wavs[i]`` then holds the ``audio.out_samples(300 * frames[i])`` samples of
+    utterance ``i`` in that format."""
     n = len(tokens)
     pros = prosody_mod.check(prosody, [int(t.shape[0]) for t in tokens], durations is not None)
     if durations is not None:
@@ -623,7 +676,12 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
                        for i, t in enumerate(tokens)]
     frames: List[int] = list(plan_frames)
     wavs: List[Optional[torch.Tensor]] = [None] * n
-    dt = torch.int16 if syn.pcm16 else torch.float32
+    fmt = syn._out_format(audio)
+    dt = fmt.dtype if fmt is not None else torch.int16 if syn.pcm16 else torch.float32
+
+    def cut(f):
+        """Samples of an utterance of ``f`` mel frames in the output format."""
+        return fmt.out_samples(HOP * f) if fmt is not None else HOP * f
     arena = arena or (HostArena() if to_host else None)
     if to_host:
         arena.reset()
@@ -651,7 +709,7 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
                 late.append((idx, dst, meta, syn.last["frame_bound"]))
             else:
                 for j, i in enumerate(idx):
-                    wavs[i] = dst[j, :HOP * frames[i]] if to_host else wav[j, :HOP * frames[i]].clone()
+                    wavs[i] = dst[j, :cut(frames[i])] if to_host else wav[j, :cut(frames[i])].clone()
 
     # With predicted durations a call synchronises on its frame counts between its two graphs: issue the NEXT
     # micro-batch's first graph before finishing the current one (one call of look-ahead; needs a second pipeline slot)
@@ -671,7 +729,7 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
         tl = [int(tokens[i].shape[0]) for i in idx]
         ml = [int(ref_mels[i].shape[1]) for i in idx]
         waiting.append((idx, syn.synthesize(tok, tl, mel, ml, dur, defer=True,
-                                            prosody=[pros[i] for i in idx] if pros else None)))
+                                            prosody=[pros[i] for i in idx] if pros else None, audio=fmt)))
         while len(waiting) > lookahead:
             collect(*waiting.pop(0))
         pending.append((tok, mel))            # pinned inputs must outlive their asynchronous copies
@@ -684,16 +742,16 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     for idx, dst, meta, bound in late:
         for j, i in enumerate(idx):
             frames[i] = int(meta[j])
-            wavs[i] = dst[j, :HOP * frames[i]]
+            wavs[i] = dst[j, :cut(frames[i])]
             if 2 * int(meta[len(idx) + j]) > bound:       # the prediction did not fit the bound: truncated there
                 redo.append(i)
     for i in redo:                                         # rare: exact two-graph pass for the utterances that overflowed
         w, _, _ = syn.synthesize(tokens[i].view(1, -1).pin_memory(), [int(tokens[i].shape[0])],
                                  ref_mels[i].unsqueeze(0).pin_memory(), [int(ref_mels[i].shape[1])], None, exact_frames=True,
-                                 prosody=[pros[i]] if pros else None)
+                                 prosody=[pros[i]] if pros else None, audio=fmt)
         frames[i] = syn.last["frames"][0]
         with torch.cuda.stream(syn.last_stream):
-            wavs[i] = w[0, :HOP * frames[i]].clone() if not to_host else w[0, :HOP * frames[i]].to("cpu")
+            wavs[i] = w[0, :cut(frames[i])].clone() if not to_host else w[0, :cut(frames[i])].to("cpu")
     if redo:
         syn.join()
         torch.cuda.current_stream(syn.device).synchronize()
@@ -705,8 +763,8 @@ def _as_bytes(t: torch.Tensor) -> torch.Tensor:
 
 
 def _pack_payload(wav: torch.Tensor, lengths: torch.Tensor, Bm: int, Sm: int, out: Optional[torch.Tensor] = None):
-    """One byte buffer per rank: ``Bm`` int64 sample counts (header) followed by the ``[Bm, Sm]`` samples.  int16 PCM
-    and fp32 both travel as bytes (the NCCL process group has no int16)."""
+    """One byte buffer per rank: ``Bm`` int64 sample counts (header) followed by the ``[Bm, Sm]`` samples.  int16 PCM,
+    uint8 G.711 codes and fp32 all travel as bytes (the NCCL process group has no int16)."""
     es = wav.element_size()
     nbytes = 8 * Bm + Bm * Sm * es
     if out is None:
@@ -728,7 +786,7 @@ def _unpack_payload(buf: torch.Tensor, dtype: torch.dtype, Bm: int, Sm: int, sha
 
 
 def gather_waveforms(wav: torch.Tensor, lengths: torch.Tensor, dst: int = 0, group=None, shapes=None):
-    """Gather per-rank ``wav`` [B_r, S_r] (fp32 or int16 PCM) + sample ``lengths`` [B_r] on ``dst`` with ONE
+    """Gather per-rank ``wav`` [B_r, S_r] (fp32, int16 PCM or uint8 G.711 codes) + sample ``lengths`` [B_r] on ``dst`` with ONE
     collective: each rank contributes one byte buffer (lengths header + samples, padded to the common maximum).
 
     Ranks may hold different batch sizes / paddings: sizes are all-gathered first unless ``shapes`` (list of

@@ -423,6 +423,34 @@ def prosody_apply(f0, n, ema, lens, ctrl, pitch_mean: float, pitch_std: float, e
          float(pitch_mean), float(pitch_std), float(energy_std))
 
 
+def resample_encode(x, lens, fmt, S_out: int, *, m0: int = 0, out=None, out_lens=None):
+    """Waveforms in an output format (``as_resample_encode``; semantics in ``artspeech_b200.audio``): ``x`` fp32
+    [B, S_in] at 24 kHz (unit element stride, any row stride), ``lens`` int32 [B] device sample counts (or None: every
+    row holds S_in samples), ``fmt`` an ``audio.AudioFormat``.  Returns ``[B, S_out]`` of ``fmt.dtype``: samples
+    ``m0 .. m0 + S_out - 1`` at the target rate, silence beyond each utterance's ``fmt.out_samples(len)``.  ``out``:
+    an optional destination; ``out_lens``: an optional int32 [B] device tensor that receives the output lengths."""
+    _require_cuda(x, "resample_encode")
+    if x.dtype != torch.float32 or x.dim() != 2 or (x.stride(1) != 1 and x.shape[1] > 1):
+        raise _lib.AsError(f"resample_encode: x must be fp32 [B, S] with unit sample stride, got {x.dtype} "
+                           f"{tuple(x.shape)} strides {x.stride()}")
+    B, S_in = x.shape
+    if out is None:
+        out = torch.empty(B, int(S_out), dtype=fmt.dtype, device=x.device)
+    elif out.dtype != fmt.dtype or tuple(out.shape) != (B, int(S_out)) or (out.stride(1) != 1 and S_out > 1) or \
+            out.device != x.device:
+        raise _lib.AsError(f"resample_encode: out must be {fmt.dtype} [{B}, {S_out}] on {x.device}")
+    for t, name in ((lens, "lens"), (out_lens, "out_lens")):
+        if t is not None and (t.dtype != torch.int32 or t.device != x.device or t.numel() != B or
+                              (B > 1 and t.stride(0) != 1)):
+            raise _lib.AsError(f"resample_encode: {name} must be int32 [{B}] on {x.device}")
+    table = fmt.device_table(x.device)
+    one = lambda n: (int(n) + 15) // 16 * 16           # a single row's stride is free: keep rows 16-byte aligned
+    _run("as_resample_encode", x, x.data_ptr(), x.stride(0) if B > 1 else one(S_in), B, S_in, _p(lens),
+         table.data_ptr(), fmt.table_ld, fmt.up, fmt.down, fmt.K, fmt.half_len, int(m0), int(S_out), out.data_ptr(),
+         out.stride(0) if B > 1 else one(S_out), fmt.code, _p(out_lens))
+    return out
+
+
 @dataclass
 class SmallConv:
     w: torch.Tensor            # fp32 [ntaps, Cout, Cin] device

@@ -28,6 +28,7 @@ import torch
 import torch.nn as nn
 from torch.nn.utils import remove_weight_norm, weight_norm
 
+from . import audio as audio_mod
 from . import nn_util, ops
 
 LRELU_SLOPE = 0.1
@@ -168,16 +169,31 @@ class Generator(nn.Module):
 
     # -- forward ----------------------------------------------------------------------------------
     @torch.no_grad()
-    def forward(self, x: torch.Tensor, lengths: Optional[torch.Tensor] = None, pcm16: bool = False) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, lengths: Optional[torch.Tensor] = None, pcm16: bool = False,
+                audio: Optional[audio_mod.AudioFormat] = None) -> torch.Tensor:
         """``x``: mel ``[B, num_mels, T]`` -> waveform ``[B, 1, T*prod(upsample_rates)]`` (fp32).
         ``pcm16=True`` (extension): int16 samples ``rint(32767 * wav)`` straight from the conv_post kernel -- the
-        samples ``soundfile.write(path, wav, 24000)`` (test.py:119) stores -- halving the device->host bytes."""
+        samples ``soundfile.write(path, wav, 24000)`` (test.py:119) stores -- halving the device->host bytes.
+        ``audio=AudioFormat(rate, encoding)`` (extension, ``artspeech_b200.audio``): the waveform resampled and
+        encoded on the device, ``[B, 1, audio.out_samples(T*hop)]`` of ``audio.dtype``; with ``lengths`` each
+        utterance has ``audio.out_samples(lengths[b]*hop)`` samples and silence codes beyond.  Not with ``pcm16``."""
+        audio_mod.check(audio, pcm16)
         mel_cl = x.detach().transpose(1, 2).to(self.compute_dtype).contiguous()   # [B, T, 80]
         if lengths is not None:  # frames beyond an utterance's length must not leak into it
             keep = torch.arange(mel_cl.shape[1], device=mel_cl.device)[None, :] < lengths.to(mel_cl.device)[:, None]
             mel_cl = mel_cl * keep.unsqueeze(-1).to(mel_cl.dtype)
         wav = self.forward_channels_last(mel_cl, lengths, torch.int16 if pcm16 else torch.float32)
+        if audio is not None:
+            lens = None if lengths is None else lengths.to(device=wav.device, dtype=torch.int32) * self.hop()
+            wav = ops.resample_encode(wav, lens, audio, audio.out_samples(wav.shape[1]))
         return wav.view(wav.shape[0], 1, -1)
+
+    def hop(self) -> int:
+        """24 kHz samples per mel frame (300)."""
+        hop = 1
+        for u in self.h.upsample_rates:
+            hop *= u
+        return hop
 
     def receptive_field_frames(self) -> int:
         """Mel frames on either side that can influence an output sample: conv_pre (k 7) + per stage the
@@ -195,27 +211,45 @@ class Generator(nn.Module):
         return int(math.ceil(rf))
 
     @torch.no_grad()
-    def stream(self, x: torch.Tensor, chunk_frames: int = 64, halo_frames: Optional[int] = None, pcm16: bool = False):
+    def stream(self, x: torch.Tensor, chunk_frames: int = 64, halo_frames: Optional[int] = None, pcm16: bool = False,
+               audio: Optional[audio_mod.AudioFormat] = None):
         """Chunked vocoding for latency-bound serving (SURVEY.md §8f-3): yields ``(first_sample, wav_chunk)`` with
         ``wav_chunk`` ``[B, 1, <=chunk_frames*hop]``.  Every chunk is vocoded with ``halo_frames`` (default: the
         receptive field) of real context on both sides and only its centre is kept, so the concatenation equals
         ``forward(x)``; the first audio is available after one ``chunk_frames + halo`` pass instead of the whole
-        utterance."""
+        utterance.
+
+        ``audio=AudioFormat(...)``: chunks in that format, ``first_sample`` counted at its rate; the chunk of frames
+        ``[t0, t1)`` is output samples ``[audio.out_samples(t0*hop), audio.out_samples(t1*hop))``, so the
+        concatenation equals ``forward(x, audio=audio)``.  The resampling filter reaches ``ceil(half_len / up)``
+        input samples (at most 30, at 8 kHz) beyond a chunk: the receptive field's ceiling (13.06 -> 14 frames for
+        the V1 config) covers that.  A window starts at a multiple of ``audio.frame_align(hop)`` frames, where the
+        24 kHz input and the output grid coincide."""
+        audio_mod.check(audio, pcm16)
         halo = self.receptive_field_frames() if halo_frames is None else int(halo_frames)
-        hop = 1
-        for u in self.h.upsample_rates:
-            hop *= u
+        hop = self.hop()
         T = x.shape[2]
+        align = 1 if audio is None else audio.frame_align(hop)
         for t0 in range(0, T, chunk_frames):
             t1 = min(T, t0 + chunk_frames)
             a, b = max(0, t0 - halo), min(T, t1 + halo)
-            wav = self.forward(x[:, :, a:b], pcm16=pcm16)
-            yield t0 * hop, wav[:, :, (t0 - a) * hop:(t1 - a) * hop]
+            if audio is None:
+                wav = self.forward(x[:, :, a:b], pcm16=pcm16)
+                yield t0 * hop, wav[:, :, (t0 - a) * hop:(t1 - a) * hop]
+                continue
+            a -= a % align
+            wav = self.forward(x[:, :, a:b])
+            lo, hi = audio.out_samples(t0 * hop), audio.out_samples(t1 * hop)
+            base = a * hop * audio.up // audio.down                     # output index of the window's first sample
+            y = ops.resample_encode(wav.view(wav.shape[0], -1), None, audio, hi - lo, m0=lo - base)
+            yield lo, y.view(y.shape[0], 1, -1)
 
     @torch.no_grad()
     def forward_channels_last(self, mel_cl: torch.Tensor, lengths: Optional[torch.Tensor] = None,
-                              out_dtype: torch.dtype = torch.float32):
-        """``mel_cl``: ``[B, T, 80]`` in the compute dtype.  Returns ``[B, T*300]`` fp32 (or int16 PCM)."""
+                              out_dtype: torch.dtype = torch.float32, return_lengths: bool = False):
+        """``mel_cl``: ``[B, T, 80]`` in the compute dtype.  Returns ``[B, T*300]`` fp32 (or int16 PCM); with
+        ``return_lengths`` also the utterances' sample counts, int32 [B] on the device (``lengths * 300``, computed
+        with the per-stage lengths; None without ``lengths``)."""
         dev = mel_cl.device
         if self._plan is None:
             self._plan = self._build_plan(dev)
@@ -296,4 +330,6 @@ class Generator(nn.Module):
                         _, a = ops.conv(t, c2s[m], res1=r, res2=xs, scale=1.0 / self.num_kernels,
                                         act_out=dt, act=ops.ACT_LRELU, slope=next_slope, lens=lens)
         _, wav = ops.conv(a, plan["post"], act_out=out_dtype, act=ops.ACT_TANH, lens=lens)
+        if return_lengths:
+            return wav.view(B, L), lens
         return wav.view(B, L)

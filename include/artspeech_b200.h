@@ -283,6 +283,27 @@ int as_prosody_apply(float* f0, int64_t f0_ld, float* n, int64_t n_ld, float* em
                      int32_t Tm, const int32_t* lens, const float* ctrl, double pitch_mean, double pitch_std,
                      double energy_std, void* stream);
 
+/* Output audio formats (artspeech_b200/audio.py): resampling of fp32 waveforms by up/down and encoding, one launch.
+ *   y[b,m] = sum_{j=0..K-1} table[p][j] * x[b, i0 - j],  n = m*down + half_len, i0 = n / up, p = n % up,
+ * with x zero outside [0, n_in_b), n_in_b = min(in_lens[b], S_in) (S_in when in_lens is NULL): one fp32 fma chain over
+ * j = 0..K-1 in that order, so a value depends only on its row's samples and m.  table fp32 [up][table_ld], 16-byte
+ * aligned, table_ld >= K and a multiple of 4.  up == down == 1 is the identity y = x (table, K, half_len ignored).
+ * x [B, >= S_in] with row stride x_ld; out [B, S_out] with row stride out_ld (elements).  Output r of row b is sample
+ * m = m0 + r: y encoded for m < n_out_b = ceil(n_in_b * up / down), the encoding's silence code beyond.  Encodings:
+ *   AS_AUDIO_F32 float y;  AS_AUDIO_PCM16 int16 clamp(rint(32767 y), -32768, 32767) (the AS_PCM16 conv epilogue);
+ *   AS_AUDIO_MULAW / AS_AUDIO_ALAW uint8 ITU-T G.711 code of that int16 (audioop.lin2ulaw / lin2alaw, width 2).
+ * Silence is 0, 0, 0xFF, 0xD5.  out_lens int32 [B] (may be NULL, must not alias in_lens) receives n_out_b.  Lengths
+ * are read and written on the device: no host synchronisation.  Filters whose shared memory
+ * (as_resample_smem_bytes) exceeds AS_AUDIO_SMEM_MAX are refused with AS_ERR_SHAPE. */
+typedef enum as_audio_encoding { AS_AUDIO_F32 = 0, AS_AUDIO_PCM16 = 1, AS_AUDIO_MULAW = 2, AS_AUDIO_ALAW = 3 } as_audio_encoding;
+#define AS_AUDIO_TILE 1024
+#define AS_AUDIO_SMEM_MAX (96 * 1024)
+size_t as_resample_smem_bytes(int32_t up, int32_t down, int32_t K, int32_t table_ld);
+int as_resample_encode(const float* x, int64_t x_ld, int32_t B, int32_t S_in, const int32_t* in_lens,
+                       const float* table, int32_t table_ld, int32_t up, int32_t down, int32_t K, int32_t half_len,
+                       int32_t m0, int32_t S_out, void* out, int64_t out_ld, int32_t encoding, int32_t* out_lens,
+                       void* stream);
+
 /* Direct convolution for tiny input-channel counts (Cin <= 16) on CUDA cores: first layers of the
  * 2-D stacks (1 -> 64, 3x3), F0/N/EMA 1x1 convs of the decoder (models.py:480-482, 502-504).
  * x [B,T,F,Cin]; w fp32 [ntaps][Cout][Cin]; taps host arrays; stride 1; zero padding; outputs as
