@@ -185,7 +185,8 @@ int as_hifigan_resblock_pair(const as_resblock_pair_params* p, void* stream);
  * gives the valid number of T positions per batch item and rows beyond it are written as zeros.
  * ------------------------------------------------------------------------------------------ */
 
-/* emb(x) * scale (Utils/RelTransformerEnc.py:372-373); out32 fp32 and/or out16 (16-bit) [B,T,C] */
+/* emb(x) * scale (Utils/RelTransformerEnc.py:372-373); out32 fp32 and/or out16 (16-bit) [B,T,C].  Token ids
+ * outside [0, n_vocab) read row 0 of the table. */
 int as_embed(const int64_t* tokens, const float* table, int32_t n_vocab, int32_t B, int32_t T,
              int32_t C, float scale, const int32_t* lens, float* out32, void* out16,
              int32_t out16_dtype, void* stream);
@@ -248,8 +249,9 @@ int as_repeat_rows(const void* x, int32_t x_dtype, int64_t x_ld, int32_t B, int3
 
 /* Length regulation (models.py:361-368 one-hot matmul == gather) fused with the decoder's x2
  * nearest upsample (models.py:500): frame r of item b copies token j where
- * cum[j] <= r / rep < cum[j+1], cum = exclusive prefix sum of dur[b, :lens_t[b]].
- * x [B,Tt,C]; dur int32 [B,Tt]; out [B,To,C] (rows >= rep*sum(dur) zero); out_lens[b] = rep*sum. */
+ * cum[j] <= r / rep < cum[j+1], cum = exclusive prefix sum of max(dur[b, j], 0) over j < min(lens_t[b], Tt)
+ * (durations and token rows beyond that are not read).  x [B,Tt,C]; dur int32 [B,Tt]; out [B,To,C] (rows >=
+ * rep*sum zero); out_lens[b] = min(rep*sum, To). */
 int as_length_regulate(const void* x, int32_t x_dtype, int64_t x_ld, int32_t B, int32_t Tt,
                        int32_t C, const int32_t* dur, const int32_t* lens_t, int32_t rep,
                        int32_t To, void* out, int32_t out_dtype, int64_t out_ld,
