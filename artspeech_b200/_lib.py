@@ -134,4 +134,9 @@ SIGNATURES.update({
     "as_expand_tokens": (C.c_int, [_V, _V, _V, _I, _I, _I, _I, _V]),
     "as_resample_smem_bytes": (C.c_size_t, [_I, _I, _I, _I]),
     "as_resample_encode": (C.c_int, [_V, _L, _I, _I, _V, _V, _I, _I, _I, _I, _I, _I, _I, _V, _L, _I, _V, _V]),
+    "as_resample_encode_gain": (C.c_int, [_V, _L, _I, _I, _V, _V, _I, _I, _I, _I, _I, _I, _I, _V, _L, _I, _V, _V,
+                                          _V]),
+    "as_loudness_workspace_bytes": (C.c_size_t, [_I, _L, _I]),
+    "as_loudness_measure": (C.c_int, [_V, _L, _I, _L, _V, _I, C.POINTER(C.c_double), c_f32_p, C.c_double,
+                                      C.c_double, _V, C.c_size_t, _V, _V, _V, _V, _V]),
 })

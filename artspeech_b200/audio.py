@@ -19,6 +19,39 @@ Semantics (per utterance of ``n_in`` samples at 24 kHz):
 
 A rate whose filter does not fit the kernel's shared-memory budget (``smem_bytes`` above ``SMEM_MAX``: very low rates
 and rates with a large ``up``, e.g. 44101 Hz) is refused on construction.
+
+**Loudness normalisation** (``Loudness(target_lufs, max_true_peak_db)``, ``as_loudness_measure``).  The meter, for
+one utterance of ``n`` fp32 samples at ``fs`` Hz (the engine meters at 24 kHz; ``measure_loudness`` takes any multiple
+of 10 Hz from 8000 to 192000):
+
+1. **K-weighting** (ITU-R BS.1770): two cascaded biquads with zero initial state, designed by the bilinear transform
+   as libebur128 does and evaluated in fp64 on the host (``k_weighting``).  Shelf: ``f0 = 1681.974450955533``,
+   ``G = 3.999843853973347``, ``Q = 0.7071752369554196``, ``K = tan(pi f0 / fs)``, ``Vh = 10^(G/20)``,
+   ``Vb = Vh^0.4996667741545416``, ``a0 = 1 + K/Q + K^2``, ``b = [Vh + Vb K/Q + K^2, 2 (K^2 - Vh),
+   Vh - Vb K/Q + K^2] / a0``, ``a = [1, 2 (K^2 - 1) / a0, (1 - K/Q + K^2) / a0]``.  High-pass:
+   ``f0 = 38.13547087602444``, ``Q = 0.5003270373238773``, ``b = [1, -2, 1]``, ``a`` as above.  At 48 kHz these are
+   BS.1770-4's table.
+2. **Blocks.**  Segments of ``fs/10`` samples (100 ms); block ``j`` covers segments ``j .. j+3`` (400 ms, 75 %
+   overlap) for ``j = 0 .. nseg - 4``, ``nseg = n // (fs/10)``; samples after the last complete segment feed no
+   block.  ``z_j`` is the mean of the squared K-weighted output over the block, ``L_j = -0.691 + 10 log10 z_j``.
+   An utterance shorter than one block (``n < 4 fs/10``, e.g. a single word) is one block over all ``n`` samples;
+   BS.1770 defines no value for such signals.
+3. **Gating.**  ``J_a = {j : L_j > -70}``, ``G_r = -0.691 + 10 log10(mean_{J_a} z) - 10``,
+   ``J_g = {j in J_a : L_j > G_r}``, integrated loudness ``L = -0.691 + 10 log10(mean_{J_g} z)`` (LUFS); ``-inf``
+   when ``J_a`` is empty or ``n = 0``.
+4. **True peak.**  ``TP = max(max_i |x_i|, max_m |y4_m|)`` with ``y4`` the 4x interpolation by this module's
+   resampler math (``_design(4, 1)``: 81 taps, ``half_len`` 40, fp32 polyphase table ``true_peak_table()``), ``x``
+   zero outside ``[0, n)``, ``m < 4 n``; ``true_peak_db = 20 log10 TP`` (``-inf`` for 0).  At 24 kHz this is a 96 kHz
+   peak: BS.1770 asks 4x for 48 kHz input, so an inter-sample peak close to Nyquist can read low.
+5. **Gain.**  ``gain_db = 0`` if ``L = -inf``, else ``min(target_lufs - L, max_true_peak_db - true_peak_db)``;
+   ``g = fp32(10^(gain_db/20))`` (computed in fp64, rounded once).  The format stage outputs ``encode(g * y)``: one
+   fp32 multiply after the resampler's value ``y`` (after ``x`` at 24 kHz), before the encoding; silence codes are
+   unchanged.  A single gain, like ffmpeg ``loudnorm`` in linear mode: no limiter or dynamic range control.
+6. **Measurement point.**  The engine meters the vocoder's 24 kHz fp32 waveform once per utterance, whatever the
+   output format, so one utterance requested in two formats gets the same gain and no extra pass at the target rate
+   is needed.  A meter run at a lower delivery rate (8 kHz) reads somewhat lower, because the band above that rate's
+   Nyquist frequency is removed.  Normalisation sets the overall level, so it overrides the overall-level effect of
+   ``Prosody.energy_db`` (the energy contour's shape stays).
 """
 from __future__ import annotations
 
@@ -183,3 +216,90 @@ def check(audio, pcm16: bool):
     if pcm16:
         raise ValueError("audio= and pcm16=True: choose the encoding with AudioFormat(..., encoding='pcm16')")
     return audio
+
+
+# ---- loudness --------------------------------------------------------------------------------------------------
+_SHELF = (1681.974450955533, 3.999843853973347, 0.7071752369554196)
+_HIGHPASS = (38.13547087602444, 0.5003270373238773)
+TRUE_PEAK_UP = 4
+
+
+def _rate_ok(fs) -> bool:
+    return not isinstance(fs, bool) and isinstance(fs, (int, np.integer)) and 8000 <= fs <= 192000 and fs % 10 == 0
+
+
+@lru_cache(maxsize=None)
+def k_weighting(fs: int) -> Tuple[Tuple[np.ndarray, np.ndarray], Tuple[np.ndarray, np.ndarray]]:
+    """((b, a) of the shelf, (b, a) of the high-pass) of BS.1770's K-weighting at ``fs`` Hz, fp64."""
+    f0, G, Q = _SHELF
+    K = math.tan(math.pi * f0 / fs)
+    Vh = 10.0 ** (G / 20.0)
+    Vb = Vh ** 0.4996667741545416
+    a0 = 1.0 + K / Q + K * K
+    shelf = (np.array([(Vh + Vb * K / Q + K * K) / a0, 2.0 * (K * K - Vh) / a0, (Vh - Vb * K / Q + K * K) / a0]),
+             np.array([1.0, 2.0 * (K * K - 1.0) / a0, (1.0 - K / Q + K * K) / a0]))
+    f0, Q = _HIGHPASS
+    K = math.tan(math.pi * f0 / fs)
+    a0 = 1.0 + K / Q + K * K
+    hp = (np.array([1.0, -2.0, 1.0]), np.array([1.0, 2.0 * (K * K - 1.0) / a0, (1.0 - K / Q + K * K) / a0]))
+    return shelf, hp
+
+
+def k_weighting_taps(fs: int) -> np.ndarray:
+    """The 10 doubles ``as_loudness_measure`` takes: b0 b1 b2 a1 a2 of the shelf, then of the high-pass."""
+    (bs, as_), (bh, ah) = k_weighting(int(fs))
+    return np.concatenate([bs, as_[1:], bh, ah[1:]])
+
+
+def true_peak_table() -> np.ndarray:
+    """The fp32 polyphase table ``[4, 24]`` of the 4x true-peak interpolator (``_design(4, 1)``: 21 taps a phase)."""
+    return _design(TRUE_PEAK_UP, 1)[1]
+
+
+@dataclass(frozen=True)
+class Loudness:
+    """Loudness normalisation of each utterance to ``target_lufs`` (integrated loudness, ITU-R BS.1770) with its true
+    peak at most ``max_true_peak_db`` dBTP: one gain per utterance, applied before the output encoding.  The default is
+    EBU R128 (-23 LUFS, -1 dBTP); ATSC A/85 is -24, streaming platforms use -14 to -16."""
+    target_lufs: float = -23.0
+    max_true_peak_db: float = -1.0
+
+    def __post_init__(self):
+        for name in ("target_lufs", "max_true_peak_db"):
+            v = getattr(self, name)
+            if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)) or \
+                    not math.isfinite(float(v)):
+                raise ValueError(f"Loudness.{name}: expected a finite number, got {v!r}")
+            object.__setattr__(self, name, float(v))
+        if self.target_lufs >= 0.0:
+            raise ValueError(f"Loudness.target_lufs: must be negative, got {self.target_lufs}")
+        if self.max_true_peak_db > 0.0:
+            raise ValueError(f"Loudness.max_true_peak_db: must be at most 0 dBTP, got {self.max_true_peak_db}")
+
+
+def check_loudness(loudness, pcm16: bool):
+    """Validate a ``loudness=`` argument: None or a ``Loudness``; with ``pcm16=True`` a ``ValueError`` (the meter and
+    the gain read the fp32 waveform)."""
+    if loudness is None:
+        return None
+    if not isinstance(loudness, Loudness):
+        raise ValueError(f"loudness: expected a Loudness, got {type(loudness).__name__}")
+    if pcm16:
+        raise ValueError("loudness= and pcm16=True: the meter reads the fp32 waveform; use Synthesizer(pcm16=False) "
+                         "with audio=AudioFormat(24000, 'pcm16')")
+    return loudness
+
+
+def measure_loudness(wav: torch.Tensor, lengths=None, sample_rate: int = NATIVE_RATE):
+    """``(lufs, true_peak_db)`` of each row of ``wav`` (fp32 [B, S] or [S], CUDA) as fp64 [B] device tensors, measured
+    on the GPU as stated in this module's docstring.  ``lengths``: per-row sample counts (int tensor or sequence;
+    None: every row holds S samples); ``sample_rate``: a multiple of 10 Hz from 8000 to 192000."""
+    from . import ops
+    if not _rate_ok(sample_rate):
+        raise ValueError(f"measure_loudness: sample_rate must be a multiple of 10 Hz in [8000, 192000], "
+                         f"got {sample_rate!r}")
+    x = wav.view(1, -1) if wav.dim() == 1 else wav
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
+    lufs, tp, _, _ = ops.loudness_measure(x, lengths, int(sample_rate))
+    return lufs, tp

@@ -9,6 +9,8 @@
 // the banks), encodes them into a shared-memory row and writes that row with 16-byte stores.  Each output is one
 // fp32 fma chain over the taps j = 0..K-1 in that order, so its bits depend on its utterance's samples and its
 // index only: not on B, S_in, the tile or the output offset m0 (batch invariance, chunked == one-shot output).
+// With a per-utterance gain (loudness normalisation, loudness.cu) the value is multiplied by gain[b] once, in fp32,
+// before it is encoded; the kernel is a template on whether there is a gain, so the gain-free path is unchanged.
 #include "common.cuh"
 #include "tc_util.cuh"
 
@@ -72,12 +74,12 @@ __device__ __forceinline__ void audio_put(unsigned char* row, int r, float y, in
   }
 }
 
-template <bool kIdentity>
+template <bool kIdentity, bool kGain>
 __global__ void __launch_bounds__(kAudioThreads) resample_encode_kernel(
     const float* __restrict__ x, long long x_ld, int S_in, const int* __restrict__ in_lens,
     const float* __restrict__ table, int table_ld, int up, int down, int K, int half_len, int m0, int S_out,
-    unsigned char* __restrict__ out, long long out_ld, int enc, int* __restrict__ out_lens, int B, int tiles,
-    int win_alloc, int vec_in, int vec_out) {
+    unsigned char* __restrict__ out, long long out_ld, int enc, int* __restrict__ out_lens,
+    const float* __restrict__ gain, int B, int tiles, int win_alloc, int vec_in, int vec_out) {
   pdl_wait();
   extern __shared__ __align__(16) float audio_smem[];
   float* tab = audio_smem;                                        // [up][table_ld]
@@ -100,6 +102,7 @@ __global__ void __launch_bounds__(kAudioThreads) resample_encode_kernel(
     const int mt = m0 + r0;
     const int nv = max(0, min(nr, n_out - mt));                   // of which inside the utterance
     const float* xb = x + (long long)b * x_ld;
+    const float g = kGain ? gain[b] : 1.f;
     __syncthreads();                                              // the previous tile's window / row are consumed
     int i_al = 0;
     if (nv > 0) {
@@ -127,7 +130,7 @@ __global__ void __launch_bounds__(kAudioThreads) resample_encode_kernel(
 #pragma unroll
       for (int o = 0; o < kAudioPer; ++o) {
         const int r = tid + o * kAudioThreads;
-        if (r < nr) audio_put(ys, r, r < nv ? xw[mt + r - i_al] : 0.f, enc);
+        if (r < nr) audio_put(ys, r, r < nv ? (kGain ? xw[mt + r - i_al] * g : xw[mt + r - i_al]) : 0.f, enc);
       }
     } else {
       const int n = (mt + tid) * down + half_len;
@@ -148,7 +151,7 @@ __global__ void __launch_bounds__(kAudioThreads) resample_encode_kernel(
             acc = fmaf(h4.w, xp[-j - 3], acc);
           }
           for (; j < K; ++j) acc = fmaf(h[j], xp[-j], acc);
-          audio_put(ys, r, acc, enc);
+          audio_put(ys, r, kGain ? acc * g : acc, enc);
         } else if (r < nr) {
           audio_put(ys, r, 0.f, enc);                             // silence: the code of 0
         }
@@ -192,10 +195,42 @@ extern "C" size_t as_resample_smem_bytes(int32_t up, int32_t down, int32_t K, in
          (size_t)kAudioTile * 4;
 }
 
-extern "C" int as_resample_encode(const float* x, int64_t x_ld, int32_t B, int32_t S_in, const int32_t* in_lens,
+template <bool kGain>
+static int resample_encode_launch(const float* x, int64_t x_ld, int32_t B, int32_t S_in, const int32_t* in_lens,
                                   const float* table, int32_t table_ld, int32_t up, int32_t down, int32_t K,
                                   int32_t half_len, int32_t m0, int32_t S_out, void* out, int64_t out_ld,
-                                  int32_t encoding, int32_t* out_lens, void* stream) {
+                                  int32_t encoding, int32_t* out_lens, const float* gain, void* stream) {
+  const bool ident = up == 1 && down == 1;
+  const int tiles = S_out > 0 ? (S_out + kAudioTile - 1) / kAudioTile : 1;
+  const size_t smem = as_resample_smem_bytes(up, down, ident ? 1 : K, ident ? 4 : table_ld);
+  const int es = encoding == AS_AUDIO_F32 ? 4 : encoding == AS_AUDIO_PCM16 ? 2 : 1;
+  const int vec_in = (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (x_ld & 3) == 0;
+  const int vec_out = (reinterpret_cast<uintptr_t>(out) & 15) == 0 && ((out_ld * es) & 15) == 0;
+  const long long work = (long long)B * tiles;
+  const int grid = (int)std::min<long long>(work, (long long)num_sms() * 16);
+  const int win = (int)audio_window(up, down, ident ? 1 : K);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  unsigned char* o = static_cast<unsigned char*>(out);
+  if (ident) {
+    ASB_SMEM_OPT_IN(AS_AUDIO_SMEM_MAX, resample_encode_kernel<true, kGain>);
+    ASB_CUDA(launch_k(resample_encode_kernel<true, kGain>, dim3(grid), dim3(kAudioThreads), smem, st, x,
+                      (long long)x_ld, (int)S_in, in_lens, table, 4, 1, 1, 1, 0, (int)m0, (int)S_out, o,
+                      (long long)out_ld, (int)encoding, out_lens, gain, (int)B, tiles, win, vec_in, vec_out));
+  } else {
+    ASB_SMEM_OPT_IN(AS_AUDIO_SMEM_MAX, resample_encode_kernel<false, kGain>);
+    ASB_CUDA(launch_k(resample_encode_kernel<false, kGain>, dim3(grid), dim3(kAudioThreads), smem, st, x,
+                      (long long)x_ld, (int)S_in, in_lens, table, (int)table_ld, (int)up, (int)down, (int)K,
+                      (int)half_len, (int)m0, (int)S_out, o, (long long)out_ld, (int)encoding, out_lens, gain,
+                      (int)B, tiles, win, vec_in, vec_out));
+  }
+  return AS_OK;
+}
+
+extern "C" int as_resample_encode_gain(const float* x, int64_t x_ld, int32_t B, int32_t S_in,
+                                       const int32_t* in_lens, const float* table, int32_t table_ld, int32_t up,
+                                       int32_t down, int32_t K, int32_t half_len, int32_t m0, int32_t S_out,
+                                       void* out, int64_t out_ld, int32_t encoding, int32_t* out_lens,
+                                       const float* gain, void* stream) {
   if (B == 0) return AS_OK;
   ASB_REQUIRE(x && out && B > 0 && S_in >= 0 && S_out >= 0 && m0 >= 0 && x_ld >= S_in && out_ld >= S_out,
               AS_ERR_SHAPE, "as_resample_encode: bad argument");
@@ -221,25 +256,16 @@ extern "C" int as_resample_encode(const float* x, int64_t x_ld, int32_t B, int32
               "as_resample_encode: %zu bytes of shared memory for up %d / down %d (at most %d)", smem, (int)up,
               (int)down, AS_AUDIO_SMEM_MAX);
   if (int rc = check_arch()) return rc;
-  const int es = encoding == AS_AUDIO_F32 ? 4 : encoding == AS_AUDIO_PCM16 ? 2 : 1;
-  const int vec_in = (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (x_ld & 3) == 0;
-  const int vec_out = (reinterpret_cast<uintptr_t>(out) & 15) == 0 && ((out_ld * es) & 15) == 0;
-  const long long work = (long long)B * tiles;
-  const int grid = (int)std::min<long long>(work, (long long)num_sms() * 16);
-  const int win = (int)audio_window(up, down, ident ? 1 : K);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  unsigned char* o = static_cast<unsigned char*>(out);
-  if (ident) {
-    ASB_SMEM_OPT_IN(AS_AUDIO_SMEM_MAX, resample_encode_kernel<true>);
-    ASB_CUDA(launch_k(resample_encode_kernel<true>, dim3(grid), dim3(kAudioThreads), smem, st, x, (long long)x_ld,
-                      (int)S_in, in_lens, table, 4, 1, 1, 1, 0, (int)m0, (int)S_out, o, (long long)out_ld,
-                      (int)encoding, out_lens, (int)B, tiles, win, vec_in, vec_out));
-  } else {
-    ASB_SMEM_OPT_IN(AS_AUDIO_SMEM_MAX, resample_encode_kernel<false>);
-    ASB_CUDA(launch_k(resample_encode_kernel<false>, dim3(grid), dim3(kAudioThreads), smem, st, x, (long long)x_ld,
-                      (int)S_in, in_lens, table, (int)table_ld, (int)up, (int)down, (int)K, (int)half_len, (int)m0,
-                      (int)S_out, o, (long long)out_ld, (int)encoding, out_lens, (int)B, tiles, win, vec_in,
-                      vec_out));
-  }
-  return AS_OK;
+  return gain ? resample_encode_launch<true>(x, x_ld, B, S_in, in_lens, table, table_ld, up, down, K, half_len, m0,
+                                             S_out, out, out_ld, encoding, out_lens, gain, stream)
+              : resample_encode_launch<false>(x, x_ld, B, S_in, in_lens, table, table_ld, up, down, K, half_len,
+                                              m0, S_out, out, out_ld, encoding, out_lens, nullptr, stream);
+}
+
+extern "C" int as_resample_encode(const float* x, int64_t x_ld, int32_t B, int32_t S_in, const int32_t* in_lens,
+                                  const float* table, int32_t table_ld, int32_t up, int32_t down, int32_t K,
+                                  int32_t half_len, int32_t m0, int32_t S_out, void* out, int64_t out_ld,
+                                  int32_t encoding, int32_t* out_lens, void* stream) {
+  return as_resample_encode_gain(x, x_ld, B, S_in, in_lens, table, table_ld, up, down, K, half_len, m0, S_out, out,
+                                 out_ld, encoding, out_lens, nullptr, stream);
 }

@@ -45,10 +45,12 @@ class _Captured:
 class _Ticket:
     """A call issued with ``synthesize(..., defer=True)``: with predicted durations everything up to the frame-count
     read-back is enqueued; ``Synthesizer.finish`` synchronises on it and enqueues the rest."""
-    __slots__ = ("result", "last", "last_stream", "slot", "run_stream", "is_side", "ent", "got", "B", "launches", "fmt")
+    __slots__ = ("result", "last", "last_stream", "slot", "run_stream", "is_side", "ent", "got", "B", "launches", "fmt",
+                 "loud")
 
     def __init__(self):
         self.result = self.last = self.last_stream = self.ent = self.got = self.run_stream = self.fmt = None
+        self.loud = None
         self.slot = self.B = self.launches = 0
         self.is_side = False
 
@@ -101,7 +103,12 @@ class Synthesizer:
     ``as_resample_encode`` launch on the call's stream after the graph replay, into a fresh stream-ordered allocation.
     It is not captured, so the format may change on every call without new graphs.  A format equal to the engine's
     native output (24 kHz fp32, or 24 kHz PCM with ``pcm16=True``) takes the unformatted path; any other format needs
-    ``pcm16=False`` (the resampler reads fp32)."""
+    ``pcm16=False`` (the resampler reads fp32).
+
+    **Loudness normalisation.**  ``synthesize(..., loudness=Loudness(target_lufs, max_true_peak_db))`` meters each
+    utterance's 24 kHz waveform on the GPU (BS.1770 integrated loudness and 4x true peak, ``as_loudness_measure``,
+    three launches) and applies one gain per utterance inside the format stage, before the encoding (with the native
+    format too).  Like the format stage it is not captured; it needs ``pcm16=False``."""
 
     def __init__(self, model, generator, device="cuda:0", use_cuda_graph: bool = True, pipeline_depth: int = 1,
                  pcm16: bool = False, acoustic_sms: Optional[int] = None, token_quantum: int = 32,
@@ -331,7 +338,7 @@ class Synthesizer:
     # ---------------------------------------------------------------------------------------
     @torch.no_grad()
     def synthesize(self, tokens, tok_lens, mels, mel_lens, durations=None, voice=None, predict_durations: bool = False,
-                   exact_frames: bool = False, defer: bool = False, prosody=None, audio=None):
+                   exact_frames: bool = False, defer: bool = False, prosody=None, audio=None, loudness=None):
         """``tokens`` int64 [B,Tt] and ``mels`` fp32 [B,80,Tr]: device tensors or (pinned) HOST tensors -- host inputs
         are copied straight into the graph's static buffers; ``tok_lens`` / ``mel_lens`` int64 [B] HOST tensors (or
         lists); ``durations`` int64 [B,Tt] HOST tensor or None (predict them, one device->host sync of B integers);
@@ -348,7 +355,10 @@ class Synthesizer:
         ``durations`` are given); ``last["pred_dur"]`` then holds the scaled durations.
         ``audio``: an ``audio.AudioFormat``; the returned waveforms are then ``[B, audio.out_samples(300*Tm_max)]``
         of ``audio.dtype`` with silence codes beyond each utterance, and ``last["sample_lengths"]`` holds the
-        utterances' sample counts at the target rate (int32, device)."""
+        utterances' sample counts at the target rate (int32, device).
+        ``loudness``: an ``audio.Loudness``; each utterance is then scaled by its normalisation gain before the
+        encoding (in ``audio``'s format, or the native 24 kHz fp32), and ``last["loudness"]``, ``last["true_peak"]``
+        and ``last["gain_db"]`` hold the values measured before the gain (fp64 [B], device)."""
         dev = self.device
         cur = torch.cuda.current_stream(dev)
         self.last_stream = cur
@@ -362,6 +372,9 @@ class Synthesizer:
         Tr = mels.shape[2]
         pros = prosody_mod.check(prosody, tl, durations is not None)
         fmt = self._out_format(audio)
+        loud = audio_mod.check_loudness(loudness, self.pcm16)
+        if loud is not None and fmt is None:
+            fmt = audio_mod.NATIVE
         controlled = pros is not None
         predict = bool(predict_durations) or durations is None
         Tt_b = _ceil_to(Tt, self.token_quantum)
@@ -383,7 +396,7 @@ class Synthesizer:
         if not graphable:
             res = self._eager(tokens, tl, mels, ml, durations, voice, predict, pros)
             if fmt is not None:
-                res = self._format_stage(res, fmt)
+                res = self._format_stage(res, fmt, loud=loud)
             return self._done_ticket(res) if defer else res
         if self._epoch != nn_util.plan_epoch():
             self.drop_graphs()
@@ -446,7 +459,7 @@ class Synthesizer:
                 t.got = torch.cuda.Event()
                 t.got.record(run_stream)
                 t.slot, t.run_stream, t.is_side, t.ent, t.B, t.launches = slot, run_stream, run_stream is not cur, ent, B, launches
-                t.fmt = fmt
+                t.fmt, t.loud = fmt, loud
                 if defer:
                     return t
                 return self.finish(t)
@@ -467,7 +480,7 @@ class Synthesizer:
             self.last = dict(out, frames=[2 * v for v in sums], graph=True)
             res = (out["wav"][:, :HOP * Tm], out["mel_lengths"], out["mel"][:, :, :Tm])
         if fmt is not None:
-            res = self._format_stage(res, fmt, slot if run_stream is not cur else None)
+            res = self._format_stage(res, fmt, slot if run_stream is not cur else None, loud)
         return self._done_ticket(res) if defer else res
 
     def _out_format(self, audio):
@@ -483,21 +496,29 @@ class Synthesizer:
                              f"(AudioFormat(24000, 'pcm16') gives the same samples as pcm16=True)")
         return audio
 
-    def _format_stage(self, res, fmt, side_slot=None):
+    def _format_stage(self, res, fmt, side_slot=None, loud=None):
         """One ``as_resample_encode`` launch on ``last_stream`` after the pass, into a fresh stream-ordered
         allocation; not captured, so it adds no graphs.  ``side_slot``: the pipeline slot whose side stream ran the
-        call (``join`` then also waits for the format stage)."""
+        call (``join`` then also waits for the format stage).  ``loud``: an ``audio.Loudness``; the meter's launches
+        then precede it on the same stream and its gain is applied."""
         wav, mel_lengths, mel = res
         with torch.cuda.stream(self.last_stream):
             n = torch.empty(wav.shape[0], dtype=torch.int32, device=wav.device)
-            y = ops.resample_encode(wav, self.last["wav_lengths"], fmt, fmt.out_samples(wav.shape[1]), out_lens=n)
+            if loud is None:
+                y = ops.resample_encode(wav, self.last["wav_lengths"], fmt, fmt.out_samples(wav.shape[1]), out_lens=n)
+            else:
+                lufs, tp, gain_db, gain = ops.loudness_measure(wav, self.last["wav_lengths"], SAMPLE_RATE,
+                                                               loud.target_lufs, loud.max_true_peak_db)
+                y = ops.resample_encode(wav, self.last["wav_lengths"], fmt, fmt.out_samples(wav.shape[1]), out_lens=n,
+                                        gain=gain)
+                self.last.update(loudness=lufs, true_peak=tp, gain_db=gain_db)
             if side_slot is not None:
                 done = torch.cuda.Event()
                 done.record(self.last_stream)
                 self._slot_done[side_slot] = done
         self.last["sample_lengths"] = n
         if self.last.get("graph"):
-            self.launches_per_call += 1
+            self.launches_per_call += 1 + (ops.LOUDNESS_LAUNCHES if loud is not None else 0)
         return y, mel_lengths, mel
 
     def _done_ticket(self, res):
@@ -542,7 +563,7 @@ class Synthesizer:
                          pred_dur=ent.state["pred_dur"])
         res = (out["wav"][:, :HOP * Tm], out["mel_lengths"], out["mel"][:, :, :Tm])
         if ticket.fmt is not None:
-            res = self._format_stage(res, ticket.fmt, slot if ticket.is_side else None)
+            res = self._format_stage(res, ticket.fmt, slot if ticket.is_side else None, ticket.loud)
         ticket.result, ticket.last, ticket.last_stream = res, self.last, self.last_stream
         return ticket.result
 
@@ -653,7 +674,7 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
                     durations: Optional[Sequence[torch.Tensor]] = None, max_batch: int = 16,
                     max_padded_frames: Optional[int] = 25600, to_host: bool = False, arena: Optional[HostArena] = None,
                     frames_per_token: float = 5.34, prosody: Optional[Sequence["prosody_mod.Prosody"]] = None,
-                    audio: Optional["audio_mod.AudioFormat"] = None):
+                    audio: Optional["audio_mod.AudioFormat"] = None, loudness: Optional["audio_mod.Loudness"] = None):
     """Mixed-length utterances through ``syn`` in length-bucketed ragged micro-batches (BASELINE config 5).
 
     ``tokens[i]`` int64 [Tt_i], ``ref_mels[i]`` fp32 [80, Tr_i], ``durations[i]`` int64 [Tt_i] (host tensors) or
@@ -665,7 +686,8 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     returns: it synchronises the copies).  ``prosody``: one ``prosody.Prosody`` per utterance (or None); the planning
     estimate of an utterance then grows with its mean ``duration_scale``.  ``audio``: an ``audio.AudioFormat`` (see
     ``Synthesizer.synthesize``); ``wavs[i]`` then holds the ``audio.out_samples(300 * frames[i])`` samples of
-    utterance ``i`` in that format."""
+    utterance ``i`` in that format.  ``loudness``: an ``audio.Loudness`` (see ``Synthesizer.synthesize``); each
+    utterance is normalised on its own waveform, so its gain does not depend on its batch-mates."""
     n = len(tokens)
     pros = prosody_mod.check(prosody, [int(t.shape[0]) for t in tokens], durations is not None)
     if durations is not None:
@@ -677,6 +699,10 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     frames: List[int] = list(plan_frames)
     wavs: List[Optional[torch.Tensor]] = [None] * n
     fmt = syn._out_format(audio)
+    loud_kw = {}
+    if loudness is not None:
+        loud_kw["loudness"] = audio_mod.check_loudness(loudness, syn.pcm16)
+        fmt = fmt or audio_mod.NATIVE
     dt = fmt.dtype if fmt is not None else torch.int16 if syn.pcm16 else torch.float32
 
     def cut(f):
@@ -729,7 +755,8 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
         tl = [int(tokens[i].shape[0]) for i in idx]
         ml = [int(ref_mels[i].shape[1]) for i in idx]
         waiting.append((idx, syn.synthesize(tok, tl, mel, ml, dur, defer=True,
-                                            prosody=[pros[i] for i in idx] if pros else None, audio=fmt)))
+                                            prosody=[pros[i] for i in idx] if pros else None, audio=fmt,
+                                            **loud_kw)))
         while len(waiting) > lookahead:
             collect(*waiting.pop(0))
         pending.append((tok, mel))            # pinned inputs must outlive their asynchronous copies
@@ -748,7 +775,7 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     for i in redo:                                         # rare: exact two-graph pass for the utterances that overflowed
         w, _, _ = syn.synthesize(tokens[i].view(1, -1).pin_memory(), [int(tokens[i].shape[0])],
                                  ref_mels[i].unsqueeze(0).pin_memory(), [int(ref_mels[i].shape[1])], None, exact_frames=True,
-                                 prosody=[pros[i]] if pros else None, audio=fmt)
+                                 prosody=[pros[i]] if pros else None, audio=fmt, **loud_kw)
         frames[i] = syn.last["frames"][0]
         with torch.cuda.stream(syn.last_stream):
             wavs[i] = w[0, :cut(frames[i])].clone() if not to_host else w[0, :cut(frames[i])].to("cpu")

@@ -423,12 +423,14 @@ def prosody_apply(f0, n, ema, lens, ctrl, pitch_mean: float, pitch_std: float, e
          float(pitch_mean), float(pitch_std), float(energy_std))
 
 
-def resample_encode(x, lens, fmt, S_out: int, *, m0: int = 0, out=None, out_lens=None):
+def resample_encode(x, lens, fmt, S_out: int, *, m0: int = 0, out=None, out_lens=None, gain=None):
     """Waveforms in an output format (``as_resample_encode``; semantics in ``artspeech_b200.audio``): ``x`` fp32
     [B, S_in] at 24 kHz (unit element stride, any row stride), ``lens`` int32 [B] device sample counts (or None: every
     row holds S_in samples), ``fmt`` an ``audio.AudioFormat``.  Returns ``[B, S_out]`` of ``fmt.dtype``: samples
     ``m0 .. m0 + S_out - 1`` at the target rate, silence beyond each utterance's ``fmt.out_samples(len)``.  ``out``:
-    an optional destination; ``out_lens``: an optional int32 [B] device tensor that receives the output lengths."""
+    an optional destination; ``out_lens``: an optional int32 [B] device tensor that receives the output lengths;
+    ``gain``: an optional fp32 [B] device tensor multiplied into each utterance's samples before they are encoded
+    (``as_resample_encode_gain``)."""
     _require_cuda(x, "resample_encode")
     if x.dtype != torch.float32 or x.dim() != 2 or (x.stride(1) != 1 and x.shape[1] > 1):
         raise _lib.AsError(f"resample_encode: x must be fp32 [B, S] with unit sample stride, got {x.dtype} "
@@ -439,16 +441,53 @@ def resample_encode(x, lens, fmt, S_out: int, *, m0: int = 0, out=None, out_lens
     elif out.dtype != fmt.dtype or tuple(out.shape) != (B, int(S_out)) or (out.stride(1) != 1 and S_out > 1) or \
             out.device != x.device:
         raise _lib.AsError(f"resample_encode: out must be {fmt.dtype} [{B}, {S_out}] on {x.device}")
-    for t, name in ((lens, "lens"), (out_lens, "out_lens")):
-        if t is not None and (t.dtype != torch.int32 or t.device != x.device or t.numel() != B or
+    for t, name, dt in ((lens, "lens", torch.int32), (out_lens, "out_lens", torch.int32),
+                        (gain, "gain", torch.float32)):
+        if t is not None and (t.dtype != dt or t.device != x.device or t.numel() != B or
                               (B > 1 and t.stride(0) != 1)):
-            raise _lib.AsError(f"resample_encode: {name} must be int32 [{B}] on {x.device}")
+            raise _lib.AsError(f"resample_encode: {name} must be {dt} [{B}] on {x.device}")
     table = fmt.device_table(x.device)
     one = lambda n: (int(n) + 15) // 16 * 16           # a single row's stride is free: keep rows 16-byte aligned
-    _run("as_resample_encode", x, x.data_ptr(), x.stride(0) if B > 1 else one(S_in), B, S_in, _p(lens),
-         table.data_ptr(), fmt.table_ld, fmt.up, fmt.down, fmt.K, fmt.half_len, int(m0), int(S_out), out.data_ptr(),
-         out.stride(0) if B > 1 else one(S_out), fmt.code, _p(out_lens))
+    args = (x.data_ptr(), x.stride(0) if B > 1 else one(S_in), B, S_in, _p(lens), table.data_ptr(), fmt.table_ld,
+            fmt.up, fmt.down, fmt.K, fmt.half_len, int(m0), int(S_out), out.data_ptr(),
+            out.stride(0) if B > 1 else one(S_out), fmt.code, _p(out_lens))
+    if gain is None:
+        _run("as_resample_encode", x, *args)
+    else:
+        _run("as_resample_encode_gain", x, *args, gain.data_ptr())
     return out
+
+
+LOUDNESS_LAUNCHES = 3            # AS_LOUDNESS_LAUNCHES
+
+
+def loudness_measure(x, lens, sample_rate: int, target: float = -23.0, ceiling: float = -1.0):
+    """Integrated loudness, true peak and normalisation gain per utterance (``as_loudness_measure``; semantics in
+    ``artspeech_b200.audio``): ``x`` fp32 [B, S] (unit element stride, any row stride) at ``sample_rate`` Hz, ``lens``
+    int32 [B] device sample counts (or None: every row holds S samples).  Returns ``(lufs, true_peak_db, gain_db,
+    gain)``: fp64 [B], fp64 [B], fp64 [B] and fp32 [B] device tensors; ``gain`` is ``10^(gain_db/20)`` rounded once,
+    the factor ``resample_encode(gain=)`` takes.  Three launches, no host synchronisation."""
+    from . import audio
+    _require_cuda(x, "loudness_measure")
+    if x.dtype != torch.float32 or x.dim() != 2 or (x.stride(1) != 1 and x.shape[1] > 1):
+        raise _lib.AsError(f"loudness_measure: x must be fp32 [B, S] with unit sample stride, got {x.dtype} "
+                           f"{tuple(x.shape)} strides {x.stride()}")
+    B, S = x.shape
+    if lens is not None and (lens.dtype != torch.int32 or lens.device != x.device or lens.numel() != B or
+                             (B > 1 and lens.stride(0) != 1)):
+        raise _lib.AsError(f"loudness_measure: lens must be int32 [{B}] on {x.device}")
+    kw = (C.c_double * 10)(*[float(v) for v in audio.k_weighting_taps(sample_rate)])
+    tp = audio.true_peak_table()
+    lufs = torch.empty(B, dtype=torch.float64, device=x.device)
+    tp_db, gain_db = torch.empty_like(lufs), torch.empty_like(lufs)
+    gain = torch.empty(B, dtype=torch.float32, device=x.device)
+    nbytes = _lib.load().as_loudness_workspace_bytes(B, S, int(sample_rate))
+    ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=x.device)
+    _run("as_loudness_measure", x, x.data_ptr(), x.stride(0) if B > 1 else S, B, S, _p(lens), int(sample_rate), kw,
+         tp.ctypes.data_as(_lib.c_f32_p), float(target), float(ceiling), ws.data_ptr(), ws.numel(), lufs.data_ptr(),
+         tp_db.data_ptr(), gain_db.data_ptr(), gain.data_ptr())
+    _count(LOUDNESS_LAUNCHES - 1)
+    return lufs, tp_db, gain_db, gain
 
 
 @dataclass

@@ -305,6 +305,41 @@ int as_resample_encode(const float* x, int64_t x_ld, int32_t B, int32_t S_in, co
                        const float* table, int32_t table_ld, int32_t up, int32_t down, int32_t K, int32_t half_len,
                        int32_t m0, int32_t S_out, void* out, int64_t out_ld, int32_t encoding, int32_t* out_lens,
                        void* stream);
+/* As as_resample_encode, with a per-utterance gain: y[b,m] above is multiplied by gain[b] (fp32 [B], device) in one
+ * fp32 multiply before it is encoded (on the identity path y = x[b,m] * gain[b]); silence codes are unchanged.
+ * gain == NULL is exactly as_resample_encode. */
+int as_resample_encode_gain(const float* x, int64_t x_ld, int32_t B, int32_t S_in, const int32_t* in_lens,
+                            const float* table, int32_t table_ld, int32_t up, int32_t down, int32_t K,
+                            int32_t half_len, int32_t m0, int32_t S_out, void* out, int64_t out_ld, int32_t encoding,
+                            int32_t* out_lens, const float* gain, void* stream);
+
+/* Loudness meter (artspeech_b200/audio.py, ITU-R BS.1770 integrated loudness and 4x true peak) and normalisation
+ * gain, per utterance of n_b = min(lens[b], S) samples (S when lens is NULL) of x [B, >= S] (row stride x_ld) at
+ * fs Hz (a multiple of 10 in [8000, 192000]).  Samples at or beyond n_b are never read.
+ *   K-weighting: two cascaded biquads (transposed direct form II, zero initial state, fp64), kw = {b0, b1, b2, a1,
+ *   a2} of the shelf stage then of the high-pass stage (host array of 10 doubles, audio.k_weighting(fs)).
+ *   Segments of g = fs/10 samples; E_s = sum of y^2 over segment s (fp64).  Blocks j = 0 .. n_b/g - 4:
+ *   z_j = (((E_j + E_{j+1}) + E_{j+2}) + E_{j+3}) / (4 g); when n_b < 4 g a single block z = (sum_s E_s) / n_b.
+ *   L_j = -0.691 + 10 log10 z_j; J_a = {L_j > -70}; G = -0.691 + 10 log10(mean_{J_a} z) - 10;
+ *   J_g = {j in J_a : L_j > G}; loudness = -0.691 + 10 log10(mean_{J_g} z), -inf when J_a is empty or n_b = 0.
+ *   True peak: TP = max(|x_i|, |y4_m|), y4[4q + r] = sum_{j=0..20} tp_table[r][j] * x[q + 10 - j] (one fp32 fma
+ *   chain, x zero outside [0, n_b)), q = 0 .. n_b - 1; tp_table is the [4][AS_LOUDNESS_TP_LD] fp32 polyphase table
+ *   of the 4x resampler (AudioFormat's design with up 4, down 1: 81 taps), a host array.  true_peak = 20 log10 TP
+ *   (-inf for 0).
+ *   gain_db = 0 when loudness is -inf, else min(target - loudness, ceiling - true_peak); gain = fp32(10^(gain_db/20)).
+ * Outputs (device, [B]): loudness_out, true_peak_out, gain_db_out fp64 (gain_db_out may be NULL), gain_out fp32 (may
+ * be NULL).  Three launches; every sum is taken in an order fixed by the utterance's own sample indices, so the results
+ * do not depend on B, S, x_ld or the other utterances.  Lengths are read on the device: no host synchronisation.
+ * workspace: device, at least as_loudness_workspace_bytes(B, S, fs) bytes, 256-byte aligned.  S is limited to
+ * AS_LOUDNESS_MAX_TILES * 8 segments (54 minutes at 24 kHz). */
+#define AS_LOUDNESS_TP_LD 24
+#define AS_LOUDNESS_MAX_TILES 4096
+#define AS_LOUDNESS_LAUNCHES 3
+size_t as_loudness_workspace_bytes(int32_t B, int64_t S, int32_t fs);
+int as_loudness_measure(const float* x, int64_t x_ld, int32_t B, int64_t S, const int32_t* lens, int32_t fs,
+                        const double* kw, const float* tp_table, double target, double ceiling, void* workspace,
+                        size_t workspace_bytes, double* loudness_out, double* true_peak_out, double* gain_db_out,
+                        float* gain_out, void* stream);
 
 /* Direct convolution for tiny input-channel counts (Cin <= 16) on CUDA cores: first layers of the
  * 2-D stacks (1 -> 64, 3x3), F0/N/EMA 1x1 convs of the decoder (models.py:480-482, 502-504).
