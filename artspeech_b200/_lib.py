@@ -140,3 +140,9 @@ SIGNATURES.update({
     "as_loudness_measure": (C.c_int, [_V, _L, _I, _L, _V, _I, C.POINTER(C.c_double), c_f32_p, C.c_double,
                                       C.c_double, _V, C.c_size_t, _V, _V, _V, _V, _V]),
 })
+SIGNATURES.update({
+    "as_watermark_embed": (C.c_int, [_V, _L, _I, _I, _V, _V, _F, _V, _L, _V]),
+    "as_audio_decode": (C.c_int, [_V, _L, _I, _I, _I, _V, _L, _V]),
+    "as_watermark_workspace_bytes": (C.c_size_t, [_I, _I]),
+    "as_watermark_detect": (C.c_int, [_V, _L, _I, _I, _V, _V, _V, _F, _V, C.c_size_t, _V, _V, _V, _V, _V]),
+})

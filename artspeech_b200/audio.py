@@ -1,5 +1,6 @@
 """Output audio formats for synthesis: any integer sample rate by polyphase resampling, and fp32 / 16-bit PCM /
-ITU-T G.711 mu-law and A-law samples, computed on the GPU after the vocoder (``as_resample_encode``).
+ITU-T G.711 mu-law and A-law samples, computed on the GPU after the vocoder (``as_resample_encode``); loudness
+normalisation; and the synthesis watermark.
 
 ``AudioFormat(sample_rate, encoding)`` names a format; the vocoder's own is ``AudioFormat(24000, "float32")``.
 
@@ -52,6 +53,42 @@ of 10 Hz from 8000 to 192000):
    is needed.  A meter run at a lower delivery rate (8 kHz) reads somewhat lower, because the band above that rate's
    Nyquist frequency is removed.  Normalisation sets the overall level, so it overrides the overall-level effect of
    ``Prosody.energy_db`` (the energy contour's shape stays).
+
+**Watermark** (``Watermark(key, message, strength_db)``, ``as_watermark_embed`` / ``as_watermark_detect``).  A mark in
+the samples that says "synthetic" and carries a 16-bit ``message``, keyed by a 64-bit secret ``key``.  Detectors
+deployed later depend on this exact format:
+
+1. **Pattern.**  ``K`` = DFT bins ``k = 154 .. 1740`` of a 4096-point period at 8 kHz (``k 8000 / 4096`` Hz inside
+   [300, 3400] Hz, the telephone band; 1587 bins).  Pattern ``i`` in {0, 1, 2} (sync, data 1, data 2) has the phases
+   ``phi_i(k) = 2 pi h(h(key) ^ (i << 32) ^ k) / 2^64`` with ``h`` splitmix64 (add ``0x9E3779B97F4A7C15``, then
+   ``x ^= x >> 30; x *= 0xBF58476D1CE4E5B9; x ^= x >> 27; x *= 0x94D049BB133111EB; x ^= x >> 31``, mod 2^64).  With
+   ``n`` samples per 0.512 s period, ``c_i^(n)[t] = sqrt(2/|K|) sum_{k in K} cos(2 pi k t / n + phi_i(k))``: unit
+   RMS, band-limited, periodic; ``c^(12288)[3t] = c^(4096)[t]``.
+2. **Embedding** (24 kHz, utterance of ``n`` samples).  ``s1 = message & 255``, ``s2 = message >> 8``;
+   ``c[t] = (c_0[t] + c_1[(t - 48 s1) mod 12288] + c_2[(t - 48 s2) mod 12288]) / sqrt(3)``, computed in fp64 and
+   rounded once to fp32 (``watermark_mark``, cached per key, message and device).  ``e_f`` is the RMS of the
+   240-sample frame ``f`` (10 ms; zeros at and beyond ``n``), ``e(t)`` interpolates linearly between the frame centres
+   ``240 f + 119.5`` and is held beyond the first and last.  ``y[t] = x[t] + (alpha e(t)) c[t mod 12288]`` (one fp32
+   fma) for ``t < n``, ``alpha = 10^(strength_db/20)``, and 0 beyond ``n``.  The mark follows the speech envelope: it
+   vanishes in digital silence and its power relative to the signal is ``strength_db`` (default -30 dB).  It depends
+   only on the utterance's own samples and ``t``.
+3. **Detection** (8 kHz fp32, utterance of ``n`` samples).  (a) ``z[t] = y[t] / e(t)`` where ``e(t) >= 1e-4``, else
+   0, with the envelope of 80-sample frames.  (b) Period ``p`` is ``z[4096 p .. 4096 p + 4095]`` (zeros beyond ``n``),
+   ``Z_p(k)`` its DFT at ``k in K``.  (c) Whitening: ``A(k) = sum_p Z_p(k)``, ``S(k) = sum_p |Z_p(k)|^2``,
+   ``G = A / S`` (0 where ``S = 0``).  (d) ``r_i[tau] = sum_k Re(G(k) e^{-j phi_i(k)} e^{j 2 pi k tau / 4096})`` for
+   every ``tau < 4096``: a crop is a circular lag, found without a search.  (e) ``tau* = argmax |r_0|`` (lowest on
+   ties), ``score = |r_0[tau*]| / sqrt(mean r_0^2)`` (0 when ``r_0`` is 0), ``detected = score >= threshold``
+   (default 6: about 2 4096 Q(6) = 8e-6 false positives per clip under a Gaussian null); polarity and gain do not
+   matter.  (f) ``s_i = argmax_{s < 256} |r_i[(tau* + 16 s) mod 4096]|``, ``message = s1 | s2 << 8``.
+4. **Input formats.**  ``detect_watermark`` decodes PCM16 as ``v / 32768`` and G.711 as ``audioop.ulaw2lin`` /
+   ``alaw2lin`` then ``/ 32768``, and resamples to 8 kHz with this module's resampler (``ToDetectionRate``:
+   ``resample_poly``'s filter for ``8000 / rate``; a ratio whose filter does not fit the kernel is refused).
+5. **Measured robustness** (fp64 reference, tests/test_watermark_cpu.py): seeded speech-like clips of 2-12 s through
+   every ``AudioFormat`` rate and encoding, cropped, polarity-flipped and loudness-normalised, are all detected with
+   their message; unmarked, wrong-key, white-noise and silent clips score at most about 5.  Not covered: lossy codecs
+   (MP3, Opus, AAC), time-stretch, pitch-shift, deliberate removal or forgery (the periodic pattern can be estimated
+   by averaging many marked clips: this is a compliance label, not a security mechanism), listening tests, and
+   ``Generator.stream`` / ``pcm16=True`` engines, which are not marked.
 """
 from __future__ import annotations
 
@@ -303,3 +340,199 @@ def measure_loudness(wav: torch.Tensor, lengths=None, sample_rate: int = NATIVE_
         lengths = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
     lufs, tp, _, _ = ops.loudness_measure(x, lengths, int(sample_rate))
     return lufs, tp
+
+
+# ---- watermark -------------------------------------------------------------------------------------------------
+WM_PERIOD = 4096                 # AS_WM_PERIOD: samples per pattern period at 8 kHz (0.512 s)
+WM_PERIOD_24K = 12288            # AS_WM_PERIOD_24K
+WM_RATE = 8000                   # the detector's rate
+WM_BINS = np.arange(154, 1741)   # AS_WM_K_LO ..: bins k * 8000 / 4096 Hz inside [300, 3400]
+WM_BINS_LD = 1588                # AS_WM_BINS_LD
+WM_SYMBOLS = 256                 # AS_WM_SYMBOLS
+WM_THRESHOLD = 6.0
+_MASK64 = (1 << 64) - 1
+
+
+def splitmix64(x: int) -> int:
+    """One splitmix64 output of the 64-bit state ``x``."""
+    x = (x + 0x9E3779B97F4A7C15) & _MASK64
+    x = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & _MASK64
+    x = ((x ^ (x >> 27)) * 0x94D049BB133111EB) & _MASK64
+    return x ^ (x >> 31)
+
+
+@lru_cache(maxsize=64)
+def watermark_phases(key: int) -> np.ndarray:
+    """fp64 ``[3, 1587]``: ``phi_i(k) = 2 pi h(h(key) ^ (i << 32) ^ k) / 2^64`` of the sync and the two data
+    patterns."""
+    hk = splitmix64(int(key))
+    return np.array([[splitmix64(hk ^ (i << 32) ^ int(k)) for k in WM_BINS] for i in range(3)],
+                    dtype=np.float64) / 2.0 ** 64 * (2.0 * math.pi)
+
+
+def watermark_pattern(key: int, i: int, n: int) -> np.ndarray:
+    """fp64 ``c_i^(n)``: ``sqrt(2/|K|) sum_k cos(2 pi k t / n + phi_i(k))``, ``t < n`` (one period, unit RMS)."""
+    spec = np.zeros(n // 2 + 1, dtype=np.complex128)
+    spec[WM_BINS] = np.exp(1j * watermark_phases(key)[i])
+    return np.fft.irfft(spec, n) * (n / 2.0) * math.sqrt(2.0 / WM_BINS.size)
+
+
+@lru_cache(maxsize=64)
+def watermark_mark(key: int, message: int) -> np.ndarray:
+    """The fp32 24 kHz pattern ``[12288]`` of ``(key, message)``: ``(c_0[t] + c_1[(t - 48 s1) mod 12288] +
+    c_2[(t - 48 s2) mod 12288]) / sqrt(3)`` in fp64, rounded once."""
+    d = WM_PERIOD_24K // WM_SYMBOLS
+    c = (watermark_pattern(key, 0, WM_PERIOD_24K) + np.roll(watermark_pattern(key, 1, WM_PERIOD_24K), (message & 255) * d)
+         + np.roll(watermark_pattern(key, 2, WM_PERIOD_24K), (message >> 8) * d)) / math.sqrt(3.0)
+    return c.astype(np.float32)
+
+
+def watermark_spectra(key: int) -> np.ndarray:
+    """fp32 ``[3, 1588, 2]``: ``e^{-j phi_i(k)}`` of the three patterns (the detector's table; the last row is 0)."""
+    out = np.zeros((3, WM_BINS_LD, 2), dtype=np.float32)
+    ph = watermark_phases(key)
+    out[:, :WM_BINS.size, 0] = np.cos(ph)
+    out[:, :WM_BINS.size, 1] = -np.sin(ph)
+    return out
+
+
+def watermark_twiddles() -> np.ndarray:
+    """fp32 ``[2048, 2]``: ``(cos, -sin)(2 pi m / 4096)`` of the detector's FFT."""
+    a = 2.0 * math.pi * np.arange(WM_PERIOD // 2, dtype=np.float64) / WM_PERIOD
+    return np.stack([np.cos(a), -np.sin(a)], 1).astype(np.float32)
+
+
+_WM_TABLES: Dict[tuple, torch.Tensor] = {}
+
+
+def _wm_table(name, args, device, make):
+    device = torch.device(device)
+    k = (name, args, device)
+    t = _WM_TABLES.get(k)
+    if t is None:
+        if len(_WM_TABLES) >= 256:
+            _WM_TABLES.clear()
+        t = torch.from_numpy(np.ascontiguousarray(make())).to(device)
+        _WM_TABLES[k] = t
+    return t
+
+
+def _int_in(v, lo, hi, what):
+    if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not lo <= int(v) < hi:
+        raise ValueError(f"{what}: expected an integer in [{lo}, {hi}), got {v!r}")
+    return int(v)
+
+
+@dataclass(frozen=True)
+class Watermark:
+    """A keyed watermark for synthesis: 64-bit secret ``key``, 16-bit ``message`` (e.g. a deployment or model-version
+    id) and ``strength_db``, the mark's power relative to the speech (-40 to -15 dB, default -30).  Validated on
+    construction (``ValueError``)."""
+    key: int
+    message: int = 0
+    strength_db: float = -30.0
+
+    def __post_init__(self):
+        object.__setattr__(self, "key", _int_in(self.key, 0, 1 << 64, "Watermark.key"))
+        object.__setattr__(self, "message", _int_in(self.message, 0, 1 << 16, "Watermark.message"))
+        v = self.strength_db
+        if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)) or \
+                not math.isfinite(float(v)) or not -40.0 <= float(v) <= -15.0:
+            raise ValueError(f"Watermark.strength_db: expected a number in [-40, -15], got {v!r}")
+        object.__setattr__(self, "strength_db", float(v))
+
+    @property
+    def alpha(self) -> float:
+        return 10.0 ** (self.strength_db / 20.0)
+
+    def device_pattern(self, device) -> torch.Tensor:
+        """``watermark_mark(key, message)`` on ``device`` (cached per key, message and device)."""
+        return _wm_table("mark", (self.key, self.message), device, lambda: watermark_mark(self.key, self.message))
+
+
+def detector_tables(key: int, device) -> Tuple[torch.Tensor, torch.Tensor]:
+    """(pattern spectra, twiddles) of ``key`` on ``device`` (cached)."""
+    key = _int_in(key, 0, 1 << 64, "key")
+    return (_wm_table("spectra", key, device, lambda: watermark_spectra(key)),
+            _wm_table("twiddles", None, device, watermark_twiddles))
+
+
+def check_watermark(watermark, pcm16: bool):
+    """Validate a ``watermark=`` argument: None or a ``Watermark``; with ``pcm16=True`` a ``ValueError`` (the mark is
+    added to the fp32 waveform)."""
+    if watermark is None:
+        return None
+    if not isinstance(watermark, Watermark):
+        raise ValueError(f"watermark: expected a Watermark, got {type(watermark).__name__}")
+    if pcm16:
+        raise ValueError("watermark= and pcm16=True: the mark is added to the fp32 waveform; use "
+                         "Synthesizer(pcm16=False) with audio=AudioFormat(24000, 'pcm16')")
+    return watermark
+
+
+class ToDetectionRate(AudioFormat):
+    """The detector's resampler: ``sample_rate`` Hz to 8 kHz fp32 with ``resample_poly``'s filter for ``8000 / rate``
+    (``_design``), run by ``as_resample_encode``.  A rate whose filter does not fit the kernel is a ``ValueError``."""
+
+    @property
+    def up(self) -> int:
+        return WM_RATE // math.gcd(self.sample_rate, WM_RATE)
+
+    @property
+    def down(self) -> int:
+        return self.sample_rate // math.gcd(self.sample_rate, WM_RATE)
+
+
+def to_detection_rate(sample_rate: int) -> ToDetectionRate:
+    try:
+        return ToDetectionRate(sample_rate, "float32")
+    except ValueError as e:
+        raise ValueError(f"detect_watermark: cannot resample {sample_rate!r} Hz to 8 kHz: {e}") from None
+
+
+def embed_watermark(wav: torch.Tensor, lengths, wm: Watermark) -> torch.Tensor:
+    """Marked copy of 24 kHz fp32 waveforms ``wav`` ([B, S] or [S], CUDA), as stated in this module's docstring;
+    ``lengths``: per-row sample counts (int tensor or sequence; None: every row holds S samples).  Samples beyond a
+    row's length are 0."""
+    from . import ops
+    if not isinstance(wm, Watermark):
+        raise ValueError(f"embed_watermark: expected a Watermark, got {type(wm).__name__}")
+    x = wav.view(1, -1) if wav.dim() == 1 else wav
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
+    y = ops.watermark_embed(x, lengths, wm)
+    return y.view(-1) if wav.dim() == 1 else y
+
+
+def detect_watermark(x: torch.Tensor, lengths, sample_rate: int, key: int, encoding: str = "float32",
+                     threshold: float = WM_THRESHOLD):
+    """``(detected bool, score fp32, message int32)`` device tensors ``[B]`` of the audio ``x`` ([B, S] or [S], CUDA;
+    fp32, int16 or uint8 for ``encoding`` float32, pcm16, mulaw / alaw) at ``sample_rate`` Hz, for ``key``.  The
+    samples are decoded to fp32 (``ops.audio_decode``), resampled to 8 kHz (``ToDetectionRate``) and detected
+    (``ops.watermark_detect``), as stated in this module's docstring; no host synchronisation."""
+    from . import ops
+    if encoding not in ENCODINGS:
+        raise ValueError(f"detect_watermark: encoding must be one of {ENCODINGS}, got {encoding!r}")
+    if not _rate_ok_any(sample_rate):
+        raise ValueError(f"detect_watermark: sample_rate must be a positive integer, got {sample_rate!r}")
+    key = _int_in(key, 0, 1 << 64, "detect_watermark: key")
+    if isinstance(threshold, bool) or not isinstance(threshold, (int, float)) or not math.isfinite(threshold):
+        raise ValueError(f"detect_watermark: threshold must be a finite number, got {threshold!r}")
+    rs = to_detection_rate(int(sample_rate))
+    x = x.view(1, -1) if x.dim() == 1 else x
+    if x.dtype != DTYPES[encoding]:
+        raise ValueError(f"detect_watermark: {encoding} samples must be {DTYPES[encoding]}, got {x.dtype}")
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
+    if encoding != "float32":
+        x = ops.audio_decode(x, encoding)
+    if not rs.is_identity:
+        n8 = torch.empty(x.shape[0], dtype=torch.int32, device=x.device)
+        x = ops.resample_encode(x, lengths, rs, rs.out_samples(x.shape[1]), out_lens=n8)
+        lengths = n8
+    detected, score, _, message = ops.watermark_detect(x, lengths, key, float(threshold))
+    return detected, score, message
+
+
+def _rate_ok_any(fs) -> bool:
+    return not isinstance(fs, bool) and isinstance(fs, (int, np.integer)) and fs > 0

@@ -3,11 +3,12 @@
 // (test.py:40-47, meldataset.py:42-49) for a batch of reference recordings, one launch.
 //
 // One CTA per frame: reflect-padded, windowed 2048-sample frame -> shared memory in bit-reversed order
-// -> in-place radix-2 FFT (fp32, twiddles from a host-computed table, 11 stages x 4 butterflies per
-// thread) -> power spectrum -> triangular mel filters over each filter's own bin range -> log ->
+// -> in-place radix-2 FFT (fft.cuh: fp32, twiddles from a host-computed table, 11 stages x 4 butterflies
+// per thread) -> power spectrum -> triangular mel filters over each filter's own bin range -> log ->
 // normalise -> [B, n_mels, n_frames] (the reference's channels-first mel layout).  fp32 throughout: a
 // tensor-core DFT in 16-bit operands would bury the bins 60 dB below the frame's peak, which the log brings up.
 #include "common.cuh"
+#include "fft.cuh"
 
 namespace asb {
 
@@ -36,26 +37,10 @@ log_mel_kernel(const float* __restrict__ wave, long long wave_ld, const int* __r
     if (s < 0) s = -s;                                   // reflect padding (torch.stft centre = True)
     if (s >= nb) s = 2 * (nb - 1) - s;
     const float v = (s >= 0 && s < nb) ? wb[s] * window[i] : 0.f;
-    buf[__brev((unsigned)i) >> (32 - FE_LOG2)] = make_float2(v, 0.f);
+    buf[fft_slot<FE_LOG2>(i)] = make_float2(v, 0.f);
   }
   __syncthreads();
-#pragma unroll 1
-  for (int st = 0; st < FE_LOG2; ++st) {
-    const int half = 1 << st;
-    const int tw_step = (FE_NFFT / 2) >> st;
-#pragma unroll
-    for (int j = 0; j < FE_NFFT / 2 / FE_THREADS; ++j) {
-      const int k = tid + j * FE_THREADS;
-      const int pos = k & (half - 1);
-      const int i0 = ((k >> st) << (st + 1)) + pos, i1 = i0 + half;
-      const float2 w = twiddle[pos * tw_step];           // (cos, -sin)(2 pi pos / (2 half))
-      const float2 a = buf[i0], c = buf[i1];
-      const float2 t = make_float2(c.x * w.x - c.y * w.y, c.x * w.y + c.y * w.x);
-      buf[i0] = make_float2(a.x + t.x, a.y + t.y);
-      buf[i1] = make_float2(a.x - t.x, a.y - t.y);
-    }
-    __syncthreads();
-  }
+  fft_radix2<FE_LOG2, FE_THREADS>(buf, twiddle, tid);
   for (int i = tid; i <= FE_NFFT / 2; i += FE_THREADS) power[i] = buf[i].x * buf[i].x + buf[i].y * buf[i].y;
   __syncthreads();
   for (int m = tid; m < n_mels; m += FE_THREADS) {

@@ -29,6 +29,11 @@ def _ceil_to(v: int, q: int) -> int:
     return (int(v) + q - 1) // q * q
 
 
+def _wm_kw(wm) -> dict:
+    """The ``watermark`` keyword of a call that has one: calls without keep their exact signature."""
+    return {} if wm is None else {"wm": wm}
+
+
 class _Captured:
     """One captured CUDA graph with its static inputs / outputs (all owned by the graph's memory pool)."""
     __slots__ = ("graph", "tok", "mels", "voice", "meta", "dur", "lens_t", "mel_lens", "pin_meta", "pin_free", "out",
@@ -46,11 +51,11 @@ class _Ticket:
     """A call issued with ``synthesize(..., defer=True)``: with predicted durations everything up to the frame-count
     read-back is enqueued; ``Synthesizer.finish`` synchronises on it and enqueues the rest."""
     __slots__ = ("result", "last", "last_stream", "slot", "run_stream", "is_side", "ent", "got", "B", "launches", "fmt",
-                 "loud")
+                 "loud", "wm")
 
     def __init__(self):
         self.result = self.last = self.last_stream = self.ent = self.got = self.run_stream = self.fmt = None
-        self.loud = None
+        self.loud = self.wm = None
         self.slot = self.B = self.launches = 0
         self.is_side = False
 
@@ -108,7 +113,12 @@ class Synthesizer:
     **Loudness normalisation.**  ``synthesize(..., loudness=Loudness(target_lufs, max_true_peak_db))`` meters each
     utterance's 24 kHz waveform on the GPU (BS.1770 integrated loudness and 4x true peak, ``as_loudness_measure``,
     three launches) and applies one gain per utterance inside the format stage, before the encoding (with the native
-    format too).  Like the format stage it is not captured; it needs ``pcm16=False``."""
+    format too).  Like the format stage it is not captured; it needs ``pcm16=False``.
+
+    **Watermark.**  ``synthesize(..., watermark=Watermark(key, message))`` adds a keyed, inaudible-by-design mark that
+    ``audio.detect_watermark`` finds in any output format (``as_watermark_embed``, one launch on the call's stream
+    after the graph, before the meter and the format stage, so those see the delivered samples).  It is not captured;
+    with no ``audio`` and no ``loudness`` the marked 24 kHz fp32 waveform is the result.  It needs ``pcm16=False``."""
 
     def __init__(self, model, generator, device="cuda:0", use_cuda_graph: bool = True, pipeline_depth: int = 1,
                  pcm16: bool = False, acoustic_sms: Optional[int] = None, token_quantum: int = 32,
@@ -338,7 +348,8 @@ class Synthesizer:
     # ---------------------------------------------------------------------------------------
     @torch.no_grad()
     def synthesize(self, tokens, tok_lens, mels, mel_lens, durations=None, voice=None, predict_durations: bool = False,
-                   exact_frames: bool = False, defer: bool = False, prosody=None, audio=None, loudness=None):
+                   exact_frames: bool = False, defer: bool = False, prosody=None, audio=None, loudness=None,
+                   watermark=None):
         """``tokens`` int64 [B,Tt] and ``mels`` fp32 [B,80,Tr]: device tensors or (pinned) HOST tensors -- host inputs
         are copied straight into the graph's static buffers; ``tok_lens`` / ``mel_lens`` int64 [B] HOST tensors (or
         lists); ``durations`` int64 [B,Tt] HOST tensor or None (predict them, one device->host sync of B integers);
@@ -358,7 +369,9 @@ class Synthesizer:
         utterances' sample counts at the target rate (int32, device).
         ``loudness``: an ``audio.Loudness``; each utterance is then scaled by its normalisation gain before the
         encoding (in ``audio``'s format, or the native 24 kHz fp32), and ``last["loudness"]``, ``last["true_peak"]``
-        and ``last["gain_db"]`` hold the values measured before the gain (fp64 [B], device)."""
+        and ``last["gain_db"]`` hold the values measured before the gain (fp64 [B], device).
+        ``watermark``: an ``audio.Watermark``; each utterance's 24 kHz waveform is then marked before the meter and the
+        format stage (``audio.embed_watermark`` of the pass's waveform, bit for bit)."""
         dev = self.device
         cur = torch.cuda.current_stream(dev)
         self.last_stream = cur
@@ -373,6 +386,7 @@ class Synthesizer:
         pros = prosody_mod.check(prosody, tl, durations is not None)
         fmt = self._out_format(audio)
         loud = audio_mod.check_loudness(loudness, self.pcm16)
+        wm = audio_mod.check_watermark(watermark, self.pcm16)
         if loud is not None and fmt is None:
             fmt = audio_mod.NATIVE
         controlled = pros is not None
@@ -395,8 +409,8 @@ class Synthesizer:
             graphable = n >= self.capture_after
         if not graphable:
             res = self._eager(tokens, tl, mels, ml, durations, voice, predict, pros)
-            if fmt is not None:
-                res = self._format_stage(res, fmt, loud=loud)
+            if fmt is not None or wm is not None:
+                res = self._format_stage(res, fmt, loud=loud, **_wm_kw(wm))
             return self._done_ticket(res) if defer else res
         if self._epoch != nn_util.plan_epoch():
             self.drop_graphs()
@@ -459,7 +473,7 @@ class Synthesizer:
                 t.got = torch.cuda.Event()
                 t.got.record(run_stream)
                 t.slot, t.run_stream, t.is_side, t.ent, t.B, t.launches = slot, run_stream, run_stream is not cur, ent, B, launches
-                t.fmt, t.loud = fmt, loud
+                t.fmt, t.loud, t.wm = fmt, loud, wm
                 if defer:
                     return t
                 return self.finish(t)
@@ -479,8 +493,8 @@ class Synthesizer:
             Tm = 2 * max(sums)
             self.last = dict(out, frames=[2 * v for v in sums], graph=True)
             res = (out["wav"][:, :HOP * Tm], out["mel_lengths"], out["mel"][:, :, :Tm])
-        if fmt is not None:
-            res = self._format_stage(res, fmt, slot if run_stream is not cur else None, loud)
+        if fmt is not None or wm is not None:
+            res = self._format_stage(res, fmt, slot if run_stream is not cur else None, loud, **_wm_kw(wm))
         return self._done_ticket(res) if defer else res
 
     def _out_format(self, audio):
@@ -496,15 +510,23 @@ class Synthesizer:
                              f"(AudioFormat(24000, 'pcm16') gives the same samples as pcm16=True)")
         return audio
 
-    def _format_stage(self, res, fmt, side_slot=None, loud=None):
+    def _format_stage(self, res, fmt, side_slot=None, loud=None, wm=None):
         """One ``as_resample_encode`` launch on ``last_stream`` after the pass, into a fresh stream-ordered
         allocation; not captured, so it adds no graphs.  ``side_slot``: the pipeline slot whose side stream ran the
         call (``join`` then also waits for the format stage).  ``loud``: an ``audio.Loudness``; the meter's launches
-        then precede it on the same stream and its gain is applied."""
+        then precede it on the same stream and its gain is applied.  ``wm``: an ``audio.Watermark``; one
+        ``as_watermark_embed`` launch first marks the waveform the meter and the format read (``fmt`` None: the marked
+        waveform is the result)."""
         wav, mel_lengths, mel = res
         with torch.cuda.stream(self.last_stream):
-            n = torch.empty(wav.shape[0], dtype=torch.int32, device=wav.device)
-            if loud is None:
+            if wm is not None:
+                wav = ops.watermark_embed(wav, self.last["wav_lengths"], wm)
+                if self.last.get("graph"):
+                    self.launches_per_call += 1
+            n = None if fmt is None else torch.empty(wav.shape[0], dtype=torch.int32, device=wav.device)
+            if fmt is None:
+                y = wav
+            elif loud is None:
                 y = ops.resample_encode(wav, self.last["wav_lengths"], fmt, fmt.out_samples(wav.shape[1]), out_lens=n)
             else:
                 lufs, tp, gain_db, gain = ops.loudness_measure(wav, self.last["wav_lengths"], SAMPLE_RATE,
@@ -516,9 +538,10 @@ class Synthesizer:
                 done = torch.cuda.Event()
                 done.record(self.last_stream)
                 self._slot_done[side_slot] = done
-        self.last["sample_lengths"] = n
-        if self.last.get("graph"):
-            self.launches_per_call += 1 + (ops.LOUDNESS_LAUNCHES if loud is not None else 0)
+        if fmt is not None:
+            self.last["sample_lengths"] = n
+            if self.last.get("graph"):
+                self.launches_per_call += 1 + (ops.LOUDNESS_LAUNCHES if loud is not None else 0)
         return y, mel_lengths, mel
 
     def _done_ticket(self, res):
@@ -562,8 +585,9 @@ class Synthesizer:
         self.last = dict(out, frames=[2 * v for v in sums], graph=True, duration=ent.state["duration"],
                          pred_dur=ent.state["pred_dur"])
         res = (out["wav"][:, :HOP * Tm], out["mel_lengths"], out["mel"][:, :, :Tm])
-        if ticket.fmt is not None:
-            res = self._format_stage(res, ticket.fmt, slot if ticket.is_side else None, ticket.loud)
+        if ticket.fmt is not None or ticket.wm is not None:
+            res = self._format_stage(res, ticket.fmt, slot if ticket.is_side else None, ticket.loud,
+                                     **_wm_kw(ticket.wm))
         ticket.result, ticket.last, ticket.last_stream = res, self.last, self.last_stream
         return ticket.result
 
@@ -674,7 +698,8 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
                     durations: Optional[Sequence[torch.Tensor]] = None, max_batch: int = 16,
                     max_padded_frames: Optional[int] = 25600, to_host: bool = False, arena: Optional[HostArena] = None,
                     frames_per_token: float = 5.34, prosody: Optional[Sequence["prosody_mod.Prosody"]] = None,
-                    audio: Optional["audio_mod.AudioFormat"] = None, loudness: Optional["audio_mod.Loudness"] = None):
+                    audio: Optional["audio_mod.AudioFormat"] = None, loudness: Optional["audio_mod.Loudness"] = None,
+                    watermark: Optional["audio_mod.Watermark"] = None):
     """Mixed-length utterances through ``syn`` in length-bucketed ragged micro-batches (BASELINE config 5).
 
     ``tokens[i]`` int64 [Tt_i], ``ref_mels[i]`` fp32 [80, Tr_i], ``durations[i]`` int64 [Tt_i] (host tensors) or
@@ -687,7 +712,8 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     estimate of an utterance then grows with its mean ``duration_scale``.  ``audio``: an ``audio.AudioFormat`` (see
     ``Synthesizer.synthesize``); ``wavs[i]`` then holds the ``audio.out_samples(300 * frames[i])`` samples of
     utterance ``i`` in that format.  ``loudness``: an ``audio.Loudness`` (see ``Synthesizer.synthesize``); each
-    utterance is normalised on its own waveform, so its gain does not depend on its batch-mates."""
+    utterance is normalised on its own waveform, so its gain does not depend on its batch-mates.  ``watermark``: an
+    ``audio.Watermark`` (see ``Synthesizer.synthesize``); each utterance's mark depends only on its own samples."""
     n = len(tokens)
     pros = prosody_mod.check(prosody, [int(t.shape[0]) for t in tokens], durations is not None)
     if durations is not None:
@@ -703,6 +729,8 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     if loudness is not None:
         loud_kw["loudness"] = audio_mod.check_loudness(loudness, syn.pcm16)
         fmt = fmt or audio_mod.NATIVE
+    if watermark is not None:
+        loud_kw["watermark"] = audio_mod.check_watermark(watermark, syn.pcm16)
     dt = fmt.dtype if fmt is not None else torch.int16 if syn.pcm16 else torch.float32
 
     def cut(f):

@@ -490,6 +490,74 @@ def loudness_measure(x, lens, sample_rate: int, target: float = -23.0, ceiling: 
     return lufs, tp_db, gain_db, gain
 
 
+def _wave_rows(x, name, dtype=torch.float32):
+    if x.dtype != dtype or x.dim() != 2 or (x.stride(1) != 1 and x.shape[1] > 1):
+        raise _lib.AsError(f"{name}: x must be {dtype} [B, S] with unit sample stride, got {x.dtype} "
+                           f"{tuple(x.shape)} strides {x.stride()}")
+    return x.shape
+
+
+def _lens_arg(lens, B, device, name):
+    if lens is not None and (lens.dtype != torch.int32 or lens.device != device or lens.numel() != B or
+                             (B > 1 and lens.stride(0) != 1)):
+        raise _lib.AsError(f"{name}: lens must be int32 [{B}] on {device}")
+    return _p(lens)
+
+
+def watermark_embed(x, lens, wm):
+    """``x`` marked with ``wm`` (an ``audio.Watermark``; ``as_watermark_embed``, semantics in
+    ``artspeech_b200.audio``): ``x`` fp32 [B, S] at 24 kHz (unit element stride, any row stride), ``lens`` int32 [B]
+    device sample counts (or None: every row holds S samples).  Returns a new fp32 [B, S]; zeros beyond each length."""
+    _require_cuda(x, "watermark_embed")
+    B, S = _wave_rows(x, "watermark_embed")
+    out = torch.empty(B, S, dtype=torch.float32, device=x.device)
+    pat = wm.device_pattern(x.device)
+    one = lambda n: (int(n) + 3) // 4 * 4              # a single row's stride is free: keep it a multiple of 4
+    _run("as_watermark_embed", x, x.data_ptr(), x.stride(0) if B > 1 else one(S), B, S,
+         _lens_arg(lens, B, x.device, "watermark_embed"), pat.data_ptr(), float(wm.alpha), out.data_ptr(),
+         out.stride(0) if B > 1 else one(S))
+    return out
+
+
+def audio_decode(x, encoding: str):
+    """fp32 [B, S] samples of encoded ``x`` (``as_audio_decode``): int16 for ``"pcm16"`` (``v / 32768``), uint8
+    G.711 codes for ``"mulaw"`` / ``"alaw"`` (``audioop.ulaw2lin`` / ``alaw2lin``, then ``/ 32768``)."""
+    from . import audio
+    _require_cuda(x, "audio_decode")
+    if encoding not in ("pcm16", "mulaw", "alaw"):
+        raise _lib.AsError(f"audio_decode: encoding must be pcm16, mulaw or alaw, got {encoding!r}")
+    B, S = _wave_rows(x, "audio_decode", audio.DTYPES[encoding])
+    out = torch.empty(B, S, dtype=torch.float32, device=x.device)
+    _run("as_audio_decode", x, x.data_ptr(), x.stride(0) if B > 1 else S, B, S, audio.CODES[encoding],
+         out.data_ptr(), S)
+    return out
+
+
+WATERMARK_DETECT_LAUNCHES = 2    # AS_WM_DETECT_LAUNCHES
+
+
+def watermark_detect(x, lens, key: int, threshold: float = 6.0):
+    """Watermark detection (``as_watermark_detect``; semantics in ``artspeech_b200.audio``) on 8 kHz fp32 ``x``
+    [B, S] (unit element stride, any row stride), ``lens`` int32 [B] device sample counts (or None).  Returns
+    ``(detected bool, score fp32, lag int32, message int32)`` device tensors [B].  Two launches, no host
+    synchronisation."""
+    from . import audio
+    _require_cuda(x, "watermark_detect")
+    B, S = _wave_rows(x, "watermark_detect")
+    spectra, twiddles = audio.detector_tables(key, x.device)
+    score = torch.empty(B, dtype=torch.float32, device=x.device)
+    lag, message = torch.empty(B, dtype=torch.int32, device=x.device), torch.empty(B, dtype=torch.int32,
+                                                                                   device=x.device)
+    detected = torch.empty(B, dtype=torch.bool, device=x.device)
+    nbytes = _lib.load().as_watermark_workspace_bytes(B, S)
+    ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=x.device)
+    _run("as_watermark_detect", x, x.data_ptr(), x.stride(0) if B > 1 else S, B, S,
+         _lens_arg(lens, B, x.device, "watermark_detect"), spectra.data_ptr(), twiddles.data_ptr(), float(threshold),
+         ws.data_ptr(), ws.numel(), score.data_ptr(), lag.data_ptr(), message.data_ptr(), detected.data_ptr())
+    _count(WATERMARK_DETECT_LAUNCHES - 1)
+    return detected, score, lag, message
+
+
 @dataclass
 class SmallConv:
     w: torch.Tensor            # fp32 [ntaps, Cout, Cin] device

@@ -341,6 +341,47 @@ int as_loudness_measure(const float* x, int64_t x_ld, int32_t B, int64_t S, cons
                         size_t workspace_bytes, double* loudness_out, double* true_peak_out, double* gain_db_out,
                         float* gain_out, void* stream);
 
+/* Synthesis watermark (artspeech_b200/audio.py states the format).  Pattern bins k = AS_WM_K_LO ..
+ * AS_WM_K_LO + AS_WM_BINS - 1 of an AS_WM_PERIOD-point period at 8 kHz (300 - 3400 Hz); AS_WM_SYMBOLS lags per symbol.
+ *
+ * as_watermark_embed: y[b,t] = x[b,t] + (alpha e(t)) c[t mod AS_WM_PERIOD_24K] (one fp32 fma) for t < n_b =
+ * min(lens[b], S) (S when lens is NULL), y[b,t] = 0 for n_b <= t < S.  e(t): RMS of the 240-sample frames (zeros at
+ * and beyond n_b), linear between frame centres 240 f + 119.5, held beyond the first and last.  pattern fp32
+ * [AS_WM_PERIOD_24K], 16-byte aligned (audio.Watermark.device_pattern).  x [B, >= S] row stride x_ld; out [B, S]
+ * row stride out_ld, not aliasing x.  Samples at or beyond n_b are never read; lengths are read on the device.  Each
+ * frame's sum has one order, so the result does not depend on B, S, the strides or the batch-mates.  One launch. */
+#define AS_WM_PERIOD 4096
+#define AS_WM_PERIOD_24K 12288
+#define AS_WM_K_LO 154
+#define AS_WM_BINS 1587
+#define AS_WM_BINS_LD 1588
+#define AS_WM_SYMBOLS 256
+#define AS_WM_DETECT_LAUNCHES 2
+int as_watermark_embed(const float* x, int64_t x_ld, int32_t B, int32_t S, const int32_t* lens, const float* pattern,
+                       float alpha, float* out, int64_t out_ld, void* stream);
+
+/* Encoded samples to fp32, elementwise: AS_AUDIO_PCM16 int16 v -> v / 32768; AS_AUDIO_MULAW / AS_AUDIO_ALAW uint8 ->
+ * audioop.ulaw2lin / alaw2lin (width 2) / 32768.  in [B, >= S] row stride in_ld (elements); out fp32 [B, S] row
+ * stride out_ld.  One launch. */
+int as_audio_decode(const void* in, int64_t in_ld, int32_t B, int32_t S, int32_t encoding, float* out, int64_t out_ld,
+                    void* stream);
+
+/* Watermark detector on 8 kHz fp32 utterances x [B, >= S] (row stride x_ld), n_b = min(lens[b], S) (S when NULL):
+ *   z[t] = x[t] / e(t) where e(t) >= 1e-4, else 0 (e as in the embedder with 80-sample frames); Z_p = DFT of
+ *   z[4096 p .. 4096 p + 4095] (zeros beyond n_b) at the pattern bins, p < ceil(n_b / 4096); A = sum_p Z_p,
+ *   S = sum_p |Z_p|^2 (fp32, p in order), G = A / S (0 where S = 0);
+ *   r_i[tau] = sum_k Re(G(k) E_i(k) e^{j 2 pi k tau / 4096}), E_i = spectra[i] = e^{-j phi_i(k)};
+ *   lag = argmax |r_0| (lowest on ties), score = |r_0[lag]| / sqrt(mean r_0^2) (0 when r_0 is 0), detected =
+ *   score >= threshold, message = s_1 | s_2 << 8 with s_i = argmax_{s < 256} |r_i[(lag + 16 s) mod 4096]|.
+ * spectra fp32 [3][AS_WM_BINS_LD][2] (complex, device); twiddles fp32 [2048][2] = (cos, -sin)(2 pi m / 4096) (device).
+ * Outputs (device, [B]): score fp32, lag / message int32, detected uint8.  workspace: device, at least
+ * as_watermark_workspace_bytes(B, S) bytes.  AS_WM_DETECT_LAUNCHES launches, no atomics, no host synchronisation;
+ * every sum's shape follows from n_b alone, so the results do not depend on B, S, x_ld or the batch-mates. */
+size_t as_watermark_workspace_bytes(int32_t B, int32_t S);
+int as_watermark_detect(const float* x, int64_t x_ld, int32_t B, int32_t S, const int32_t* lens, const float* spectra,
+                        const float* twiddles, float threshold, void* workspace, size_t workspace_bytes, float* score,
+                        int32_t* lag, int32_t* message, uint8_t* detected, void* stream);
+
 /* Direct convolution for tiny input-channel counts (Cin <= 16) on CUDA cores: first layers of the
  * 2-D stacks (1 -> 64, 3x3), F0/N/EMA 1x1 convs of the decoder (models.py:480-482, 502-504).
  * x [B,T,F,Cin]; w fp32 [ntaps][Cout][Cin]; taps host arrays; stride 1; zero padding; outputs as
