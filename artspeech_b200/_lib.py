@@ -143,6 +143,10 @@ SIGNATURES.update({
 SIGNATURES.update({
     "as_watermark_embed": (C.c_int, [_V, _L, _I, _I, _V, _V, _F, _V, _L, _V]),
     "as_audio_decode": (C.c_int, [_V, _L, _I, _I, _I, _V, _L, _V]),
+    "as_audio_to_mono": (C.c_int, [_V, _L, _I, _I, _I, _I, _V, _V, _L, _V]),
+    "as_trim_workspace_bytes": (C.c_size_t, [_I, _I]),
+    "as_trim_bounds": (C.c_int, [_V, _L, _I, _I, _V, C.c_double, _V, C.c_size_t, _V, _V]),
+    "as_log_mel_span": (C.c_int, [_V, _L, _V, _V, _I, _I, _V, _V, _V, _V, _I, _I, _I, _F, _F, _F, _V, _I, _V]),
     "as_watermark_workspace_bytes": (C.c_size_t, [_I, _I]),
     "as_watermark_detect": (C.c_int, [_V, _L, _I, _I, _V, _V, _V, _F, _V, C.c_size_t, _V, _V, _V, _V, _V]),
 })

@@ -483,6 +483,30 @@ class ToDetectionRate(AudioFormat):
         return self.sample_rate // math.gcd(self.sample_rate, WM_RATE)
 
 
+class ToNativeRate(AudioFormat):
+    """The enrollment resampler: ``sample_rate`` Hz to the model's 24 kHz fp32 with ``resample_poly``'s filter for
+    ``24000 / rate`` (``_design``), run by ``as_resample_encode``.  A rate whose filter does not fit the kernel is a
+    ``ValueError``.  This is not librosa's default resampler (``soxr_hq``): the two differ in the transition band near
+    12 kHz, which the top mel filters see."""
+
+    @property
+    def up(self) -> int:
+        return NATIVE_RATE // math.gcd(self.sample_rate, NATIVE_RATE)
+
+    @property
+    def down(self) -> int:
+        return self.sample_rate // math.gcd(self.sample_rate, NATIVE_RATE)
+
+
+def to_native_rate(sample_rate) -> ToNativeRate:
+    if not _rate_ok_any(sample_rate):
+        raise ValueError(f"sample_rate must be a positive integer, got {sample_rate!r}")
+    try:
+        return ToNativeRate(int(sample_rate), "float32")
+    except ValueError as e:
+        raise ValueError(f"cannot resample {sample_rate!r} Hz to 24 kHz: {e}") from None
+
+
 def to_detection_rate(sample_rate: int) -> ToDetectionRate:
     try:
         return ToDetectionRate(sample_rate, "float32")

@@ -1,4 +1,5 @@
-// Synthesis watermark (artspeech_b200/audio.py, header: as_watermark_embed / as_audio_decode / as_watermark_detect):
+// Synthesis watermark (artspeech_b200/audio.py, header: as_watermark_embed / as_watermark_detect; the detector's input
+// decoder as_audio_decode is in audio_in.cu):
 // a keyed, band-limited, periodic spread-spectrum pattern added to the vocoder's 24 kHz waveform under its own
 // envelope, and a detector that finds it at 8 kHz at any circular lag (so cropped excerpts need no search).
 //
@@ -111,40 +112,6 @@ __global__ void __launch_bounds__(kWmThreads) wm_embed_kernel(
     }
   } else {
     for (int i = tid; i < nt; i += kWmThreads) ob[t0 + i] = 0.f;
-  }
-}
-
-// CPython audioop.ulaw2lin / alaw2lin, width 2 (st_ulaw2linear16 / st_alaw2linear16)
-__device__ __forceinline__ int wm_ulaw2lin(unsigned u) {
-  u = ~u & 0xFFu;
-  int t = (int)(((u & 0xFu) << 3) + 0x84u);
-  t <<= (u & 0x70u) >> 4;
-  return (u & 0x80u) ? 0x84 - t : t - 0x84;
-}
-
-__device__ __forceinline__ int wm_alaw2lin(unsigned a) {
-  a ^= 0x55u;
-  int t = (int)((a & 0xFu) << 4);
-  const int seg = (int)((a & 0x70u) >> 4);
-  if (seg == 0) t += 8;
-  else if (seg == 1) t += 0x108;
-  else t = (t + 0x108) << (seg - 1);
-  return (a & 0x80u) ? t : -t;
-}
-
-__global__ void __launch_bounds__(kWmThreads) audio_decode_kernel(const void* __restrict__ in, long long in_ld,
-                                                                  int S, int enc, float* __restrict__ out,
-                                                                  long long out_ld) {
-  pdl_wait();
-  const int b = blockIdx.y;
-  for (int i = blockIdx.x * kWmThreads * 4 + threadIdx.x, e = 0; e < 4 && i < S; ++e, i += kWmThreads) {
-    int v;
-    if (enc == AS_AUDIO_PCM16) v = reinterpret_cast<const int16_t*>(in)[(long long)b * in_ld + i];
-    else {
-      const unsigned u = reinterpret_cast<const unsigned char*>(in)[(long long)b * in_ld + i];
-      v = enc == AS_AUDIO_MULAW ? wm_ulaw2lin(u) : wm_alaw2lin(u);
-    }
-    out[(long long)b * out_ld + i] = (float)v * (1.f / 32768.f);
   }
 }
 
@@ -297,20 +264,6 @@ extern "C" int as_watermark_embed(const float* x, int64_t x_ld, int32_t B, int32
   dim3 grid((unsigned)((S + kEmbTile - 1) / kEmbTile), (unsigned)B);
   ASB_CUDA(launch_k(wm_embed_kernel, grid, dim3(kWmThreads), 0, static_cast<cudaStream_t>(stream), x,
                     (long long)x_ld, (int)S, lens, pattern, alpha, out, (long long)out_ld, vec_in, vec_out));
-  return AS_OK;
-}
-
-extern "C" int as_audio_decode(const void* in, int64_t in_ld, int32_t B, int32_t S, int32_t encoding, float* out,
-                               int64_t out_ld, void* stream) {
-  if (B == 0 || S == 0) return AS_OK;
-  ASB_REQUIRE(in && out && B > 0 && S > 0 && in_ld >= S && out_ld >= S && B <= 65535, AS_ERR_SHAPE,
-              "as_audio_decode: bad argument");
-  ASB_REQUIRE(encoding == AS_AUDIO_PCM16 || encoding == AS_AUDIO_MULAW || encoding == AS_AUDIO_ALAW, AS_ERR_DTYPE,
-              "as_audio_decode: encoding %d is not PCM16, mu-law or A-law", (int)encoding);
-  if (int rc = check_arch()) return rc;
-  dim3 grid((unsigned)((S + kWmThreads * 4 - 1) / (kWmThreads * 4)), (unsigned)B);
-  ASB_CUDA(launch_k(audio_decode_kernel, grid, dim3(kWmThreads), 0, static_cast<cudaStream_t>(stream), in,
-                    (long long)in_ld, (int)S, (int)encoding, out, (long long)out_ld));
   return AS_OK;
 }
 

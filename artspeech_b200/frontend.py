@@ -6,17 +6,52 @@ The transform's constants (periodic Hann window zero-padded to ``n_fft``, HTK tr
 torchaudio's default ``sample_rate=16000`` — the reference never passes its 24 kHz rate, which is kept for
 checkpoint compatibility — and the FFT twiddles) are computed once on the host; the arithmetic is one
 launch of ``as_log_mel`` (``csrc/frontend.cu``) for a whole batch of recordings.
+
+**Voice enrollment from recordings** (``reference_mels``, ``Synthesizer.enroll``): what the reference does to a
+reference recording before that log-mel (``test.py:100-108``: ``librosa.load(path, sr=24000)``,
+``librosa.effects.trim(wave, top_db=30)``, ``preprocess``), on the GPU.  Input: a batch of B recordings, ``x`` ``[B, S]``
+(mono) or ``[B, S, C]`` (C interleaved channels, 1 <= C <= 8); ``lengths[b] <= S`` samples per channel at
+``sample_rate`` Hz; ``encoding`` ``float32``, ``pcm16``, ``mulaw`` or ``alaw`` (the dtypes of ``audio.DTYPES``).
+
+1. **Decode and downmix** (``as_audio_to_mono``).  Each sample is decoded as ``audio.detect_watermark`` decodes
+   (``v / 32768``, or ``audioop.ulaw2lin`` / ``alaw2lin`` then ``/ 32768``), then ``m[t] = (x_0[t] + ... +
+   x_{C-1}[t]) / C``: an fp32 sum in channel order and one fp32 divide, numpy's float32 ``mean(axis=0)`` that
+   librosa's ``to_mono`` uses.  fp32 mono input takes no launch.
+2. **Resample to 24 kHz** (``audio.ToNativeRate``, ``as_resample_encode``).  ``resample_poly``'s filter for
+   ``24000 / rate``; ``n24 = ceil(n up / down)`` samples.  24 kHz takes no launch; a rate whose filter does not fit
+   the kernel is a ``ValueError`` (8, 11.025, 12, 16, 22.05, 32, 44.1, 48, 88.2, 96 and 192 kHz fit).  This is not
+   librosa's resampler (``soxr_hq``): the two differ in the transition band near 12 kHz, which the top mel filters see.
+3. **Trim** (``as_trim_bounds``; ``top_db``, default 30, ``None`` for no trim).  librosa 0.10's ``effects.trim``
+   with its defaults (frame 2048, hop 512), evaluated at 24 kHz in fp64: ``q_j`` is the sum of ``y^2`` over block
+   ``[512 j, 512 j + 512)`` (zeros at and beyond ``n``); frame ``f < F = 1 + n // 512`` has the power
+   ``p_f = (q_{f-2} + q_{f-1} + q_f + q_{f+1}) / 2048`` (blocks out of range count 0: ``feature.rms(center=True,
+   pad_mode="constant")`` squared); ``P = max_f p_f``; frame ``f`` is non-silent iff ``10 log10(max(1e-10, p_f)) -
+   10 log10(max(1e-10, P)) > -top_db`` (``amplitude_to_db(ref=np.max, amin=1e-5)``); ``start = 512 first``,
+   ``end = min(n, 512 (last + 1))``, and ``(0, 0)`` for ``n = 0``.  As in librosa, digital silence is entirely
+   non-silent and keeps ``(0, n)``.  The one known difference: librosa sums in fp32, so a frame within about 1e-6 dB
+   of the threshold can be decided differently.
+4. **Log-mel of the span** (``as_log_mel_span``).  Exactly ``LogMel`` of ``y[start:end]``, reflect-padded at the
+   span's own ends: ``1 + L // 300`` frames for ``L = end - start``.  A row with ``L <= 1024`` is a ``ValueError``
+   naming the row (``torch.stft``'s reflect padding, and so the reference, cannot take it).
+
+Outputs: ``mels`` fp32 ``[B, 80, T_max]`` with zeros beyond each row's frames, ``mel_lens`` int64 ``[B]`` on the host
+(what ``synthesize`` / ``encode_voice`` take), ``bounds`` int32 ``[B, 2]`` on the device, ``(start, end)`` in 24 kHz
+samples.  A row's outputs depend only on its own samples, bit for bit: not on the batch, the padding or the row
+stride.  The call makes at most five launches and one device-to-host read-back (the B bounds, into pinned memory,
+between the trim and the log-mel: it sizes ``T_max`` and finds short rows).  Container formats (WAV, FLAC, MP3
+headers) are the caller's: it hands over sample arrays.
 """
 from __future__ import annotations
 
 import math
-from typing import Optional
+import numbers
+from typing import Optional, Sequence, Union
 
 import numpy as np
 import torch
 import torch.nn as nn
 
-from . import _lib, ops
+from . import _lib, audio, ops
 
 N_FFT, WIN_LENGTH, HOP_LENGTH, N_MELS = 2048, 1200, 300, 80
 LOG_EPS, MEAN, STD = 1e-5, -4.0, 4.0
@@ -55,7 +90,11 @@ def filter_ranges(fb: torch.Tensor) -> torch.Tensor:
 
 
 class LogMel(nn.Module):
-    """``forward(wave [B, N] fp32 CUDA, lengths=None) -> [B, 80, 1 + N // 300]`` normalised log-mel."""
+    """``forward(wave [B, N] fp32 CUDA, lengths=None) -> [B, 80, 1 + N // 300]`` normalised log-mel.
+
+    ``starts=`` (int32 [B] device, with ``lengths``) takes recording ``b`` as the ``lengths[b]`` samples from
+    ``wave[b, starts[b]]`` (``as_log_mel_span``), with the bits ``LogMel`` gives for those samples copied to the start
+    of a row; ``n_frames`` then sets the output's frame count (default ``1 + N // 300``)."""
 
     def __init__(self, n_mels: int = N_MELS, n_fft: int = N_FFT, win_length: int = WIN_LENGTH,
                  hop_length: int = HOP_LENGTH, mean: float = MEAN, std: float = STD):
@@ -72,7 +111,8 @@ class LogMel(nn.Module):
         self.register_buffer("twiddle", torch.from_numpy(tw.astype(np.float32)).contiguous(), persistent=False)
 
     @torch.no_grad()
-    def forward(self, wave: torch.Tensor, lengths: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward(self, wave: torch.Tensor, lengths: Optional[torch.Tensor] = None,
+                starts: Optional[torch.Tensor] = None, n_frames: Optional[int] = None) -> torch.Tensor:
         ops._require_cuda(wave, "log_mel")
         if wave.dim() == 1:
             wave = wave.unsqueeze(0)
@@ -80,12 +120,21 @@ class LogMel(nn.Module):
         if wave.stride(-1) != 1:
             wave = wave.contiguous()
         B, N = wave.shape
-        n_frames = 1 + N // self.hop_length
+        if n_frames is None:
+            n_frames = 1 + N // self.hop_length
         out = torch.empty(B, self.n_mels, n_frames, dtype=torch.float32, device=wave.device)
-        lens = None if lengths is None else lengths.to(device=wave.device, dtype=torch.int32)
-        ops._run("as_log_mel", wave, wave.data_ptr(), wave.stride(0), ops._p(lens), B, N, self.window.data_ptr(),
-                 self.twiddle.data_ptr(), self.fb.data_ptr(), self.fb_range.data_ptr(), self.n_fft, self.hop_length,
-                 self.n_mels, float(LOG_EPS), float(self.mean), float(self.std), out.data_ptr(), n_frames)
+        lens = None if lengths is None else lengths.to(device=wave.device, dtype=torch.int32).contiguous()
+        consts = (self.window.data_ptr(), self.twiddle.data_ptr(), self.fb.data_ptr(), self.fb_range.data_ptr(),
+                  self.n_fft, self.hop_length, self.n_mels, float(LOG_EPS), float(self.mean), float(self.std),
+                  out.data_ptr(), n_frames)
+        if starts is None:
+            ops._run("as_log_mel", wave, wave.data_ptr(), wave.stride(0), ops._p(lens), B, N, *consts)
+        else:
+            if lens is None:
+                raise ValueError("LogMel: starts= needs lengths")
+            st = starts.to(device=wave.device, dtype=torch.int32).contiguous()
+            ops._run("as_log_mel_span", wave, wave.data_ptr(), wave.stride(0), st.data_ptr(), lens.data_ptr(), B, N,
+                     *consts)
         return out
 
 
@@ -99,3 +148,117 @@ def preprocess(wave, device="cuda") -> torch.Tensor:
         _default[dev] = LogMel().to(dev)
     w = torch.from_numpy(wave) if isinstance(wave, np.ndarray) else wave
     return _default[dev](w.to(dev))
+
+
+# ---- voice enrollment from recordings -----------------------------------------------------------------------------
+MIN_SPAN = N_FFT // 2            # a trimmed span must be longer than this (reflect padding of the first frame)
+
+
+def _check_top_db(top_db):
+    if top_db is None:
+        return None
+    if isinstance(top_db, bool) or not isinstance(top_db, numbers.Real) or not math.isfinite(float(top_db)) or \
+            float(top_db) <= 0.0:
+        raise ValueError(f"top_db must be a finite positive number or None, got {top_db!r}")
+    return float(top_db)
+
+
+def trim_bounds(wave: torch.Tensor, lengths=None, top_db: float = 30.0) -> torch.Tensor:
+    """``(start, end)`` int32 ``[B, 2]`` device tensor of the non-silent span of each row of 24 kHz fp32 ``wave``
+    (``[B, S]`` or ``[S]``, CUDA) as step 3 of this module's docstring states; ``lengths``: per-row sample counts (int
+    tensor or sequence; None: every row holds S samples).  Two launches, no host synchronisation."""
+    top_db = _check_top_db(top_db)
+    if top_db is None:
+        raise ValueError("trim_bounds: top_db must be a finite positive number")
+    x = wave.view(1, -1) if wave.dim() == 1 else wave
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
+    return ops.trim_bounds(x, lengths, top_db)
+
+
+def _read_back(t: torch.Tensor) -> torch.Tensor:
+    """Host copy of a small device tensor through pinned memory: the one synchronisation of ``reference_mels``."""
+    if not t.is_cuda:
+        return t.clone()
+    h = torch.empty(t.shape, dtype=t.dtype).pin_memory()
+    h.copy_(t, non_blocking=True)
+    torch.cuda.current_stream(t.device).synchronize()
+    return h
+
+
+def _host_lengths(lengths, B: int, S: int) -> torch.Tensor:
+    if lengths is None:
+        return torch.full((B,), S, dtype=torch.int64)
+    if isinstance(lengths, torch.Tensor):
+        if lengths.is_cuda:
+            raise ValueError("lengths: expected a host tensor or sequence (reading a device tensor would synchronise)")
+        if lengths.is_floating_point() or lengths.dtype == torch.bool:
+            raise ValueError(f"lengths: expected integers, got {lengths.dtype}")
+        L = lengths.to(torch.int64).flatten()
+    else:
+        vals = list(lengths)
+        if any(isinstance(v, bool) or not isinstance(v, (numbers.Integral, np.integer)) for v in vals):
+            raise ValueError(f"lengths: expected integers, got {vals!r}")
+        L = torch.tensor([int(v) for v in vals], dtype=torch.int64)
+    if L.numel() != B:
+        raise ValueError(f"lengths: expected {B} values, got {L.numel()}")
+    if B and (int(L.min()) < 0 or int(L.max()) > S):
+        raise ValueError(f"lengths: every length must be in [0, {S}], got {L.tolist()}")
+    return L
+
+
+_enroll_logmel = {}
+
+
+def reference_mels(x: torch.Tensor, lengths: Union[Sequence[int], torch.Tensor, None], sample_rate: int,
+                   encoding: str = "float32", top_db: Optional[float] = 30.0, device=None):
+    """Reference mels of recordings, as this module's docstring states: ``x`` ``[B, S]`` or ``[B, S, C]`` (host or
+    CUDA) of ``audio.DTYPES[encoding]`` at ``sample_rate`` Hz, ``lengths`` host samples per channel (None: S).
+    Returns ``(mels fp32 [B, 80, T_max] device, mel_lens int64 [B] host, bounds int32 [B, 2] device)``.  ``device``:
+    where to run when ``x`` is on the host (default ``cuda``).  At most five launches, one read-back."""
+    if encoding not in audio.ENCODINGS:
+        raise ValueError(f"encoding must be one of {audio.ENCODINGS}, got {encoding!r}")
+    rs = audio.to_native_rate(sample_rate)
+    top_db = _check_top_db(top_db)
+    if not isinstance(x, torch.Tensor) or x.dim() not in (2, 3):
+        raise ValueError(f"x: expected a [B, S] or [B, S, C] tensor, got {getattr(x, 'shape', type(x))}")
+    if x.dtype != audio.DTYPES[encoding]:
+        raise ValueError(f"x: {encoding} samples must be {audio.DTYPES[encoding]}, got {x.dtype}")
+    B, S = x.shape[:2]
+    C = x.shape[2] if x.dim() == 3 else 1
+    if not 1 <= C <= 8:
+        raise ValueError(f"x: 1 to 8 interleaved channels, got {C}")
+    n = _host_lengths(lengths, B, S)
+    dev = x.device if x.is_cuda else torch.device(device if device is not None else "cuda")
+    if B == 0:
+        return (torch.zeros(0, N_MELS, 0, device=dev), torch.zeros(0, dtype=torch.int64),
+                torch.zeros(0, 2, dtype=torch.int32, device=dev))
+    if not x.is_cuda:
+        x = x.contiguous().to(dev, non_blocking=False)
+    lens = n.to(torch.int32).to(dev)
+    m = x if x.dim() == 2 else x[..., 0]
+    if encoding != "float32" or C > 1:
+        m = ops.audio_to_mono(x, lens, encoding)
+    if rs.is_identity:
+        y, n24, n24_host = m, lens, n
+    else:
+        n24 = torch.empty(B, dtype=torch.int32, device=dev)
+        y = ops.resample_encode(m, lens, rs, rs.out_samples(S), out_lens=n24)
+        n24_host = torch.tensor([rs.out_samples(int(v)) for v in n], dtype=torch.int64)
+    if top_db is None:
+        host = torch.stack([torch.zeros_like(n24_host), n24_host], 1).to(torch.int32)
+        bounds = host.to(dev)
+    else:
+        bounds = ops.trim_bounds(y, n24, top_db)
+        host = _read_back(bounds)
+    span = (host[:, 1] - host[:, 0]).to(torch.int64)
+    short = [b for b in range(B) if int(span[b]) <= MIN_SPAN]
+    if short:
+        raise ValueError(f"reference_mels: rows {short} keep {[int(span[b]) for b in short]} samples at 24 kHz after "
+                         f"the trim; a log-mel needs more than {MIN_SPAN}")
+    mel_lens = 1 + span // HOP_LENGTH
+    starts_lens = torch.stack([host[:, 0], span.to(torch.int32)]).to(dev)
+    if dev not in _enroll_logmel:
+        _enroll_logmel[dev] = LogMel().to(dev)
+    mels = _enroll_logmel[dev](y, starts_lens[1], starts=starts_lens[0], n_frames=int(mel_lens.max()))
+    return mels, mel_lens, bounds

@@ -533,6 +533,49 @@ def audio_decode(x, encoding: str):
     return out
 
 
+def audio_to_mono(x, lens, encoding: str):
+    """Mono fp32 [B, S] of encoded samples ``x`` (``as_audio_to_mono``; semantics in ``artspeech_b200.frontend``):
+    ``x`` [B, S] (one channel) or [B, S, C] (C interleaved channels, 1 <= C <= 8), float32 / int16 / uint8 for
+    ``encoding`` float32 / pcm16 / mulaw, alaw; unit element stride, dense channels, any row stride.  ``lens`` int32
+    [B] device samples per channel (or None: every row holds S).  Output ``(x_0 + ... + x_{C-1}) / C`` of the decoded
+    samples, zeros beyond each length.  One launch, no host synchronisation."""
+    from . import audio
+    _require_cuda(x, "audio_to_mono")
+    if encoding not in audio.ENCODINGS:
+        raise _lib.AsError(f"audio_to_mono: encoding must be one of {audio.ENCODINGS}, got {encoding!r}")
+    if x.dtype != audio.DTYPES[encoding] or x.dim() not in (2, 3):
+        raise _lib.AsError(f"audio_to_mono: x must be {audio.DTYPES[encoding]} [B, S] or [B, S, C], got {x.dtype} "
+                           f"{tuple(x.shape)}")
+    B, S = x.shape[:2]
+    C_ = x.shape[2] if x.dim() == 3 else 1
+    if x.dim() == 3 and (x.stride(2) != 1 and C_ > 1 or x.stride(1) != C_ and S > 1):
+        raise _lib.AsError(f"audio_to_mono: channels must be interleaved densely, strides {x.stride()}")
+    if x.dim() == 2 and x.stride(1) != 1 and S > 1:
+        raise _lib.AsError(f"audio_to_mono: x must have unit sample stride, strides {x.stride()}")
+    out = torch.empty(B, S, dtype=torch.float32, device=x.device)
+    _run("as_audio_to_mono", x, x.data_ptr(), x.stride(0) if B > 1 else S * C_, B, S, C_, audio.CODES[encoding],
+         _lens_arg(lens, B, x.device, "audio_to_mono"), out.data_ptr(), S)
+    return out
+
+
+TRIM_LAUNCHES = 2                # AS_TRIM_LAUNCHES
+
+
+def trim_bounds(y, lens, top_db: float):
+    """Leading / trailing silence of 24 kHz fp32 ``y`` [B, S] (unit element stride, any row stride; ``as_trim_bounds``,
+    semantics in ``artspeech_b200.frontend``), ``lens`` int32 [B] device sample counts (or None).  Returns int32
+    [B, 2] device ``(start, end)``.  Two launches, no host synchronisation."""
+    _require_cuda(y, "trim_bounds")
+    B, S = _wave_rows(y, "trim_bounds")
+    bounds = torch.empty(B, 2, dtype=torch.int32, device=y.device)
+    nbytes = _lib.load().as_trim_workspace_bytes(B, S)
+    ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=y.device)
+    _run("as_trim_bounds", y, y.data_ptr(), y.stride(0) if B > 1 else S, B, S, _lens_arg(lens, B, y.device,
+         "trim_bounds"), float(top_db), ws.data_ptr(), ws.numel(), bounds.data_ptr())
+    _count(TRIM_LAUNCHES - 1)
+    return bounds
+
+
 WATERMARK_DETECT_LAUNCHES = 2    # AS_WM_DETECT_LAUNCHES
 
 

@@ -362,9 +362,35 @@ int as_watermark_embed(const float* x, int64_t x_ld, int32_t B, int32_t S, const
 
 /* Encoded samples to fp32, elementwise: AS_AUDIO_PCM16 int16 v -> v / 32768; AS_AUDIO_MULAW / AS_AUDIO_ALAW uint8 ->
  * audioop.ulaw2lin / alaw2lin (width 2) / 32768.  in [B, >= S] row stride in_ld (elements); out fp32 [B, S] row
- * stride out_ld.  One launch. */
+ * stride out_ld.  One launch: as_audio_to_mono with C = 1 and no lengths. */
 int as_audio_decode(const void* in, int64_t in_ld, int32_t B, int32_t S, int32_t encoding, float* out, int64_t out_ld,
                     void* stream);
+
+/* Encoded samples with C interleaved channels (1 <= C <= AS_AUDIO_MAX_CHANNELS) to mono fp32 (voice enrollment,
+ * artspeech_b200/frontend.py):  out[b,t] = (d(x[b, t C]) + ... + d(x[b, t C + C - 1])) / C, an fp32 sum in channel
+ * order then one fp32 divide (numpy's float32 mean over the channels), for t < n_b = min(lens[b], S) (S when lens is
+ * NULL); out[b,t] = 0 for n_b <= t < S.  d decodes as as_audio_decode (AS_AUDIO_F32: the value itself).  in [B,
+ * >= S C] elements of the encoding's type with row stride in_ld (elements); out fp32 [B, S] row stride out_ld, not
+ * aliasing in.  Samples at or beyond n_b are never read; lengths are read on the device.  One launch. */
+#define AS_AUDIO_MAX_CHANNELS 8
+int as_audio_to_mono(const void* in, int64_t in_ld, int32_t B, int32_t S, int32_t C, int32_t encoding,
+                     const int32_t* lens, float* out, int64_t out_ld, void* stream);
+
+/* Leading / trailing silence of 24 kHz fp32 utterances (librosa 0.10 effects.trim with frame 2048, hop 512),
+ * y [B, >= S] row stride y_ld, n_b = min(lens[b], S) (S when lens is NULL):
+ *   q_j = sum of y^2 over block j = [512 j, 512 j + 512) in fp64, zeros at and beyond n_b;
+ *   p_f = (((q_{f-2} + q_{f-1}) + q_f) + q_{f+1}) / 2048 for frames f < F = 1 + n_b / 512 (blocks outside
+ *   [0, ceil(n_b / 512)) count as 0): the squared RMS of librosa's centred, zero-padded frames;
+ *   P = max_f p_f; frame f is non-silent iff 10 log10(max(1e-10, p_f)) - 10 log10(max(1e-10, P)) > -top_db;
+ *   bounds[b] = (512 first, min(n_b, 512 (last + 1))) over the non-silent frames; (0, 0) when n_b = 0.
+ * bounds int32 [B][2] (device).  Two launches (block sums, then one CTA per utterance), no atomics, no host
+ * synchronisation; every sum's shape follows from n_b alone, so the bounds do not depend on B, S, y_ld or the
+ * batch-mates.  Samples at or beyond n_b are never read.  workspace: device, at least
+ * as_trim_workspace_bytes(B, S) bytes, 8-byte aligned.  top_db finite and positive. */
+#define AS_TRIM_LAUNCHES 2
+size_t as_trim_workspace_bytes(int32_t B, int32_t S);
+int as_trim_bounds(const float* y, int64_t y_ld, int32_t B, int32_t S, const int32_t* lens, double top_db,
+                   void* workspace, size_t workspace_bytes, int32_t* bounds, void* stream);
 
 /* Watermark detector on 8 kHz fp32 utterances x [B, >= S] (row stride x_ld), n_b = min(lens[b], S) (S when NULL):
  *   z[t] = x[t] / e(t) where e(t) >= 1e-4, else 0 (e as in the embedder with 80-sample frames); Z_p = DFT of
@@ -460,6 +486,13 @@ int as_log_mel(const float* wave, int64_t wave_ld, const int32_t* lens, int32_t 
                const float* window, const float* twiddle, const float* fb, const int32_t* fb_range,
                int32_t n_fft, int32_t hop, int32_t n_mels, float log_eps, float mean, float std,
                float* out, int32_t n_frames, void* stream);
+/* as_log_mel of a span of each row: recording b is the lens[b] samples wave[b * wave_ld + starts[b] ...] (both int32
+ * [B], device, required), reflect-padded at the span's own ends; starts[b] + lens[b] <= N.  The arithmetic is
+ * as_log_mel's: a span gives the bits as_log_mel gives for the same samples copied to the start of a row. */
+int as_log_mel_span(const float* wave, int64_t wave_ld, const int32_t* starts, const int32_t* lens, int32_t B,
+                    int32_t N, const float* window, const float* twiddle, const float* fb, const int32_t* fb_range,
+                    int32_t n_fft, int32_t hop, int32_t n_mels, float log_eps, float mean, float std, float* out,
+                    int32_t n_frames, void* stream);
 
 #ifdef __cplusplus
 }
