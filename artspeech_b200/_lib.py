@@ -149,4 +149,7 @@ SIGNATURES.update({
     "as_log_mel_span": (C.c_int, [_V, _L, _V, _V, _I, _I, _V, _V, _V, _V, _I, _I, _I, _F, _F, _F, _V, _I, _V]),
     "as_watermark_workspace_bytes": (C.c_size_t, [_I, _I]),
     "as_watermark_detect": (C.c_int, [_V, _L, _I, _I, _V, _V, _V, _F, _V, C.c_size_t, _V, _V, _V, _V, _V]),
+    "as_denoise_workspace_bytes": (C.c_size_t, [_I, _I]),
+    "as_denoise": (C.c_int, [_V, _L, _I, _I, _V, C.c_double, _V, _V, _V, C.c_double, C.c_double, C.c_double,
+                             C.c_double, _V, C.c_size_t, _V, _L, _V]),
 })

@@ -172,14 +172,16 @@ class Synthesizer:
                                               host_lengths=ml))
 
     @torch.no_grad()
-    def enroll(self, x, lengths, sample_rate: int, encoding: str = "float32", top_db: Optional[float] = 30.0):
-        """Voices from recordings: ``frontend.reference_mels`` (decode, downmix, resample to 24 kHz, trim silence,
-        log-mel; semantics in ``artspeech_b200.frontend``) then ``encode_voice``, eagerly.  ``x`` ``[B, S]`` or
-        ``[B, S, C]`` samples of ``encoding`` at ``sample_rate`` Hz, ``lengths`` host samples per channel.  Returns
-        ``(mels, mel_lens, voice)``, which ``synthesize(tokens, tok_lens, mels, mel_lens, voice=voice)`` takes as they
-        are."""
+    def enroll(self, x, lengths, sample_rate: int, encoding: str = "float32", top_db: Optional[float] = 30.0,
+               noise_reduction_db: Optional[float] = None):
+        """Voices from recordings: ``frontend.reference_mels`` (decode, downmix, resample to 24 kHz, optionally reduce
+        stationary noise by up to ``noise_reduction_db``, trim silence, log-mel; semantics in
+        ``artspeech_b200.frontend``) then ``encode_voice``, eagerly.  ``x`` ``[B, S]`` or ``[B, S, C]`` samples of
+        ``encoding`` at ``sample_rate`` Hz, ``lengths`` host samples per channel.  Returns ``(mels, mel_lens, voice)``,
+        which ``synthesize(tokens, tok_lens, mels, mel_lens, voice=voice)`` takes as they are."""
         from . import frontend
-        mels, mel_lens, _ = frontend.reference_mels(x, lengths, sample_rate, encoding, top_db, device=self.device)
+        mels, mel_lens, _ = frontend.reference_mels(x, lengths, sample_rate, encoding, top_db, device=self.device,
+                                                    noise_reduction_db=noise_reduction_db)
         return mels, mel_lens, self.encode_voice(mels, mel_lens)
 
     # -- the two phases (models.ArtsSpeech.encode / decode + the vocoder) ---------------------------------------

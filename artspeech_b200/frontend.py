@@ -21,6 +21,32 @@ reference recording before that log-mel (``test.py:100-108``: ``librosa.load(pat
    ``24000 / rate``; ``n24 = ceil(n up / down)`` samples.  24 kHz takes no launch; a rate whose filter does not fit
    the kernel is a ``ValueError`` (8, 11.025, 12, 16, 22.05, 32, 44.1, 48, 88.2, 96 and 192 kHz fit).  This is not
    librosa's resampler (``soxr_hq``): the two differ in the transition band near 12 kHz, which the top mel filters see.
+
+2b. **Noise reduction** (``as_denoise``; ``noise_reduction_db``, default ``None``: no stage, exactly the launches and
+   bits of the chain without it; the standalone stage is ``denoise``).  A stationary-noise spectral suppressor on each
+   whole 24 kHz row ``y[0 .. n)``, before the trim, so that the leading and trailing noise informs the noise estimate;
+   the trim and the log-mel then read the denoised row.  With ``reduction_db`` in [0, 60]:
+
+   1. STFT: N = 512, hop 128, periodic Hann window ``w``; frame ``f < F = 1 + n // 128`` holds ``w[i] y[128 f - 256 +
+      i]`` with zeros outside ``[0, n)``, and ``X[f, k]`` is its 257-bin real FFT (``torch.stft(center=True,
+      pad_mode="constant", onesided=True)``).
+   2. Power ``P = re^2 + im^2`` in fp32, two rounded products and one rounded add.
+   3. Noise profile (stationary, from the whole recording): ``lambda[k] = max(1e-20, P_(r)[k] / c)`` in fp64, where
+      ``P_(r)[k]`` is the ``r``-th smallest (0-based) of ``P[0 .. F), k]``, ``r = F // 10``, and ``c = -log1p(-0.1)``
+      is the 10 % quantile of an exponential with mean 1: for Gaussian noise, ``lambda`` estimates the noise PSD
+      without bias.
+   4. Decision-directed Wiener gain (Ephraim-Malah), fp64, ``alpha = 0.98``: ``gamma = P / lambda``, ``xi_0 =
+      max(gamma_0 - 1, 0)``, ``xi_f = alpha A_{f-1} + (1 - alpha) max(gamma_f - 1, 0)``, ``W_f = xi_f / (1 + xi_f)``,
+      ``A_f = W_f W_f gamma_f``, ``G_f = max(W_f, g_min)`` stored as fp32, ``g_min = 10^(-reduction_db / 20)``.  The
+      host computes ``c``, ``g_min``, ``alpha`` and ``1 - alpha`` in fp64; the kernel evaluates each operation rounded
+      once in this order, so ``G`` is bit-equal to a numpy float64 model fed the kernel's ``P``.
+   5. Synthesis: ``y'[t] = sum_f w[j] irfft(G_f X_f)[j] / sum_f w[j]^2``, ``j = t - 128 f + 256``, over the frames
+      covering ``t`` in ascending ``f`` (``torch.istft(length=n)``); zeros beyond ``n``.  At ``reduction_db = 0``,
+      ``g_min = 1`` and this is the STFT round trip.
+
+   A row's output depends only on its own samples, bit for bit.  Digital silence stays silence.  A recording whose
+   quietest tenth of frames is digital silence is left almost unchanged (``lambda`` is at its floor).  Non-stationary
+   noise (babble, music) is not tracked.  Three launches, no read-back.
 3. **Trim** (``as_trim_bounds``; ``top_db``, default 30, ``None`` for no trim).  librosa 0.10's ``effects.trim``
    with its defaults (frame 2048, hop 512), evaluated at 24 kHz in fp64: ``q_j`` is the sum of ``y^2`` over block
    ``[512 j, 512 j + 512)`` (zeros at and beyond ``n``); frame ``f < F = 1 + n // 512`` has the power
@@ -37,9 +63,9 @@ reference recording before that log-mel (``test.py:100-108``: ``librosa.load(pat
 Outputs: ``mels`` fp32 ``[B, 80, T_max]`` with zeros beyond each row's frames, ``mel_lens`` int64 ``[B]`` on the host
 (what ``synthesize`` / ``encode_voice`` take), ``bounds`` int32 ``[B, 2]`` on the device, ``(start, end)`` in 24 kHz
 samples.  A row's outputs depend only on its own samples, bit for bit: not on the batch, the padding or the row
-stride.  The call makes at most five launches and one device-to-host read-back (the B bounds, into pinned memory,
-between the trim and the log-mel: it sizes ``T_max`` and finds short rows).  Container formats (WAV, FLAC, MP3
-headers) are the caller's: it hands over sample arrays.
+stride.  The call makes at most five launches, eight with noise reduction, and one device-to-host read-back (the B
+bounds, into pinned memory, between the trim and the log-mel: it sizes ``T_max`` and finds short rows).  Container
+formats (WAV, FLAC, MP3 headers) are the caller's: it hands over sample arrays.
 """
 from __future__ import annotations
 
@@ -176,6 +202,34 @@ def trim_bounds(wave: torch.Tensor, lengths=None, top_db: float = 30.0) -> torch
     return ops.trim_bounds(x, lengths, top_db)
 
 
+def _check_reduction_db(v, name="reduction_db"):
+    if v is None:
+        return None
+    if isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(float(v)) or \
+            not 0.0 <= float(v) <= 60.0:
+        raise ValueError(f"{name} must be a finite number in [0, 60], got {v!r}")
+    return float(v)
+
+
+def denoise(wave: torch.Tensor, lengths=None, reduction_db: float = 18.0) -> torch.Tensor:
+    """Stationary-noise suppression of 24 kHz fp32 ``wave`` (``[B, S]`` or ``[S]``, CUDA) as step 2b of this module's
+    docstring states; ``lengths``: per-row sample counts (int tensor or sequence; None: every row holds S samples).
+    Returns the denoised rows in ``wave``'s shape, zeros beyond each length: listen to them, or feed them to
+    ``LogMel``.  Three launches, no host synchronisation."""
+    reduction_db = _check_reduction_db(reduction_db)
+    if reduction_db is None:
+        raise ValueError("denoise: reduction_db must be a finite number in [0, 60]")
+    ops._require_cuda(wave, "denoise")
+    x = wave.unsqueeze(0) if wave.dim() == 1 else wave
+    x = x.float()
+    if x.stride(-1) != 1 and x.shape[-1] > 1:
+        x = x.contiguous()
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
+    out = ops.denoise(x, lengths, reduction_db)
+    return out[0] if wave.dim() == 1 else out
+
+
 def _read_back(t: torch.Tensor) -> torch.Tensor:
     """Host copy of a small device tensor through pinned memory: the one synchronisation of ``reference_mels``."""
     if not t.is_cuda:
@@ -211,15 +265,18 @@ _enroll_logmel = {}
 
 
 def reference_mels(x: torch.Tensor, lengths: Union[Sequence[int], torch.Tensor, None], sample_rate: int,
-                   encoding: str = "float32", top_db: Optional[float] = 30.0, device=None):
+                   encoding: str = "float32", top_db: Optional[float] = 30.0, device=None,
+                   noise_reduction_db: Optional[float] = None):
     """Reference mels of recordings, as this module's docstring states: ``x`` ``[B, S]`` or ``[B, S, C]`` (host or
     CUDA) of ``audio.DTYPES[encoding]`` at ``sample_rate`` Hz, ``lengths`` host samples per channel (None: S).
     Returns ``(mels fp32 [B, 80, T_max] device, mel_lens int64 [B] host, bounds int32 [B, 2] device)``.  ``device``:
-    where to run when ``x`` is on the host (default ``cuda``).  At most five launches, one read-back."""
+    where to run when ``x`` is on the host (default ``cuda``).  ``noise_reduction_db``: None (no noise reduction) or
+    the ``reduction_db`` of step 2b, in [0, 60].  At most five launches (eight with noise reduction), one read-back."""
     if encoding not in audio.ENCODINGS:
         raise ValueError(f"encoding must be one of {audio.ENCODINGS}, got {encoding!r}")
     rs = audio.to_native_rate(sample_rate)
     top_db = _check_top_db(top_db)
+    noise_reduction_db = _check_reduction_db(noise_reduction_db, "noise_reduction_db")
     if not isinstance(x, torch.Tensor) or x.dim() not in (2, 3):
         raise ValueError(f"x: expected a [B, S] or [B, S, C] tensor, got {getattr(x, 'shape', type(x))}")
     if x.dtype != audio.DTYPES[encoding]:
@@ -245,6 +302,8 @@ def reference_mels(x: torch.Tensor, lengths: Union[Sequence[int], torch.Tensor, 
         n24 = torch.empty(B, dtype=torch.int32, device=dev)
         y = ops.resample_encode(m, lens, rs, rs.out_samples(S), out_lens=n24)
         n24_host = torch.tensor([rs.out_samples(int(v)) for v in n], dtype=torch.int64)
+    if noise_reduction_db is not None:
+        y = ops.denoise(y, n24, noise_reduction_db)
     if top_db is None:
         host = torch.stack([torch.zeros_like(n24_host), n24_host], 1).to(torch.int32)
         bounds = host.to(dev)

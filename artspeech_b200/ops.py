@@ -9,9 +9,11 @@ concatenations are fused away.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass, field
 from typing import Optional, Sequence
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -574,6 +576,58 @@ def trim_bounds(y, lens, top_db: float):
          "trim_bounds"), float(top_db), ws.data_ptr(), ws.numel(), bounds.data_ptr())
     _count(TRIM_LAUNCHES - 1)
     return bounds
+
+
+DENOISE_LAUNCHES = 3             # AS_DENOISE_LAUNCHES
+DENOISE_BINS, DENOISE_N, DENOISE_HOP = 257, 512, 128
+DENOISE_ALPHA, DENOISE_QUANTILE = 0.98, 0.1
+_denoise_tables = {}
+
+
+def _denoise_consts(device):
+    """(window, twiddle, itwiddle) fp32 device tensors of ``as_denoise``, computed once per device in fp64."""
+    t = _denoise_tables.get(device)
+    if t is None:
+        i, m = np.arange(DENOISE_N), np.arange(DENOISE_N // 2)
+        ang = 2.0 * np.pi * m / DENOISE_N
+        tabs = (0.5 - 0.5 * np.cos(2.0 * np.pi * i / DENOISE_N), np.stack([np.cos(ang), -np.sin(ang)], 1),
+                np.stack([np.cos(ang), np.sin(ang)], 1))
+        t = tuple(torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(device) for a in tabs)
+        _denoise_tables[device] = t
+    return t
+
+
+def denoise(y, lens, reduction_db: float, *, planes: bool = False):
+    """Stationary-noise suppression of 24 kHz fp32 ``y`` [B, S] (unit element stride, any row stride; ``as_denoise``,
+    semantics in ``artspeech_b200.frontend`` step 2b), ``lens`` int32 [B] device sample counts (or None: every row
+    holds S samples), ``reduction_db`` in [0, 60].  Returns a new fp32 [B, S], zeros beyond each length.  With
+    ``planes=True`` also the workspace's ``X`` (complex64 [B, 1 + S // 128, 257]), ``lambda`` (fp64 [B, 257]) and
+    ``G`` (fp32 [B, 1 + S // 128, 257]) as views; frame rows at and beyond a row's ``1 + len // 128`` are not
+    written.  Three launches, no host synchronisation."""
+    _require_cuda(y, "denoise")
+    B, S = _wave_rows(y, "denoise")
+    rdb = float(reduction_db)
+    if not 0.0 <= rdb <= 60.0:
+        raise _lib.AsError(f"denoise: reduction_db must be in [0, 60], got {reduction_db!r}")
+    window, tw, itw = _denoise_consts(y.device)
+    out = torch.empty(B, S, dtype=torch.float32, device=y.device)
+    nbytes = int(_lib.load().as_denoise_workspace_bytes(B, S))
+    ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=y.device)
+    alpha = DENOISE_ALPHA
+    _run("as_denoise", y, y.data_ptr(), y.stride(0) if B > 1 else S, B, S, _lens_arg(lens, B, y.device, "denoise"),
+         rdb, window.data_ptr(), tw.data_ptr(), itw.data_ptr(), -math.log1p(-DENOISE_QUANTILE), 10.0 ** (-rdb / 20.0),
+         alpha, 1.0 - alpha, ws.data_ptr(), ws.numel(), out.data_ptr(), S)
+    _count(DENOISE_LAUNCHES - 1)
+    if not planes:
+        return out
+    F = 1 + S // DENOISE_HOP
+    align = lambda v: (v + 255) // 256 * 256
+    nx, ng = B * F * DENOISE_BINS * 8, B * F * DENOISE_BINS * 4
+    X = ws[:nx].view(torch.complex64).view(B, F, DENOISE_BINS)
+    G = ws[align(nx):align(nx) + ng].view(torch.float32).view(B, F, DENOISE_BINS)
+    lo = align(nx) + align(ng)
+    lam = ws[lo:lo + B * DENOISE_BINS * 8].view(torch.float64).view(B, DENOISE_BINS)
+    return out, X, lam, G
 
 
 WATERMARK_DETECT_LAUNCHES = 2    # AS_WM_DETECT_LAUNCHES

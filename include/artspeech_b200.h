@@ -392,6 +392,33 @@ size_t as_trim_workspace_bytes(int32_t B, int32_t S);
 int as_trim_bounds(const float* y, int64_t y_ld, int32_t B, int32_t S, const int32_t* lens, double top_db,
                    void* workspace, size_t workspace_bytes, int32_t* bounds, void* stream);
 
+/* Stationary-noise suppression of 24 kHz fp32 rows (voice enrollment, artspeech_b200/frontend.py step 2b), y [B, >= S]
+ * row stride y_ld, n_b = min(lens[b], S) (S when lens is NULL), F_b = 1 + n_b / 128 frames:
+ *   X[f, k]: 257-bin real FFT of the frame w[i] y[128 f - 256 + i], i < 512 (zeros outside [0, n_b)), fp32;
+ *   P = re^2 + im^2 as two rounded fp32 products and one rounded add;
+ *   lambda[k] = max(1e-20, P_(r)[k] / c) in fp64, P_(r)[k] the (F_b / 10)-th smallest (0-based) of P[0 .. F_b), k];
+ *   in fp64 (__dmul_rn, __dadd_rn, __ddiv_rn, in this order): gamma = P / lambda, m = max(gamma - 1, 0),
+ *   xi_0 = m_0, xi_f = alpha A_{f-1} + one_minus_alpha m_f, W = xi / (1 + xi), A = (W W) gamma, and
+ *   G = max(W, g_min) rounded to fp32;
+ *   out[t] = sum_f w[j] irfft(G_f X_f)[j] / sum_f w[j]^2, j = t - 128 f + 256, over f < F_b covering t, ascending;
+ *   out[t] = 0 for n_b <= t < S.
+ * window fp32 [512] (periodic Hann), twiddle / itwiddle fp32 [256][2] = (cos, -sin) / (cos, sin)(2 pi m / 512), device.
+ * reduction_db in [0, 60]; g_min = 10^(-reduction_db / 20), c = -log1p(-0.1), alpha = 0.98 and one_minus_alpha =
+ * 1 - alpha, computed on the host in fp64.  out [B, S] row stride out_ld, not aliasing y.
+ * workspace: device, 256-byte aligned, at least as_denoise_workspace_bytes(B, S) bytes = X (complex fp32
+ * [B][1 + S / 128][AS_DENOISE_BINS], 16 bytes per input sample) at offset 0, then G (fp32, same shape), then lambda
+ * (fp64 [B][AS_DENOISE_BINS]), each starting on a 256-byte boundary.  AS_DENOISE_LAUNCHES launches (STFT; noise
+ * profile and gain; inverse FFT and overlap-add), no floating-point atomics, no host synchronisation; every value of a
+ * row follows from its own samples, so the output does not depend on B, S, the strides or the batch-mates.  Samples
+ * at or beyond n_b are never read. */
+#define AS_DENOISE_BINS 257
+#define AS_DENOISE_LAUNCHES 3
+size_t as_denoise_workspace_bytes(int32_t B, int32_t S);
+int as_denoise(const float* y, int64_t y_ld, int32_t B, int32_t S, const int32_t* lens, double reduction_db,
+               const float* window, const float* twiddle, const float* itwiddle, double c, double g_min, double alpha,
+               double one_minus_alpha, void* workspace, size_t workspace_bytes, float* out, int64_t out_ld,
+               void* stream);
+
 /* Watermark detector on 8 kHz fp32 utterances x [B, >= S] (row stride x_ld), n_b = min(lens[b], S) (S when NULL):
  *   z[t] = x[t] / e(t) where e(t) >= 1e-4, else 0 (e as in the embedder with 80-sample frames); Z_p = DFT of
  *   z[4096 p .. 4096 p + 4095] (zeros beyond n_b) at the pattern bins, p < ceil(n_b / 4096); A = sum_p Z_p,
