@@ -1,8 +1,10 @@
 """Output audio formats for synthesis: any integer sample rate by polyphase resampling, and fp32 / 16-bit PCM /
-ITU-T G.711 mu-law and A-law samples, computed on the GPU after the vocoder (``as_resample_encode``); loudness
-normalisation; and the synthesis watermark.
+ITU-T G.711 mu-law and A-law samples, computed on the GPU after the vocoder (``as_resample_encode``); FLAC files of
+the 16-bit PCM (``as_flac_encode``); loudness normalisation; and the synthesis watermark.
 
-``AudioFormat(sample_rate, encoding)`` names a format; the vocoder's own is ``AudioFormat(24000, "float32")``.
+``AudioFormat(sample_rate, encoding, container)`` names a format; the vocoder's own is ``AudioFormat(24000,
+"float32")``.  ``container`` is ``"raw"`` (samples) or ``"flac"`` (one FLAC file per utterance, ``encoding="pcm16"``
+only).
 
 Semantics (per utterance of ``n_in`` samples at 24 kHz):
 
@@ -20,6 +22,42 @@ Semantics (per utterance of ``n_in`` samples at 24 kHz):
 
 A rate whose filter does not fit the kernel's shared-memory budget (``smem_bytes`` above ``SMEM_MAX``: very low rates
 and rates with a large ``up``, e.g. 44101 Hz) is refused on construction.
+
+**FLAC** (``AudioFormat(rate, "pcm16", container="flac")``, ``as_flac_encode``, ``encode_flac``).  The encoder input
+of an utterance is its ``n`` int16 samples: exactly what the same call gives with ``AudioFormat(rate, "pcm16")``.
+The output is one RFC 9639 stream inside the streamable subset, reproduced bit for bit by the GPU:
+
+1. **Stream.**  ``fLaC``, one STREAMINFO block (last-metadata flag set, length 34): min / max block size 4096, min /
+   max frame size of this stream in bytes (0 without frames), the sample rate, 1 channel, 16 bits per sample, total
+   samples ``n``, MD5 all zero ("not computed").  Then frames ``f = 0 .. ceil(n / 4096) - 1`` of ``bs = min(4096,
+   n - 4096 f)`` samples.  ``n = 0`` is the 42-byte header alone.  Rates are 1 .. 65535 Hz (the frame header carries
+   any other rate than the table's in 16 bits).
+2. **Frame header.**  Sync ``0xFFF8`` (fixed block size: the header carries the frame number); block-size code
+   ``0b1100`` for 4096, else ``0b0111`` and 16-bit ``bs - 1``; sample-rate code from the table for 8, 16, 22.05, 24,
+   32, 44.1 and 48 kHz, else ``0b1101`` and the 16-bit rate in Hz; channels ``0b0000``, sample size ``0b100``,
+   reserved bits 0; the frame number in FLAC's UTF-8-style coding; CRC-8 (polynomial 0x07, initial 0, MSB first).
+3. **Subframe.**  The exact bit size of every candidate is computed and the smallest kept, the earlier on ties, in
+   this order: CONSTANT (all samples equal; 8 + 16 bits), FIXED orders 0-4 with ``bs > order`` (8 + 16 order +
+   residual), LPC orders ``p = 1 .. 8`` with ``bs > p`` (8 + 16 p + 4 + 5 + 12 p + residual), VERBATIM (8 + 16 bs).
+   No wasted-bits flag.
+4. **LPC.**  ``R[l] = sum_{i=l}^{bs-1} x[i] x[i-l]``, l = 0..8, exact in int64 (no window), then fp64.
+   Levinson-Durbin in fp64 without fused multiply-add: ``E = R0``; for each order ``m``: stop if ``E <= 0``;
+   ``acc = R[m]``, ``acc = acc - a_j R[m-j]`` for ``j = 1 .. m-1`` ascending, ``k = acc / E`` (stop if not finite);
+   ``a_j <- a_j - k a_{m-j}`` from the old values, ``a_m = k``; ``E = E (1 - k k)``.  Orders reached are candidates.
+   Quantisation at precision 12 (any ``a_j`` not finite: no candidate): ``cmax = max |a_j|``, ``(_, e) = frexp(cmax)``,
+   ``shift = 11 - e`` (negative: no candidate; above 15: 15); ``err = 0``, for ``j = 1 .. p``: ``err += a_j 2^shift``,
+   ``q_j = clamp(llround(err), -2048, 2047)``, ``err -= q_j``, written in this order.  Residual ``r[i] = x[i] -
+   ((sum_j q_j x[i-j]) >> shift)`` for ``i >= p`` in int64 with an arithmetic shift; the first ``p`` samples are the
+   warm-up.  FIXED order ``o`` is the same with the binomial predictor and shift 0.
+5. **Residual.**  Method ``00`` (4-bit Rice parameters, no escape).  Zigzag ``u = 2 r`` or ``-2 r - 1``; a candidate
+   with any ``|r| >= 2^31`` is dropped.  Partition orders ``o = 0 .. 8`` with ``bs % 2^o == 0`` and ``(bs >> o) >
+   order``; per partition the parameter ``k in 0 .. 14`` minimises ``4 + sum ((u >> k) + 1 + k)`` (the smaller k on
+   ties); the order minimises ``2 + 4 + sum over partitions`` (the smaller o on ties).
+6. **Frame end.**  Zero padding to a byte boundary, then CRC-16 of the whole frame (polynomial 0x8005, initial 0,
+   MSB first).
+7. **Bound.**  A file is at most ``42 + 2 n + 18 ceil(n / 4096)`` bytes (``flac_max_bytes``): VERBATIM is always a
+   candidate and a frame header is at most 15 bytes.  Rows of FLAC output are this long for the row's sample count,
+   zero after each stream's last byte; the byte counts come separately.
 
 **Loudness normalisation** (``Loudness(target_lufs, max_true_peak_db)``, ``as_loudness_measure``).  The meter, for
 one utterance of ``n`` fp32 samples at ``fs`` Hz (the engine meters at 24 kHz; ``measure_loudness`` takes any multiple
@@ -103,6 +141,9 @@ import torch
 
 NATIVE_RATE = 24000
 ENCODINGS = ("float32", "pcm16", "mulaw", "alaw")
+CONTAINERS = ("raw", "flac")
+FLAC_BLOCK = 4096                # AS_FLAC_BLOCK
+FLAC_MAX_RATE = 65535
 CODES = {"float32": 0, "pcm16": 1, "mulaw": 2, "alaw": 3}            # AS_AUDIO_F32 .. AS_AUDIO_ALAW
 DTYPES = {"float32": torch.float32, "pcm16": torch.int16, "mulaw": torch.uint8, "alaw": torch.uint8}
 SILENCE = {"float32": 0, "pcm16": 0, "mulaw": 0xFF, "alaw": 0xD5}
@@ -143,12 +184,20 @@ def smem_bytes(up: int, down: int, K: int, table_ld: int) -> int:
 _TABLES: Dict[tuple, torch.Tensor] = {}
 
 
+def flac_max_bytes(n: int) -> int:
+    """The largest FLAC file of ``n`` samples: ``42 + 2 n + 18 ceil(n / 4096)`` bytes."""
+    n = int(n)
+    return 42 + 2 * n + 18 * (-(-n // FLAC_BLOCK))
+
+
 @dataclass(frozen=True)
 class AudioFormat:
-    """An output format: integer ``sample_rate`` (Hz) and ``encoding`` in ``ENCODINGS``; validated on
-    construction (``ValueError``)."""
+    """An output format: integer ``sample_rate`` (Hz), ``encoding`` in ``ENCODINGS`` and ``container`` in
+    ``CONTAINERS`` (``"flac"`` needs ``encoding="pcm16"`` and a rate of at most 65535 Hz); validated on construction
+    (``ValueError``)."""
     sample_rate: int = NATIVE_RATE
     encoding: str = "float32"
+    container: str = "raw"
 
     def __post_init__(self):
         rate = self.sample_rate
@@ -162,6 +211,13 @@ class AudioFormat:
             raise ValueError(f"AudioFormat.sample_rate: must be positive, got {rate}")
         if self.encoding not in ENCODINGS:
             raise ValueError(f"AudioFormat.encoding: expected one of {ENCODINGS}, got {self.encoding!r}")
+        if self.container not in CONTAINERS:
+            raise ValueError(f"AudioFormat.container: expected one of {CONTAINERS}, got {self.container!r}")
+        if self.container == "flac" and self.encoding != "pcm16":
+            raise ValueError(f"AudioFormat: container='flac' holds 16-bit PCM; use encoding='pcm16', "
+                             f"got {self.encoding!r}")
+        if self.container == "flac" and rate > FLAC_MAX_RATE:
+            raise ValueError(f"AudioFormat: container='flac' takes rates up to {FLAC_MAX_RATE} Hz, got {rate}")
         object.__setattr__(self, "sample_rate", rate)
         if smem_bytes(self.up, self.down, self.K, self.table_ld) > SMEM_MAX:
             raise ValueError(f"AudioFormat.sample_rate: {rate} Hz (up {self.up}, down {self.down}) needs "
@@ -222,9 +278,19 @@ class AudioFormat:
         """Output samples of an utterance of ``n_in`` samples at 24 kHz: ``ceil(n_in * up / down)``."""
         return -(-int(n_in) * self.up // self.down)
 
+    def out_bytes(self, n_in: int) -> int:
+        """Row length of a FLAC output for ``n_in`` samples at 24 kHz: ``flac_max_bytes(out_samples(n_in))``."""
+        return flac_max_bytes(self.out_samples(n_in))
+
+    @property
+    def raw(self) -> "AudioFormat":
+        """The sample format inside the container (``self`` for ``"raw"``)."""
+        return self if self.container == "raw" else AudioFormat(self.sample_rate, self.encoding)
+
     @property
     def dtype(self) -> torch.dtype:
-        return DTYPES[self.encoding]
+        """The element type of the output: the encoding's, bytes (uint8) for FLAC."""
+        return torch.uint8 if self.container == "flac" else DTYPES[self.encoding]
 
     @property
     def code(self) -> int:
@@ -556,6 +622,23 @@ def detect_watermark(x: torch.Tensor, lengths, sample_rate: int, key: int, encod
         lengths = n8
     detected, score, _, message = ops.watermark_detect(x, lengths, key, float(threshold))
     return detected, score, message
+
+
+def encode_flac(x: torch.Tensor, lengths, sample_rate: int):
+    """FLAC files (this module's format) of 16-bit PCM ``x`` (int16 [B, S] or [S], CUDA) at ``sample_rate`` Hz
+    (1 .. 65535); ``lengths``: per-row sample counts (int tensor or sequence; None: every row holds S samples).
+    Returns ``(files, nbytes)`` device tensors: uint8 ``[B, flac_max_bytes(S)]`` (row ``b``'s file is
+    ``files[b, :nbytes[b]]``, zeros after it) and int64 ``[B]``; no host synchronisation."""
+    from . import ops
+    if not _rate_ok_any(sample_rate) or int(sample_rate) > FLAC_MAX_RATE:
+        raise ValueError(f"encode_flac: sample_rate must be an integer in [1, {FLAC_MAX_RATE}], got {sample_rate!r}")
+    if not torch.is_tensor(x) or x.dtype != torch.int16 or x.dim() not in (1, 2):
+        raise ValueError(f"encode_flac: x must be an int16 [B, S] or [S] tensor, got "
+                         f"{getattr(x, 'dtype', type(x).__name__)} {tuple(getattr(x, 'shape', ()))}")
+    x = x.view(1, -1) if x.dim() == 1 else x
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
+    return ops.flac_encode(x, lengths, int(sample_rate))
 
 
 def _rate_ok_any(fs) -> bool:

@@ -384,7 +384,10 @@ class Synthesizer:
         encoding (in ``audio``'s format, or the native 24 kHz fp32), and ``last["loudness"]``, ``last["true_peak"]``
         and ``last["gain_db"]`` hold the values measured before the gain (fp64 [B], device).
         ``watermark``: an ``audio.Watermark``; each utterance's 24 kHz waveform is then marked before the meter and the
-        format stage (``audio.embed_watermark`` of the pass's waveform, bit for bit)."""
+        format stage (``audio.embed_watermark`` of the pass's waveform, bit for bit).
+        A FLAC ``audio`` (``container="flac"``) returns uint8 ``[B, audio.out_bytes(300*Tm_max)]``: row ``b`` is one
+        complete file of the samples the same call gives with ``container="raw"``, zeros after it, and
+        ``last["byte_lengths"]`` (int64, device) holds the files' lengths."""
         dev = self.device
         cur = torch.cuda.current_stream(dev)
         self.last_stream = cur
@@ -525,11 +528,12 @@ class Synthesizer:
 
     def _format_stage(self, res, fmt, side_slot=None, loud=None, wm=None):
         """One ``as_resample_encode`` launch on ``last_stream`` after the pass, into a fresh stream-ordered
-        allocation; not captured, so it adds no graphs.  ``side_slot``: the pipeline slot whose side stream ran the
-        call (``join`` then also waits for the format stage).  ``loud``: an ``audio.Loudness``; the meter's launches
-        then precede it on the same stream and its gain is applied.  ``wm``: an ``audio.Watermark``; one
-        ``as_watermark_embed`` launch first marks the waveform the meter and the format read (``fmt`` None: the marked
-        waveform is the result)."""
+        allocation; not captured, so it adds no graphs.  A FLAC format encodes that launch's int16 output with
+        ``as_flac_encode`` (three more launches) and puts the byte counts in ``last["byte_lengths"]``.  ``side_slot``:
+        the pipeline slot whose side stream ran the call (``join`` then also waits for the format stage).  ``loud``: an
+        ``audio.Loudness``; the meter's launches then precede it on the same stream and its gain is applied.  ``wm``: an
+        ``audio.Watermark``; one ``as_watermark_embed`` launch first marks the waveform the meter and the format read
+        (``fmt`` None: the marked waveform is the result)."""
         wav, mel_lengths, mel = res
         with torch.cuda.stream(self.last_stream):
             if wm is not None:
@@ -537,16 +541,20 @@ class Synthesizer:
                 if self.last.get("graph"):
                     self.launches_per_call += 1
             n = None if fmt is None else torch.empty(wav.shape[0], dtype=torch.int32, device=wav.device)
+            raw = None if fmt is None else fmt.raw
             if fmt is None:
                 y = wav
             elif loud is None:
-                y = ops.resample_encode(wav, self.last["wav_lengths"], fmt, fmt.out_samples(wav.shape[1]), out_lens=n)
+                y = ops.resample_encode(wav, self.last["wav_lengths"], raw, raw.out_samples(wav.shape[1]), out_lens=n)
             else:
                 lufs, tp, gain_db, gain = ops.loudness_measure(wav, self.last["wav_lengths"], SAMPLE_RATE,
                                                                loud.target_lufs, loud.max_true_peak_db)
-                y = ops.resample_encode(wav, self.last["wav_lengths"], fmt, fmt.out_samples(wav.shape[1]), out_lens=n,
+                y = ops.resample_encode(wav, self.last["wav_lengths"], raw, raw.out_samples(wav.shape[1]), out_lens=n,
                                         gain=gain)
                 self.last.update(loudness=lufs, true_peak=tp, gain_db=gain_db)
+            if fmt is not None and fmt.container == "flac":
+                y, nbytes = ops.flac_encode(y, n, fmt.sample_rate)
+                self.last["byte_lengths"] = nbytes
             if side_slot is not None:
                 done = torch.cuda.Event()
                 done.record(self.last_stream)
@@ -554,7 +562,8 @@ class Synthesizer:
         if fmt is not None:
             self.last["sample_lengths"] = n
             if self.last.get("graph"):
-                self.launches_per_call += 1 + (ops.LOUDNESS_LAUNCHES if loud is not None else 0)
+                self.launches_per_call += 1 + (ops.LOUDNESS_LAUNCHES if loud is not None else 0) + \
+                    (ops.FLAC_LAUNCHES if fmt.container == "flac" else 0)
         return y, mel_lengths, mel
 
     def _done_ticket(self, res):
@@ -724,9 +733,11 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     returns: it synchronises the copies).  ``prosody``: one ``prosody.Prosody`` per utterance (or None); the planning
     estimate of an utterance then grows with its mean ``duration_scale``.  ``audio``: an ``audio.AudioFormat`` (see
     ``Synthesizer.synthesize``); ``wavs[i]`` then holds the ``audio.out_samples(300 * frames[i])`` samples of
-    utterance ``i`` in that format.  ``loudness``: an ``audio.Loudness`` (see ``Synthesizer.synthesize``); each
-    utterance is normalised on its own waveform, so its gain does not depend on its batch-mates.  ``watermark``: an
-    ``audio.Watermark`` (see ``Synthesizer.synthesize``); each utterance's mark depends only on its own samples."""
+    utterance ``i`` in that format; for a FLAC format ``wavs[i]`` is utterance ``i``'s complete file (uint8), cut to
+    its length once the call's byte counts have come back (one pinned copy per micro-batch).  ``loudness``: an
+    ``audio.Loudness`` (see ``Synthesizer.synthesize``); each utterance is normalised on its own waveform, so its gain
+    does not depend on its batch-mates.  ``watermark``: an ``audio.Watermark`` (see ``Synthesizer.synthesize``); each
+    utterance's mark depends only on its own samples."""
     n = len(tokens)
     pros = prosody_mod.check(prosody, [int(t.shape[0]) for t in tokens], durations is not None)
     if durations is not None:
@@ -749,10 +760,19 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     def cut(f):
         """Samples of an utterance of ``f`` mel frames in the output format."""
         return fmt.out_samples(HOP * f) if fmt is not None else HOP * f
+    flac = fmt is not None and fmt.container == "flac"
     arena = arena or (HostArena() if to_host else None)
     if to_host:
         arena.reset()
-    pending, late = [], []
+    pending, late, sized, copied = [], [], [], []
+
+    def mark_copies():
+        """Event after the copies just queued on the call's stream: the host waits on it before reading them (on a
+        pipelined engine that stream is a slot's side stream, which ``join`` covers only up to the format stage)."""
+        if syn.last_stream is not None:
+            ev = torch.cuda.Event()
+            ev.record(syn.last_stream)
+            copied.append(ev)
 
     def collect(idx, ticket):
         """Finish a deferred call and queue the copies of its waveforms (on the call's stream)."""
@@ -766,17 +786,26 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
                 S = wav.shape[1]
                 dst = arena.take(len(idx) * S, dt).view(len(idx), S)
                 dst.copy_(wav, non_blocking=True)
+            elif flac:
+                dst = wav                       # a fresh allocation of this call's format stage, not a graph buffer
             else:
                 dst = wav.clone() if got is None else None
+            if flac:
+                # FLAC rows are cut to their byte counts after the final synchronisation
+                nb = arena.take(len(idx), torch.int64) if to_host else \
+                    torch.empty(len(idx), dtype=torch.int64).pin_memory()
+                nb.copy_(syn.last["byte_lengths"], non_blocking=True)
+                sized.append((idx, dst, nb))
             if got is None:
                 # sync-free pass (Synthesizer(duration_bound=...)): the frame counts come back with the waveforms
                 meta = arena.take(2 * len(idx), torch.int32) if to_host else torch.empty(2 * len(idx), dtype=torch.int32).pin_memory()
                 meta[:len(idx)].copy_(mel_lengths, non_blocking=True)
                 meta[len(idx):].copy_(syn.last["pred_sum"], non_blocking=True)
                 late.append((idx, dst, meta, syn.last["frame_bound"]))
-            else:
+            elif not flac:
                 for j, i in enumerate(idx):
                     wavs[i] = dst[j, :cut(frames[i])] if to_host else wav[j, :cut(frames[i])].clone()
+            mark_copies()
 
     # With predicted durations a call synchronises on its frame counts between its two graphs: issue the NEXT
     # micro-batch's first graph before finishing the current one (one call of look-ahead; needs a second pipeline slot)
@@ -804,8 +833,10 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
     while waiting:
         collect(*waiting.pop(0))
     syn.join()
-    if to_host or late:
+    if to_host or late or sized:
         torch.cuda.current_stream(syn.device).synchronize()
+        for ev in copied:
+            ev.synchronize()
     redo = []
     for idx, dst, meta, bound in late:
         for j, i in enumerate(idx):
@@ -813,16 +844,29 @@ def synthesize_many(syn: "Synthesizer", tokens: Sequence[torch.Tensor], ref_mels
             wavs[i] = dst[j, :cut(frames[i])]
             if 2 * int(meta[len(idx) + j]) > bound:       # the prediction did not fit the bound: truncated there
                 redo.append(i)
+    for idx, dst, nb in sized:
+        for j, i in enumerate(idx):
+            wavs[i] = dst[j, :int(nb[j])]
+    redo_sized = []
     for i in redo:                                         # rare: exact two-graph pass for the utterances that overflowed
         w, _, _ = syn.synthesize(tokens[i].view(1, -1).pin_memory(), [int(tokens[i].shape[0])],
                                  ref_mels[i].unsqueeze(0).pin_memory(), [int(ref_mels[i].shape[1])], None, exact_frames=True,
                                  prosody=[pros[i]] if pros else None, audio=fmt, **loud_kw)
         frames[i] = syn.last["frames"][0]
         with torch.cuda.stream(syn.last_stream):
-            wavs[i] = w[0, :cut(frames[i])].clone() if not to_host else w[0, :cut(frames[i])].to("cpu")
+            if flac:
+                wavs[i] = w[0] if not to_host else w[0].to("cpu")
+                redo_sized.append((i, syn.last["byte_lengths"]))
+            else:
+                wavs[i] = w[0, :cut(frames[i])].clone() if not to_host else w[0, :cut(frames[i])].to("cpu")
+            mark_copies()
     if redo:
         syn.join()
         torch.cuda.current_stream(syn.device).synchronize()
+        for ev in copied:
+            ev.synchronize()
+    for i, nb in redo_sized:
+        wavs[i] = wavs[i][:int(nb[0])]
     return wavs, frames
 
 

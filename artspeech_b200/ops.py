@@ -434,6 +434,8 @@ def resample_encode(x, lens, fmt, S_out: int, *, m0: int = 0, out=None, out_lens
     ``gain``: an optional fp32 [B] device tensor multiplied into each utterance's samples before they are encoded
     (``as_resample_encode_gain``)."""
     _require_cuda(x, "resample_encode")
+    if getattr(fmt, "container", "raw") != "raw":
+        raise _lib.AsError(f"resample_encode: writes samples; {fmt} is a container (encode its .raw format first)")
     if x.dtype != torch.float32 or x.dim() != 2 or (x.stride(1) != 1 and x.shape[1] > 1):
         raise _lib.AsError(f"resample_encode: x must be fp32 [B, S] with unit sample stride, got {x.dtype} "
                            f"{tuple(x.shape)} strides {x.stride()}")
@@ -628,6 +630,30 @@ def denoise(y, lens, reduction_db: float, *, planes: bool = False):
     lo = align(nx) + align(ng)
     lam = ws[lo:lo + B * DENOISE_BINS * 8].view(torch.float64).view(B, DENOISE_BINS)
     return out, X, lam, G
+
+
+FLAC_LAUNCHES = 3                # AS_FLAC_LAUNCHES
+
+
+def flac_encode(x, lens, sample_rate: int):
+    """FLAC files of int16 mono rows (``as_flac_encode``; format in ``artspeech_b200.audio``): ``x`` int16 [B, S]
+    (unit element stride, any row stride) at ``sample_rate`` Hz (1 .. 65535), ``lens`` int32 [B] device sample counts
+    (or None: every row holds S samples).  Returns ``(out, nbytes)``: uint8 [B, audio.flac_max_bytes(S)], each row one
+    complete stream followed by zeros, and int64 [B] device byte counts.  Three launches, no host synchronisation."""
+    from . import audio
+    _require_cuda(x, "flac_encode")
+    B, S = _wave_rows(x, "flac_encode", torch.int16)
+    rate = int(sample_rate)
+    if not 1 <= rate <= 65535:
+        raise _lib.AsError(f"flac_encode: sample_rate must be in [1, 65535] Hz, got {sample_rate!r}")
+    out = torch.empty(B, audio.flac_max_bytes(S), dtype=torch.uint8, device=x.device)
+    nbytes = torch.empty(B, dtype=torch.int64, device=x.device)
+    ws = torch.empty(max(int(_lib.load().as_flac_workspace_bytes(B, S)), 1), dtype=torch.uint8, device=x.device)
+    _run("as_flac_encode", x, x.data_ptr(), x.stride(0) if B > 1 else S, B, S, _lens_arg(lens, B, x.device,
+         "flac_encode"), rate, ws.data_ptr(), ws.numel(), out.data_ptr(), out.stride(0) if B > 1 else out.shape[1],
+         nbytes.data_ptr())
+    _count(FLAC_LAUNCHES - 1)
+    return out, nbytes
 
 
 WATERMARK_DETECT_LAUNCHES = 2    # AS_WM_DETECT_LAUNCHES

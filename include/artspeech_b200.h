@@ -419,6 +419,25 @@ int as_denoise(const float* y, int64_t y_ld, int32_t B, int32_t S, const int32_t
                double one_minus_alpha, void* workspace, size_t workspace_bytes, float* out, int64_t out_ld,
                void* stream);
 
+/* FLAC (RFC 9639, streamable subset) of int16 mono utterances x [B, >= S] (row stride x_ld), n_b = min(lens[b], S) (S
+ * when lens is NULL), at sample_rate Hz (1 .. 65535).  The stream is artspeech_b200/audio.py's format: fLaC, one
+ * STREAMINFO block (block size 4096, min / max frame size, MD5 zero), then frames of AS_FLAC_BLOCK samples (the last
+ * may be shorter), each the smallest of CONSTANT, FIXED 0..4, LPC 1..8 (fp64 Levinson without FMA, precision 12) and
+ * VERBATIM, earlier on ties, with Rice-coded residuals (partition order 0..8, parameter 0..14).
+ * out [B, >= as_flac_max_bytes(S)] uint8 (row stride out_ld, any alignment): row b holds its stream followed by zeros
+ * up to as_flac_max_bytes(S); out_bytes int64 [B] (device) receives each stream's length.  workspace: device,
+ * 256-byte aligned, at least as_flac_workspace_bytes(B, S) bytes (a decision record and an offset per frame).
+ * AS_FLAC_LAUNCHES launches (analysis; layout; emit), no floating-point atomics, no host synchronisation; every byte
+ * of a row follows from its own samples and n_b, so the output does not depend on B, S, the strides or the
+ * batch-mates.  Samples at or beyond n_b are never read. */
+#define AS_FLAC_BLOCK 4096
+#define AS_FLAC_LAUNCHES 3
+int64_t as_flac_max_bytes(int64_t n);
+size_t as_flac_workspace_bytes(int32_t B, int64_t S);
+int as_flac_encode(const int16_t* x, int64_t x_ld, int32_t B, int64_t S, const int32_t* lens, int32_t sample_rate,
+                   void* workspace, size_t workspace_bytes, uint8_t* out, int64_t out_ld, int64_t* out_bytes,
+                   void* stream);
+
 /* Watermark detector on 8 kHz fp32 utterances x [B, >= S] (row stride x_ld), n_b = min(lens[b], S) (S when NULL):
  *   z[t] = x[t] / e(t) where e(t) >= 1e-4, else 0 (e as in the embedder with 80-sample frames); Z_p = DFT of
  *   z[4096 p .. 4096 p + 4095] (zeros beyond n_b) at the pattern bins, p < ceil(n_b / 4096); A = sum_p Z_p,
